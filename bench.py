@@ -9,11 +9,14 @@ device (ssa_ukf_catalog_stats) and all-gathers them over NCCL — both inside th
 couple (SURVEY 8e), so that gather is the only collective.  Rank 0 prints ONE JSON line; C2 (the 20 000-orbit
 catalog) and C3 (4 096 vectorised environments) are measured briefly on rank 0 and reported under `extra`.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c4|c2|c3] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c4|c2|c3] [--impl reference] [--dump-outputs DIR]
 
 `--impl reference` times the CPU oracle port of the reference's algorithm (oracle/ukf_oracle.c, OpenMP over all
 host cores) on a bounded sample of the same workload — the reference itself is pure Python around filterpy and
 cannot be built or installed offline (DESIGN.md "Reference arm").
+
+`--dump-outputs DIR` writes what the last timed step returned as DIR/<name>.npy.  Every input is drawn from fixed seeds,
+so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes
@@ -73,7 +76,44 @@ def parse():
     ap.add_argument("--no-extra", action="store_true", help="skip the short C2 / C3 measurements reported under `extra`")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=10.0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float32 / float64; "
+                         f"c2 / c4: rank 0's shard, a fixed sample of at most {DUMP_MAX_OBJECTS} objects) to compare builds")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
+    return a
+
+
+# --dump-outputs of c2 / c4: rows of a fixed RandomState(0) sample of the shard, in index order (528 B per object)
+DUMP_MAX_OBJECTS = 65536
+
+
+def write_outputs(out_dir, arrays):
+    """Save each array as out_dir/<name>.npy; float32 and float64 stay as they are, anything else becomes float64."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in arrays.items():
+        arr = np.asarray(arr)
+        if arr.dtype not in (np.float32, np.float64):
+            arr = arr.astype(np.float64)
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+
+
+def dump_catalog_outputs(out_dir, ukf, gathered):
+    """The per-object results of the last timed step of this rank's shard (a sample of DUMP_MAX_OBJECTS objects when the
+    shard is larger) and, c4, the reward terms gathered from every rank [world, 5]."""
+    from ssa_gym_b200 import _lib as F
+    n = ukf.N
+    rows = np.arange(n) if n <= DUMP_MAX_OBJECTS else np.sort(np.random.RandomState(0).choice(n, DUMP_MAX_OBJECTS, replace=False))
+    fields = {"x_true": F.F_X_TRUE, "x_filter": F.F_X_FILTER, "P_filter": F.F_P_FILTER, "obs": F.F_OBS,
+              "delta_pos": F.F_DELTA_POS, "delta_vel": F.F_DELTA_VEL, "sigma_pos": F.F_SIGMA_POS, "sigma_vel": F.F_SIGMA_VEL,
+              "trace": F.F_TRACE, "status": F.F_STATUS, "inflations": F.F_INFLATIONS}
+    out = {name: ukf.download(f)[rows] for name, f in fields.items()}
+    if gathered is not None:
+        out["catalog_stats"] = gathered.cpu().numpy().reshape(-1, 5)
+    write_outputs(out_dir, out)
 
 
 def workload_inputs(n_objects, rank, steps, lo=0, hi=None):
@@ -233,12 +273,12 @@ def make_cfg(N):
     return c
 
 
-def c3_measure(a, rank, local_rank, world, steps, warmup, gather):
+def c3_measure(a, rank, local_rank, world, steps, warmup, gather, dump_dir=None):
     """BASELINE.json config 3: E parallel environments x default RSO count, one vectorised env step per call, actions
     from the device-side greedy tasker, obs [E, m*12] fp64 handed to the host every step (the RLlib rollout shape).
     Metric: env-steps per second through the public API (VecSSATaskerEnv.vector_step), i.e. end to end by
     construction: every step copies the actions host->device and obs / reward / done device->host.  Returns the
-    JSON line as a dict (rank 0) or None."""
+    JSON line as a dict (rank 0) or None; dump_dir: rank 0 writes the last timed step's obs / reward / done there."""
     import torch
     import torch.distributed as dist
     from ssa_gym_b200 import env_config, _lib as F
@@ -297,6 +337,8 @@ def c3_measure(a, rank, local_rank, world, steps, warmup, gather):
     barrier()
     t_wall = time.perf_counter() - tw0
     clocks = sampler.stop()
+    if dump_dir and rank == 0:
+        write_outputs(dump_dir, {"obs": obs, "reward": r, "done": d})
     ms = e0.elapsed_time(e1)
     launches = env.ukf.launch_count - launches0
     nw = world if multi else 1
@@ -526,7 +568,7 @@ def main():
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
     try:
         if a.workload == "c3":
-            line = c3_measure(a, rank, local_rank, world, a.steps, a.warmup, a.gather)
+            line = c3_measure(a, rank, local_rank, world, a.steps, a.warmup, a.gather, a.dump_outputs)
             if rank == 0:
                 if a.collector == "mlp":
                     line["extra"]["ppo_collector_on_device"] = c3_collector_measure(a, local_rank, a.steps, a.warmup)
@@ -662,6 +704,8 @@ def run_catalog(a, rank, local_rank, world):
         evs.append((e0, e1))
     barrier()
     t_wall = time.perf_counter() - t_wall0
+    if a.dump_outputs and rank == 0:   # before the profiling and e2e passes below advance the state further
+        dump_catalog_outputs(a.dump_outputs, ukf, gathered)
     step_ms = [e0.elapsed_time(e1) for e0, e1 in evs]
     total_ms = float(np.sum(step_ms))
     launches = ukf.launch_count - launches0

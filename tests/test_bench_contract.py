@@ -41,6 +41,13 @@ def test_gpus_flag_must_match_the_launch():
     assert out.returncode != 0 and "torch.distributed.run" in (out.stderr + out.stdout)
 
 
+def test_steps_and_dump_arguments_are_checked():
+    out = _run("--steps", "0")
+    assert out.returncode != 0 and "--steps must be at least 1" in out.stderr
+    out = _run("--impl", "reference", "--dump-outputs", "unused")
+    assert out.returncode != 0 and "--dump-outputs" in out.stderr
+
+
 def test_c4_shards_are_slices_of_one_catalog():
     """Strong scaling: the job's inputs must not depend on the number of ranks."""
     from ssa_gym_b200.dist import shard_bounds
@@ -70,9 +77,16 @@ def test_catalog_layout_and_bookkeeping_constants():
 
 
 @pytest.mark.gpu
-def test_bench_line_carries_the_contract():
-    out = _run("--steps", "3", "--warmup", "3", "--objects", "60000", "--cpu-seconds", "1", timeout=900)
+def test_bench_line_carries_the_contract(tmp_path):
+    out = _run("--steps", "3", "--warmup", "3", "--objects", "60000", "--cpu-seconds", "1", "--dump-outputs", str(tmp_path), timeout=900)
     assert out.returncode == 0, out.stderr[-800:]
+    dump = {f[:-4]: np.load(tmp_path / f) for f in os.listdir(tmp_path)}
+    shapes = {"x_true": (60000, 6), "x_filter": (60000, 6), "P_filter": (60000, 6, 6), "obs": (60000, 12), "delta_pos": (60000,),
+              "delta_vel": (60000,), "sigma_pos": (60000,), "sigma_vel": (60000,), "trace": (60000,), "status": (60000,),
+              "inflations": (60000,), "catalog_stats": (1, 5)}
+    assert {k: v.shape for k, v in dump.items()} == shapes and all(v.dtype == np.float64 for v in dump.values())
+    assert np.isfinite(dump["x_filter"]).all() and dump["catalog_stats"][0, 2] == 60000
+    assert dump["catalog_stats"][0, 0] == dump["delta_pos"].max()
     d = json.loads(out.stdout.strip().splitlines()[-1])
     assert BASE_KEYS | {"cpu_baseline"} <= set(d), BASE_KEYS - set(d)
     assert d["unit"] == "object-updates/s" and d["higher_is_better"] is True and d["scaling"] == "strong" and d["dtype"] == "f64"
