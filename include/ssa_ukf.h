@@ -116,7 +116,13 @@ enum ssa_field {
 #define SSA_TASKER_SHANNON 5          /* argmax log(det P_i / det P_{i-1}) over visible objects   agents.py:15-26 */
 #define SSA_N_TASKERS 6
 /* a visible-* tasker returns -1 when the reference would fall back to action_space.sample()
- * (`not np.any(visible)` — also true when the only visible index is 0, agents.py:37).            */
+ * (`not np.any(visible)` — also true when the only visible index is 0, agents.py:37).
+ * SSA_TASKER_SHANNON keeps a determinant history per environment, keyed to the step index i the reduction runs at
+ * (ssa_ukf_env_reduce's step_index or SSA_F_STEP_INDEX; the episodic mode's own counters): at a LARGER i than the
+ * stored one the ratio is det P / det P of the stored step, which then becomes the history; at the SAME i it is
+ * evaluated against the same previous determinant again and nothing moves, so repeated calls at one step give the
+ * same picks; at i = 0, a smaller i, or with no history (after ssa_ukf_reset) the history restarts with ratio 1 and
+ * the first visible object is picked.                                                                                */
 
 /* flags for ssa_ukf_step */
 #define SSA_STEP_TRUTH 0x1        /* propagate the true states (SS2:265-266) */
@@ -236,7 +242,7 @@ int ssa_ukf_update(ssa_ukf* h, const double M[9], int all, void* stream); /* upd
 
 /* per-environment reductions: reward / done (SS2:324-354) and the greedy taskers (agents.py).
  * step_index = i after the increment of SS2:259; a negative step_index selects the uploaded per-env
- * SSA_F_STEP_INDEX table.  'shaped' rewards need the reward history: the device returns ENV_STATS and the
+ * SSA_F_STEP_INDEX table.  The step index also keys SSA_TASKER_SHANNON's determinant history (see there).  'shaped' rewards need the reward history: the device returns ENV_STATS and the
  * host finishes them (SS2:339-351).                                                                       */
 int ssa_ukf_env_reduce(ssa_ukf* h, const double M[9], int step_index, void* stream);
 /* reward.py score terms from the current covariances: out double[N][6] =

@@ -11,7 +11,9 @@ work that has to match exactly:
   * "no candidate" is tested as `not np.any(indices)` (agents.py:37) - the INDEX array, so the case "only object 0
     is visible" also counts as empty and a random action is sampled.
 The arrays read here (`env.P_filter[env.i]`, `env.delta_pos`, ...) were produced by the GPU step.  For vectorised
-environments the four argmax rules run on the device (`ssa_ukf_env_reduce`, SSA_TASKER_*), see vec_env.py.
+environments the argmax rules run on the device (`ssa_ukf_env_reduce`, SSA_TASKER_*), see vec_env.py; there
+agent_shannon's P_{i-1} is the covariance of the previous step index the reduction ran at, and a fresh episode (step 0)
+gets ratio 1 everywhere, as the reference's zeroed history row gives equal ratios.
 """
 import numpy as np
 

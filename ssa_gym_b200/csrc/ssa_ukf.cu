@@ -138,6 +138,7 @@ __global__ void __launch_bounds__(kCtaThreads) ssa_step_kernel(const KParams p) 
   const int team = threadIdx.x >> 4;
   const long obj = (long)blockIdx.x * kTeamsPerCta + team;
   if (obj >= p.N) return;  // a team leaves together
+  if (p.env_gate && !p.env_gate[obj / p.m]) return;  // (one object per team: the team leaves together)
   double* ws = ws_all + team * kWsStride;
   const int flags = p.flags;
   const long ld = p.ld;
@@ -1027,8 +1028,12 @@ struct EnvParams {
   int greedy_only;  // refresh greedy / env_stats only (after an auto-reset); reward and done stay
   const double* P; long ld;   // packed covariances (agent_shannon: determinants)
   const double* det_cur;      // [N] det P of the current covariances (ssa_det_kernel, thread per object)
-  double* det_prev;           // [N] det P of the previous call (P_filter[i-1] of agents.py:24)
-  const uint8_t* reset_mask;  // episodic refresh after an auto-reset: only these environments restart their det history
+  // agent_shannon's determinant history, keyed to the step index (see SSA_TASKER_SHANNON in ssa_ukf.h): det_last holds
+  // det P of step det_step[e], det_prev the denominator of that step's ratio (det P of the step before it)
+  double* det_prev;           // [N]
+  double* det_last;           // [N]
+  int32_t* det_step;          // [E] step index det_last belongs to (< 0: no history, ssa_ukf_reset)
+  const uint8_t* reset_mask;  // episodic refresh after an auto-reset: only these environments are re-evaluated
 };
 
 
@@ -1083,22 +1088,33 @@ __device__ __forceinline__ void env_reduce_body(const EnvParams& p, const int e)
   ArgMax a_trace{0.0, -1}, a_vtrace{0.0, -1}, a_vdpos{0.0, -1}, a_vdvel{0.0, -1}, a_spos{0.0, -1}, a_dpos{0.0, -1};
   ArgMax a_vaer{0.0, -1}, a_vshan{0.0, -1};
   int tri = 0, nvis = 0, vis_nonzero = 0;
-  const bool restart = p.greedy_only && (!p.reset_mask || p.reset_mask[e]);  // fresh episode: no previous covariance yet
+  int step_i = p.step_index >= 0 ? p.step_index : p.step_idx[e];
+  if (p.increment) step_i += 1;
+  // agent_shannon's history: a later step than the stored one shifts it, the same step re-reads it (so that calling
+  // the reduction again at one step gives the same picks), and step 0, an earlier step or no history restart it
+  const int hist = p.det_step[e];
+  const bool restart = step_i <= 0 || hist < 0 || step_i < hist, shift = !restart && step_i > hist;
   for (int j = j0; j < p.m; j += jstep) {
     const double dp = p.dpos[base + j], dv = p.dvel[base + j], sp = p.spos[base + j], tr = p.trace[base + j];
     const int vis = p.visible[base + j];
-    // agent_shannon (agents.py:15-26): log(det P_i / det P_{i-1}); the first call of an episode has no P_{i-1} (the
+    // agent_shannon (agents.py:15-26): log(det P_i / det P_{i-1}); the first step of an episode has no P_{i-1} (the
     // reference reads row -1 of its history array there): the ratio is taken as 1
-    double shan = 0.0;
-    if (p.det_prev && !(p.greedy_only && !restart)) {
-      // (det_cur null: the determinant is evaluated here — the RL-sized environments, one lane per object — instead of
-      // by ssa_det_kernel: one launch fewer per episodic step)
-      const double det = p.det_cur ? p.det_cur[base + j] : ssa_det6_sym(p.P + base + j, p.ld);
-      double prev = p.det_prev[base + j];
-      if (restart || prev != prev) prev = det;  // (NaN = never set: ssa_ukf_reset)
-      shan = ssa_log(ssa_div(det, prev));
+    // (det_cur null: the determinant is evaluated here — the RL-sized environments, one lane per object — instead of
+    // by ssa_det_kernel: one launch fewer per episodic step)
+    const double det = p.det_cur ? p.det_cur[base + j] : ssa_det6_sym(p.P + base + j, p.ld);
+    double prev;
+    if (restart) {
+      prev = det;
       p.det_prev[base + j] = det;
+      p.det_last[base + j] = det;
+    } else if (shift) {
+      prev = p.det_last[base + j];
+      p.det_prev[base + j] = prev;
+      p.det_last[base + j] = det;
+    } else {
+      prev = p.det_prev[base + j];
     }
+    const double shan = ssa_log(ssa_div(det, prev));
     if (vis) {
       // agent_visible_greedy_aer (agents.py:57-63): the 'aer' observation's trace column after nan_to_num (SS2:839)
       const double tr_aer = (tr - tr == 0.0) ? tr : 0.001;
@@ -1149,8 +1165,8 @@ __device__ __forceinline__ void env_reduce_body(const EnvParams& p, const int e)
     }
     const int c0 = WARP ? (int)(threadIdx.x >> 5) : 0;  // column of the per-environment results
     const double max_dpos = sm[5][c0].v;
-    int step_i = p.step_index >= 0 ? p.step_index : p.step_idx[e];
-    if (p.increment) { step_i += 1; p.step_idx[e] = step_i; }
+    if (p.increment) p.step_idx[e] = step_i;
+    p.det_step[e] = step_i;
     // `if not np.any(visible)` tests the INDEX array: it is also false-y when the only visible
     // object is index 0 (agents.py:37) -> the reference samples a random action; we return -1.
     const int any_vis = si[2][c0];
@@ -1159,7 +1175,7 @@ __device__ __forceinline__ void env_reduce_body(const EnvParams& p, const int e)
     p.greedy[e * SSA_N_TASKERS + SSA_TASKER_POS_ERROR_GREEDY] = any_vis ? sm[2][c0].i : -1;
     p.greedy[e * SSA_N_TASKERS + SSA_TASKER_VEL_ERROR_GREEDY] = any_vis ? sm[3][c0].i : -1;
     p.greedy[e * SSA_N_TASKERS + SSA_TASKER_VISIBLE_GREEDY_AER] = any_vis ? sm[6][c0].i : -1;
-    if (!(p.greedy_only && !restart)) p.greedy[e * SSA_N_TASKERS + SSA_TASKER_SHANNON] = any_vis ? sm[7][c0].i : -1;
+    p.greedy[e * SSA_N_TASKERS + SSA_TASKER_SHANNON] = any_vis ? sm[7][c0].i : -1;
     const double trinary = ((double)si[0][c0] / (double)p.m) / 2.0;
     p.env_stats[e * 4 + 0] = max_dpos;
     p.env_stats[e * 4 + 1] = trinary;
@@ -1650,13 +1666,14 @@ struct ssa_ukf {
   long launches;
   // one slab for all fp64 SoA state
   double* slab;
-  double *xt, *x, *P, *dpos, *dvel, *spos, *svel, *trace, *det_prev, *det_cur;
+  double *xt, *x, *P, *dpos, *dvel, *spos, *svel, *trace, *det_prev, *det_last, *det_cur;
   double *obs, *z_noise, *z_true, *y, *S, *sigmas_h, *scores, *reward, *env_stats;
   double* stage;  // staging for AoS<->SoA conversion ([N][39] doubles)
   double* qr;     // packed Q (21) + R (9)
   double* scratch;  // U[21] F[78] ZS[39] UVW[39] ZT[3] rows of ld doubles
   double* Menv;     // [E][9]
   int32_t* step_idx;  // [E]
+  int32_t* det_step;  // [E] (EnvParams::det_step)
   int32_t *code, *exc;
   long chunk;     // objects per chunk of the split pipeline (scratch capacity); N when everything fits in L2
   long staged_max;  // chunks up to this many objects use the TMA-staged k_update (default: all)
@@ -1761,7 +1778,7 @@ int ssa_ukf_create(const ssa_ukf_cfg* cfg, int device, ssa_ukf** out) {
   h->ld = (N + 31) / 32 * 32;
   const long ld = h->ld;
   // fp64 slab: xt 6, x 6, P 21, dpos dvel spos svel trace 5 (SoA rows of ld) + AoS outputs
-  const size_t n_soa = (size_t)(6 + 6 + 21 + 5 + 2) * ld;
+  const size_t n_soa = (size_t)(6 + 6 + 21 + 5 + 3) * ld;
   const size_t n_aos = (size_t)N * (12 + 3 + 3 + 3 + 9 + 39 + 6 + 2) + (size_t)E * (1 + 4 + 9) + 32;
   cudaError_t e = cudaMalloc(&h->slab, (n_soa + n_aos) * sizeof(double));
   if (e != cudaSuccess) { delete h; return set_err("cudaMalloc(slab)", e); }
@@ -1772,6 +1789,7 @@ int ssa_ukf_create(const ssa_ukf_cfg* cfg, int device, ssa_ukf** out) {
   h->P = q; q += 21 * ld;
   h->dpos = q; q += ld; h->dvel = q; q += ld; h->spos = q; q += ld; h->svel = q; q += ld; h->trace = q; q += ld;
   h->det_prev = q; q += ld;
+  h->det_last = q; q += ld;
   h->det_cur = q; q += ld;
   h->obs = q; q += N * 12;
   h->z_noise = q; q += N * 3;
@@ -1795,17 +1813,19 @@ int ssa_ukf_create(const ssa_ukf_cfg* cfg, int device, ssa_ukf** out) {
   }
   h->stage_bytes = (size_t)N * 39 * sizeof(double);
   if ((e = cudaMalloc(&h->stage, h->stage_bytes)) != cudaSuccess) { ssa_ukf_destroy(h); return set_err("cudaMalloc(stage)", e); }
-  if ((e = cudaMalloc(&h->status, sizeof(int32_t) * (4 * ld + 2 * E + E * SSA_N_TASKERS))) != cudaSuccess) {
+  if ((e = cudaMalloc(&h->status, sizeof(int32_t) * (4 * ld + 3 * E + E * SSA_N_TASKERS))) != cudaSuccess) {
     ssa_ukf_destroy(h);
     return set_err("cudaMalloc(int)", e);
   }
-  cudaMemset(h->status, 0, sizeof(int32_t) * (4 * ld + 2 * E + E * SSA_N_TASKERS));
+  cudaMemset(h->status, 0, sizeof(int32_t) * (4 * ld + 3 * E + E * SSA_N_TASKERS));
   h->infl = h->status + ld;
   h->code = h->infl + ld;
   h->exc = h->code + ld;
   h->actions = h->exc + ld;
   h->greedy = h->actions + E;
   h->step_idx = h->greedy + E * SSA_N_TASKERS;
+  h->det_step = h->step_idx + E;
+  cudaMemset(h->det_step, 0xFF, sizeof(int32_t) * E);  // -1: no determinant history yet
   // Scratch of the split pipeline is sized for one CHUNK of objects (180 doubles = 1.44 KB per object); batches
   // larger than the chunk run chunk by chunk.  Measured on B200 with 1 M objects: L2-sized chunks (24 k..196 k
   // objects) are SLOWER than one pass (2.4-4.0 ms vs 2.16 ms per step) — the per-launch tails cost more than the
@@ -1922,7 +1942,7 @@ int ssa_ukf_reset(ssa_ukf* h, const double* x_true, const double* x_filter, cons
   CK(cudaGetLastError());
   CK(cudaMemsetAsync(h->status, 0, sizeof(int32_t) * 2 * h->ld, st));
   CK(cudaMemsetAsync(h->visible, 0, 2 * h->ld, st));
-  CK(cudaMemsetAsync(h->det_prev, 0xFF, sizeof(double) * h->ld, st));  // NaN: no previous covariance yet (agent_shannon)
+  CK(cudaMemsetAsync(h->det_step, 0xFF, sizeof(int32_t) * h->cfg.n_envs, st));  // -1: no previous covariance yet (agent_shannon)
   CK(cudaStreamSynchronize(st));
   return SSA_OK;
 }
@@ -2441,8 +2461,8 @@ static void rollout_env_params(ssa_ukf* h, EnvParams* p, int increment, int gree
   p->env_stats = h->env_stats;
   p->E = h->cfg.n_envs; p->m = h->cfg.m; p->reward_type = h->cfg.reward_type; p->n_steps = h->cfg.n_steps;
   p->step_index = -1; p->step_idx = h->step_idx; p->increment = increment; p->greedy_only = greedy_only;
-  p->P = h->P; p->ld = h->ld; p->det_prev = h->det_prev; p->det_cur = h->det_cur;
-  p->reset_mask = nullptr;
+  p->P = h->P; p->ld = h->ld; p->det_prev = h->det_prev; p->det_last = h->det_last; p->det_step = h->det_step;
+  p->det_cur = h->det_cur; p->reset_mask = nullptr;
 }
 
 static void launch_env_reduce(ssa_ukf* h, const EnvParams& ep, cudaStream_t st) {
@@ -2711,7 +2731,8 @@ int ssa_ukf_env_reduce(ssa_ukf* h, const double M[9], int step_index, void* stre
   p.step_index = step_index;
   p.step_idx = h->step_idx;
   p.increment = 0; p.greedy_only = 0;
-  p.P = h->P; p.ld = h->ld; p.det_prev = h->det_prev; p.det_cur = h->det_cur; p.reset_mask = nullptr;
+  p.P = h->P; p.ld = h->ld; p.det_prev = h->det_prev; p.det_last = h->det_last; p.det_step = h->det_step;
+  p.det_cur = h->det_cur; p.reset_mask = nullptr;
   launch_env_reduce(h, p, st);
   CK(cudaGetLastError());
   return SSA_OK;

@@ -250,8 +250,8 @@ SSA_HD double ssa_nis3(const double* S, const double* y, int* flags) {
 // Determinant of a packed symmetric 6x6 (agent_shannon, agents.py:24: np.linalg.det(P)).  numpy factors with a pivoted
 // LU; for the symmetric (normally positive definite) covariances of the path the unpivoted symmetric elimination
 // P = L D L^T is just as stable, needs half the arithmetic and keeps its 21 entries in registers with static indices:
-// det = prod d_j.  The value agrees with LAPACK's to rounding (the tasker's argmax is compared with numpy up to ties
-// inside 1e-9 in tests/test_gpu_vs_oracle.py).  A zero pivot returns 0.
+// det = prod d_j.  Against exact rational determinants it is as close as LAPACK's (tests/test_det_exact.py).  A zero
+// pivot returns 0.
 SSA_HD double ssa_det6_sym(const double* P, long stride) {
   double a[SSA_NP];
 #pragma unroll

@@ -167,6 +167,9 @@ class VecSSATaskerEnv:
     def _epilogue_only(self):
         self.ukf.upload(F.F_TRANS_ENV, self.trans_matrix[self.i])
         self.ukf.step(None, F.STEP_EPILOGUE | F.STEP_M_PER_ENV)
+        # greedy taskers of the fresh state; agent_shannon's history of a re-drawn environment starts at its P0 (step 0)
+        self.ukf.upload(F.F_STEP_INDEX, self.i)
+        self.ukf.env_reduce(step_index=-1)
 
     def reset_at(self, e):
         """Reset environment e only (device state of the other environments is untouched)."""

@@ -316,3 +316,276 @@ class TwinBackedUKF:
 
     def close(self):
         pass
+
+
+# ---- agent_shannon and the per-environment reductions in the device's arithmetic ---------------------------------
+def twin_det6(P):
+    """ssa_det6_sym of each covariance (full [N,6,6] or packed [N,21]) through the host twin: bit-equal to the device."""
+    P = np.asarray(P, dtype=np.float64)
+    Pp = np.ascontiguousarray(pack_P(P) if P.shape[-2:] == (6, 6) else P.reshape(-1, 21))
+    out = np.empty(len(Pp))
+    twin().twin_det6_sym(p(Pp), p(out), len(Pp))
+    return out
+
+
+def twin_log_ratio(det, prev):
+    """ssa_log(ssa_div(det, prev)) elementwise (numpy's log is not bit-equal to ssa_log, test_math_accuracy.py)."""
+    det = np.ascontiguousarray(det, dtype=np.float64)
+    prev = np.ascontiguousarray(np.broadcast_to(prev, det.shape), dtype=np.float64)
+    out = np.empty_like(det)
+    twin().twin_log_ratio(p(det), p(prev), p(out), det.size)
+    return out
+
+
+class ShannonHistory:
+    """The determinant history of SSA_TASKER_SHANNON (include/ssa_ukf.h) for E environments of m objects: `last` is
+    det P at step `step[e]`, `prev` the denominator of that step's ratio.  A larger step shifts the history, the same
+    step re-reads it, step 0 / a smaller step / no history (step -1) restarts it with ratio 1."""
+
+    def __init__(self, E, m):
+        self.E, self.m = E, m
+        self.prev, self.last = np.zeros((E, m)), np.zeros((E, m))
+        self.step = np.full(E, -1, np.int64)
+
+    def scores(self, P, steps, sel=None):
+        """log(det P / det P_prev) [E, m] at the per-env step indices `steps`; only the environments in `sel` (bool
+        [E], default all) are evaluated and move their history, the others' rows are NaN."""
+        E, m = self.E, self.m
+        sel = np.ones(E, bool) if sel is None else np.asarray(sel, bool)
+        steps = np.asarray(steps, dtype=np.int64)
+        det = twin_det6(P).reshape(E, m)
+        restart = (steps <= 0) | (self.step < 0) | (steps < self.step)
+        shift = ~restart & (steps > self.step)
+        prev = np.where(restart[:, None], det, np.where(shift[:, None], self.last, self.prev))
+        last = np.where(restart[:, None] | shift[:, None], det, self.last)
+        out = np.full((E, m), np.nan)
+        out[sel] = twin_log_ratio(det[sel], prev[sel])
+        self.prev[sel], self.last[sel], self.step[sel] = prev[sel], last[sel], steps[sel]
+        return out
+
+
+def first_visible_argmax(score, vis):
+    """The visible-* rule of ssa_env_reduce_kernel for one environment: the first maximum of `score` among the visible
+    objects, a NaN score ordered like +inf (np.argmax: NaN wins); -1 where agents.py:37 `not np.any(idx)` samples."""
+    idx = np.where(vis)[0]
+    if not np.any(idx):
+        return -1
+    s = np.asarray(score, dtype=np.float64)[idx]
+    return int(idx[np.argmax(np.where(np.isnan(s), np.inf, s))])
+
+
+def emu_env_reduce(st, E, m, step_idx, reward_type, n_steps, shannon=None, sel=None):
+    """numpy restatement of ssa_env_reduce_kernel (SS2:324-354, agents.py:7-81) on twin outputs.  `shannon` is the
+    ShannonHistory that the call advances (its column stays -1 without one); `sel` restricts the Shannon history to
+    the environments a refresh re-evaluates."""
+    dpos = st.dpos.reshape(E, m); dvel = st.dvel.reshape(E, m); tr = st.trace.reshape(E, m)
+    vis = st.visible.reshape(E, m).astype(bool)
+    max_dpos = dpos.max(1)
+    tri = ((dpos < 1e4).astype(int) + (dpos < 1e7).astype(int)).sum(1)
+    trinary = (tri.astype(float) / float(m)) / 2.0
+    reward = np.zeros(E); done = np.zeros(E, bool)
+    if reward_type == "jones":
+        hi, lo = max_dpos > 5e6, max_dpos < 3e4
+        done |= hi | lo
+        reward[lo & ~hi] = 1.0
+    else:
+        reward = trinary
+    done |= (np.asarray(step_idx) + 1 >= n_steps)
+    greedy = np.full((E, _lib.N_TASKERS), -1, np.int32)
+    greedy[:, _lib.TASKER_NAIVE_GREEDY] = tr.argmax(1)
+    sh = shannon.scores(st.P, step_idx, sel) if shannon is not None else None
+    for e in range(E):
+        greedy[e, _lib.TASKER_VISIBLE_GREEDY] = first_visible_argmax(tr[e], vis[e])
+        greedy[e, _lib.TASKER_POS_ERROR_GREEDY] = first_visible_argmax(dpos[e], vis[e])
+        greedy[e, _lib.TASKER_VEL_ERROR_GREEDY] = first_visible_argmax(dvel[e], vis[e])
+        greedy[e, _lib.TASKER_VISIBLE_GREEDY_AER] = first_visible_argmax(
+            np.nan_to_num(tr[e], nan=0.001, posinf=0.001, neginf=0.001), vis[e])
+        if sh is not None:
+            greedy[e, _lib.TASKER_SHANNON] = first_visible_argmax(sh[e], vis[e])
+    return reward, done, greedy
+
+
+_REFRESHED = ("obs", "dpos", "dvel", "spos", "svel", "trace", "visible", "updated")
+
+
+class EpisodicTwin:
+    """Step-by-step host statement of the device-resident episodic mode (ssa_ukf_rollout_reset / ssa_ukf_rollout_step)
+    of a VecSSATaskerEnv(rng='device'): the same counter-based draws (twin_env_reset / twin_env_noise), twin_step with
+    the env's trans_matrix row, numpy reward / done / greedy taskers including agent_shannon's determinant history.
+    After an auto-reset only the re-drawn environments are refreshed: the others keep this step's outputs."""
+
+    def __init__(self, vec, cfg):
+        self.E, self.m, self.n = vec.E, vec.m, vec.n
+        self.N = self.E * self.m
+        self.reward_type, self.update_interval = cfg["reward_type"], cfg["update_interval"]
+        self.keys = np.array(vec.init_seeds, dtype=np.uint64)
+        self.table = np.ascontiguousarray(vec.trans_matrix).reshape(self.n, 9)
+        self.sig = np.concatenate([vec.x_sigma, vec.z_sigma, vec.P_0[np.triu_indices(6)]])
+        self.orbits = np.ascontiguousarray(vec.orbits, dtype=np.float64)
+        self.cfg = make_cfg(self.N, E=self.E, m=self.m, dt=cfg["time_step"], alpha=cfg["alpha"], beta=cfg["beta"],
+                            kappa=cfg["kappa"], q_sigma=cfg["q_sigma"], R=vec.R, observer_deg=cfg["observer"],
+                            obs_limit_deg=cfg["obs_limit"], n_steps=self.n)
+        self.episode = np.zeros(self.E, np.uint32)
+        self.step_idx = np.zeros(self.E, np.int32)
+        self.shannon = ShannonHistory(self.E, self.m)
+        self.st = None
+
+    def _draw(self, done):
+        N, tw = self.N, twin()
+        xt, xf, Pp = np.zeros((N, 6)), np.zeros((N, 6)), np.zeros((N, 21))
+        status, infl = np.zeros(N, np.int32), np.zeros(N, np.int32)
+        d8 = None if done is None else np.ascontiguousarray(done, dtype=np.uint8)
+        tw.twin_env_reset(self.E, self.m, p(self.keys), p(self.episode), p(self.step_idx), p(d8), p(self.orbits),
+                          len(self.orbits), p(self.sig), p(xt), p(xf), p(Pp), p(status), p(infl))
+        if self.st is None:
+            self.st = HostState(xt, xf, unpack_P(Pp))
+            return
+        rows = np.repeat(np.asarray(done, bool), self.m)
+        st = self.st
+        st.x_true[rows] = xt[rows]; st.x[rows] = xf[rows]; st.P[rows] = unpack_P(Pp)[rows]
+        st.status[rows] = 0; st.infl[rows] = 0
+
+    def _refresh(self, envs):
+        """obs / errors / visibility of the fresh objects of `envs` (bool [E]) and their greedy taskers."""
+        st, rows = self.st, np.repeat(envs, self.m)
+        keep = {k: getattr(st, k).copy() for k in _REFRESHED}
+        cpu_step("twin", self.cfg, st, self.table[np.minimum(self.step_idx, self.n - 1)].reshape(self.E, 9),
+                 _lib.STEP_EPILOGUE | _lib.STEP_M_PER_ENV)
+        for k, v in keep.items():
+            getattr(st, k)[~rows] = v[~rows]
+        _, _, g = emu_env_reduce(st, self.E, self.m, self.step_idx, self.reward_type, self.n, self.shannon, envs)
+        self.greedy[envs] = g[envs]
+
+    def reset(self):
+        """rollout_reset: every environment drawn, step index 0; returns obs [N, 12] and greedy [E, taskers]."""
+        self._draw(None)
+        self.greedy = np.full((self.E, _lib.N_TASKERS), -1, np.int32)
+        self._refresh(np.ones(self.E, bool))
+        return self.st.obs.copy(), self.greedy.copy()
+
+    def step(self, actions, auto_reset=True):
+        """rollout_step; returns obs [N, 12], reward [E], done [E], greedy [E, taskers] as the device's output block."""
+        E, m, st = self.E, self.m, self.st
+        zn = np.zeros((self.N, 3))
+        twin().twin_env_noise(E, m, p(self.keys), p(self.episode), p(self.step_idx), p(self.sig), p(zn))
+        nxt = self.step_idx + 1
+        a_eff = np.where(nxt % self.update_interval == 0, actions, -1).astype(np.int32)
+        cpu_step("twin", self.cfg, st, self.table[np.minimum(nxt, self.n - 1)].reshape(E, 9),
+                 _lib.STEP_TRUTH | _lib.STEP_PREDICT | _lib.STEP_UPDATE_ACT | _lib.STEP_EPILOGUE | _lib.STEP_M_PER_ENV,
+                 actions=a_eff, z_noise=zn)
+        self.step_idx[:] = nxt
+        reward, done, self.greedy = emu_env_reduce(st, E, m, self.step_idx, self.reward_type, self.n, self.shannon)
+        if auto_reset and done.any():
+            self._draw(done)
+            self._refresh(done)
+        return st.obs.copy(), reward, done, self.greedy.copy()
+
+
+def episodic_vs_twin(cfg, E, total_steps, seed0=500, action_seed=11):
+    """Run VecSSATaskerEnv(cfg, E, rng='device') and EpisodicTwin side by side (actions alternate between random and
+    the device's visible-greedy picks) and demand equality at every step: observations, rewards, dones and all six
+    greedy columns exact, vec.i equal to the step counters; at the end x, x_true, P, status, inflation counts, updated
+    and visible.  Returns counters of what the run went through (auto-resets, environments with nothing / only
+    object 0 visible after a step)."""
+    from ssa_gym_b200.vec_env import VecSSATaskerEnv
+    vec = VecSSATaskerEnv(cfg, E, seeds=list(range(seed0, seed0 + E)), rng="device")
+    emu = EpisodicTwin(vec, cfg)
+    E, m, N = emu.E, emu.m, emu.N
+    obs_e, g_e = emu.reset()
+    assert bits_equal(vec.obs.reshape(N, 12), obs_e)
+    assert np.array_equal(vec._io["greedy"], g_e), (vec._io["greedy"], g_e)
+    rng = np.random.RandomState(action_seed)
+    seen = {"resets": 0, "none_visible": 0, "only_object_0": 0}
+    for t in range(total_steps):
+        a = vec.greedy_actions(_lib.TASKER_VISIBLE_GREEDY) if t % 2 else rng.randint(0, m, size=E)
+        a = np.asarray(a, dtype=np.int32)
+        obs_v, r_v, d_v, _ = vec.vector_step(a)
+        obs_e, r_e, d_e, g_e = emu.step(a)
+        assert np.array_equal(d_v, d_e), (t, d_v, d_e)
+        assert bits_equal(r_v, r_e), (t, r_v, r_e)
+        assert bits_equal(obs_v.reshape(N, 12), obs_e), t
+        g_v = vec._io["greedy"]
+        for k in range(_lib.N_TASKERS):
+            assert np.array_equal(g_v[:, k], g_e[:, k]), (t, k, np.where(g_v[:, k] != g_e[:, k])[0], g_v[:, k], g_e[:, k])
+        assert np.array_equal(vec.i, emu.step_idx), t
+        vis = emu.st.visible.reshape(E, m).astype(bool)
+        seen["resets"] += int(d_e.sum())
+        seen["none_visible"] += int((~vis.any(1)).sum())
+        seen["only_object_0"] += int((vis[:, 0] & ~vis[:, 1:].any(1)).sum())
+    st, u = emu.st, vec.ukf
+    assert bits_equal(u.download(_lib.F_X_FILTER), st.x) and bits_equal(u.download(_lib.F_X_TRUE), st.x_true)
+    assert bits_equal(pack_P(u.download(_lib.F_P_FILTER)), pack_P(st.P))
+    for f, a in ((_lib.F_STATUS, st.status), (_lib.F_INFLATIONS, st.infl), (_lib.F_UPDATED, st.updated),
+                 (_lib.F_VISIBLE, st.visible)):
+        assert np.array_equal(u.download(f).reshape(a.shape), a), f
+    vec.close()
+    return seen
+
+
+def scores_det_restated(P):
+    """score_det_P and score_det_pos_P of ssa_scores_kernel restated in its operation order (plain IEEE double
+    operations, the library is built with -fmad=false): the 3x3 cofactor formula of the position block and a 6x6
+    Gaussian elimination with partial pivoting.  Bit-equal to the device; returns (det6 [N], det3 [N])."""
+    P = np.asarray(P, dtype=np.float64).reshape(-1, 6, 6)
+    det6, det3 = np.empty(len(P)), np.empty(len(P))
+    for n in range(len(P)):
+        a = [[float(P[n][min(i, j)][max(i, j)]) for j in range(6)] for i in range(6)]  # the upper triangle, mirrored
+        m00, m01, m02, m11, m12, m22 = a[0][0], a[0][1], a[0][2], a[1][1], a[1][2], a[2][2]
+        det3[n] = m00 * (m11 * m22 - m12 * m12) - m01 * (m01 * m22 - m12 * m02) + m02 * (m01 * m12 - m11 * m02)
+        det = 1.0
+        for c in range(6):
+            pv = c
+            for i in range(c + 1, 6):
+                if abs(a[i][c]) > abs(a[pv][c]):
+                    pv = i
+            if pv != c:
+                a[c], a[pv] = a[pv], a[c]
+                det = -det
+            det *= a[c][c]
+            if a[c][c] == 0.0:
+                break
+            rp = 1.0 / a[c][c]
+            for i in range(c + 1, 6):
+                lf = a[i][c] * rp
+                for j in range(c + 1, 6):
+                    a[i][j] -= lf * a[c][j]
+        det6[n] = det
+    return det6, det3
+
+
+def exact_det(A):
+    """Exact determinant (fractions.Fraction) of a square float matrix: every double is an exact rational."""
+    from fractions import Fraction
+    a = [[Fraction(float(v)) for v in row] for row in np.asarray(A)]
+    n, det = len(a), Fraction(1)
+    for c in range(n):
+        pv = next((r for r in range(c, n) if a[r][c] != 0), None)
+        if pv is None:
+            return Fraction(0)
+        if pv != c:
+            a[c], a[pv] = a[pv], a[c]
+            det = -det
+        det *= a[c][c]
+        for r in range(c + 1, n):
+            lf = a[r][c] / a[c][c]
+            if lf:
+                for k in range(c, n):
+                    a[r][k] -= lf * a[c][k]
+    return det
+
+
+def rel_err_exact(value, exact):
+    """|value - exact| / |exact| computed exactly, rounded once to float (0 / inf when exact is 0)."""
+    from fractions import Fraction
+    if exact == 0:
+        return 0.0 if value == 0 else np.inf
+    if not np.isfinite(value):
+        return np.inf
+    return float(abs(Fraction(float(value)) - exact) / abs(exact))
+
+
+def corr_cond(P):
+    """Condition number of the correlation matrices of P [N, k, k] (scale-free conditioning of a determinant)."""
+    P = np.asarray(P, dtype=np.float64)
+    d = np.sqrt(np.abs(np.einsum("nii->ni", P)))
+    return np.linalg.cond(P / (d[:, :, None] * d[:, None, :]))

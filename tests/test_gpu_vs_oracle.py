@@ -91,7 +91,8 @@ def test_fused_step_c2_against_oracle():
 
 def test_env_reduce_and_scores():
     """Per-environment reductions (reward/done, greedy taskers) against numpy on the downloaded arrays: integer
-    outputs bit-exact incl. first-maximum ties and the `np.any(visible)` index-0 quirk; reward.py terms."""
+    outputs bit-exact incl. first-maximum ties and the `np.any(visible)` index-0 quirk, agent_shannon against the twin
+    emulation of its determinant history (repeated calls at one step index give the same picks); reward.py terms."""
     E, m = 257, 10
     N = E * m
     cat, x, P0, zn = H.c2_inputs(N, 3)
@@ -102,22 +103,30 @@ def test_env_reduce_and_scores():
         for s in range(3):
             ukf.upload(F.F_ACTIONS, rng.randint(0, m, E).astype(np.int32)); ukf.upload(F.F_Z_NOISE, zn[s])
             ukf.step(H.CEL2TER06AXY, F.STEP_TRUTH | F.STEP_PREDICT | F.STEP_UPDATE_ACT | F.STEP_EPILOGUE)
-        P_prev = ukf.download(F.F_P_FILTER).reshape(E, m, 6, 6)
+        hist = H.ShannonHistory(E, m)    # agent_shannon's determinant history in the device's arithmetic
         ukf.env_reduce(step_index=3)     # first call: no previous covariance -> every log-determinant ratio is 0
         g0 = ukf.download(F.F_GREEDY)
         vis0 = ukf.download(F.F_VISIBLE).reshape(E, m).astype(bool)
+        sh0 = hist.scores(ukf.download(F.F_P_FILTER), np.full(E, 3))
+        assert np.all(sh0 == 0.0)
         for e in range(E):
             v = np.where(vis0[e])[0]
             assert g0[e, F.TASKER_SHANNON] == (v[0] if np.any(v) else -1)
+        ukf.env_reduce(step_index=3)     # again at the same step: the same picks
+        assert np.array_equal(ukf.download(F.F_GREEDY), g0)
         for s in range(3, 5):
             ukf.upload(F.F_ACTIONS, rng.randint(0, m, E).astype(np.int32)); ukf.upload(F.F_Z_NOISE, zn[s % 3])
             ukf.step(H.CEL2TER06AXY, F.STEP_TRUTH | F.STEP_PREDICT | F.STEP_UPDATE_ACT | F.STEP_EPILOGUE)
+        ukf.env_reduce(step_index=5)     # the ratio is between the two steps the reduction ran at (3 and 5)
+        g5 = ukf.download(F.F_GREEDY)
         ukf.env_reduce(step_index=5)
         ukf.sync()
+        assert np.array_equal(ukf.download(F.F_GREEDY), g5)
         dpos, dvel, tr = (ukf.download(f).reshape(E, m) for f in (F.F_DELTA_POS, F.F_DELTA_VEL, F.F_TRACE))
         vis = ukf.download(F.F_VISIBLE).reshape(E, m).astype(bool)
         greedy, rew, done = ukf.download(F.F_GREEDY), ukf.download(F.F_REWARD), ukf.download(F.F_DONE)
         P = ukf.download(F.F_P_FILTER).reshape(E, m, 6, 6)
+        sh = hist.scores(P, np.full(E, 5))
         for e in range(E):
             assert greedy[e, F.TASKER_NAIVE_GREEDY] == np.argmax([np.trace(Pj) for Pj in P[e]])
             v = np.where(vis[e])[0]
@@ -129,15 +138,9 @@ def test_env_reduce_and_scores():
                 assert greedy[e, F.TASKER_VEL_ERROR_GREEDY] == v[np.argmax(dvel[e, v])]
                 # agent_visible_greedy_aer (agents.py:57-63): the 'aer' observation's trace column after nan_to_num
                 assert greedy[e, F.TASKER_VISIBLE_GREEDY_AER] == v[np.argmax(np.nan_to_num(tr[e, v], nan=0.001, posinf=0.001, neginf=0.001))]
-                # agent_shannon (agents.py:15-26): argmax log(det P_i / det P_{i-1}); the determinants come from an LU with
-                # partial pivoting on both sides but not from the same BLAS: equal up to ties inside 1e-9
-                with np.errstate(divide="ignore", invalid="ignore"):
-                    sc = np.array([np.log(np.linalg.det(P[e, j]) / np.linalg.det(P_prev[e, j])) for j in v])
-                pick = list(v).index(greedy[e, F.TASKER_SHANNON])
-                if np.isnan(sc).any():
-                    assert np.isnan(sc[pick])          # np.argmax: the first NaN wins
-                else:
-                    assert sc[pick] >= np.max(sc) - 1e-9 * max(1.0, abs(np.max(sc))), (e, sc, pick)
+                # agent_shannon (agents.py:15-26): argmax log(det P_5 / det P_3) in the device's arithmetic, exact
+                # (ssa_det6_sym against exact determinants: tests/test_det_exact.py)
+                assert greedy[e, F.TASKER_SHANNON] == H.first_visible_argmax(sh[e], vis[e]), (e, sh[e], vis[e])
             if reward_type == "trinary":
                 assert rew[e] == np.mean(((dpos[e] < 1e4) * 1 + (dpos[e] < 1e7) * 1)) / 2 and done[e] == 0
             else:
@@ -147,6 +150,10 @@ def test_env_reduce_and_scores():
         if reward_type == "jones":
             from oracle import dynamics_restated as D
             sc = ukf.scores().reshape(E, m, 6)
+            # the determinant columns: bit-equal to the restatement of ssa_scores_kernel, which
+            # tests/test_det_exact.py bounds against exact determinants
+            det6, det3 = H.scores_det_restated(P.reshape(N, 6, 6))
+            assert H.bits_equal(sc[:, :, 3].ravel(), det6) and H.bits_equal(sc[:, :, 4].ravel(), det3)
             for e in range(0, E, 37):
                 for j in range(m):
                     assert np.isclose(sc[e, j, 0], D.score_scaled_trace_P(P[e, j]), rtol=1e-14)

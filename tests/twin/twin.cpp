@@ -256,6 +256,14 @@ void twin_robust_chol(const double* P, double lam, double* U, int32_t* ret, int 
 void twin_inv3(const double* S, double* SI, int32_t* ok, int n) {
   for (int i = 0; i < n; ++i) ok[i] = ssa_inv3(S + 9 * i, SI + 9 * i);
 }
+// determinants of packed symmetric 6x6 matrices [n][21] (agent_shannon: ssa_env_reduce_kernel / ssa_det_kernel)
+void twin_det6_sym(const double* P, double* out, int n) {
+  for (int i = 0; i < n; ++i) out[i] = ssa_det6_sym(P + 21 * (size_t)i, 1);
+}
+// agent_shannon's score log(det / prev) in the device's arithmetic
+void twin_log_ratio(const double* det, const double* prev, double* out, int n) {
+  for (int i = 0; i < n; ++i) out[i] = ssa_log(ssa_div(det[i], prev[i]));
+}
 #define TW1(name, fn) \
   void name(const double* x, double* y, int n) { for (int i = 0; i < n; ++i) y[i] = fn(x[i]); }
 TW1(twin_sin, ssa_sin) TW1(twin_cos, ssa_cos) TW1(twin_tan, ssa_tan) TW1(twin_atan, ssa_atan)
