@@ -104,6 +104,7 @@ enum ssa_field {
   SSA_F_ROLLOUT_ACTIONS = 31, /* int32 [E]: the device-side action buffer read by ssa_ukf_rollout_step(.., auto_reset | 2, ..) */
   SSA_F_ROLLOUT_DONE = 32,    /* uint8 [E]  and                                                                    */
   SSA_F_ROLLOUT_GREEDY = 33,  /* int32 [E][SSA_N_TASKERS] of the episodic output block                             */
+  SSA_F_ROLLOUT_OBS_AER = 34, /* double [N][4]: the episodic mode's 'aer' observation block (SSA_ROLLOUT_OBS_AER)     */
   SSA_F_COUNT_
 };
 
@@ -206,12 +207,16 @@ int ssa_ukf_host_stats(ssa_ukf* h, int parity, double** stats_host, double** sta
  * z_noise[i], update_interval gate SS2:292, reward / done SS2:324-354) and the auto-reset of finished episodes.
  * Random numbers are counter-based (Philox4x32-10 keyed by the environment's seed, addressed by episode / object /
  * step - csrc/ssa_rng.h): same distributions as the reference, NOT the same streams as its np_random (the host-RNG
- * path ssa_ukf_reset + ssa_ukf_step keeps stream parity).  'shaped' rewards are not available here.
+ * path ssa_ukf_reset + ssa_ukf_step keeps stream parity).  All three reward types: for 'shaped' (SS2:339-351) the
+ * handle keeps each environment's reward history [E][n_steps] and the argmax sigma_pos of its previous step on the
+ * device; the history sum 1 - np.sum(rewards[:i]) of a success is evaluated in numpy's pairwise order, and the action
+ * compared with that argmax is the requested one, also on steps that update_interval skips.
  *   rollout_config  catalog [n_orbits][6], trans_matrix table [n_table][9] (row i = step i), one 64-bit seed per env,
  *                   x_sigma[6], z_sigma[3] (radians / metres), P0[36], update_interval
  *   rollout_io      pinned host blocks owned by the handle: actions [E] (in); obs [N][12], reward [E],
  *                   greedy [E][SSA_N_TASKERS], done [E] (out)
- *   rollout_reset   draw every environment, step index 0; outputs: obs, greedy
+ *   rollout_reset   draw every environment, step index 0; outputs: obs, greedy, and the 'aer' block of
+ *                   ssa_ukf_rollout_obs_aer
  *   rollout_step    one step of every environment with the actions in the pinned block: ONE H2D copy, ONE CUDA-graph
  *                   launch (noise, the five UKF kernels, reward / done, reset of the finished environments and their
  *                   fresh obs when auto_reset, greedy taskers of the new state), ONE D2H copy.  Asynchronous on
@@ -231,9 +236,18 @@ int ssa_ukf_rollout_reset(ssa_ukf* h, void* stream);
  * 48 N bytes (+ the reward / greedy / done tail) instead of 96 N — for a learner that casts its observations to float32
  * anyway (RLlib's preprocessors do, rl_agents/RLLib_PPO_training.py).  The float64 rows stay valid on the device.    */
 #define SSA_ROLLOUT_OBS_F32 4
+/* bit 3 (SSA_ROLLOUT_OBS_AER): the reference's 'aer' observation layout (SS2:834-840): the last kernel of the step's
+ * graph writes [az, el, range] of every filter mean x[0..2] (through the environment's trans_matrix row
+ * min(step index, n_table - 1), after an auto-reset that of the new episode's step 0), then np.trace of its diag P
+ * columns summed left to right, each of the four with NaN / +-inf replaced by 0.001, into [N][4] doubles; the D2H copy
+ * moves those 32 N bytes (+ the reward / greedy / done tail) instead of 96 N.  Not combinable with SSA_ROLLOUT_OBS_F32
+ * (SSA_EINVAL).  The float64 rows stay valid on the device.                                                         */
+#define SSA_ROLLOUT_OBS_AER 8
 int ssa_ukf_rollout_step(ssa_ukf* h, int auto_reset, void* stream);
 /* the float32 observation blocks of SSA_ROLLOUT_OBS_F32: pinned host mirror and device block, [N][12] floats          */
 int ssa_ukf_rollout_obs_f32(ssa_ukf* h, float** host, float** device);
+/* the 'aer' observation blocks of SSA_ROLLOUT_OBS_AER: pinned host mirror and device block, [N][4] doubles           */
+int ssa_ukf_rollout_obs_aer(ssa_ukf* h, double** host, double** device);
 /* make `stream` wait for every outstanding internal copy of ssa_ukf_step_host / ssa_ukf_step_pinned */
 int ssa_ukf_host_join(ssa_ukf* h, void* stream);
 /* Convenience wrappers with the reference's call structure */
@@ -243,7 +257,7 @@ int ssa_ukf_update(ssa_ukf* h, const double M[9], int all, void* stream); /* upd
 /* per-environment reductions: reward / done (SS2:324-354) and the greedy taskers (agents.py).
  * step_index = i after the increment of SS2:259; a negative step_index selects the uploaded per-env
  * SSA_F_STEP_INDEX table.  The step index also keys SSA_TASKER_SHANNON's determinant history (see there).  'shaped' rewards need the reward history: the device returns ENV_STATS and the
- * host finishes them (SS2:339-351).                                                                       */
+ * host finishes them (SS2:339-351); the episodic mode keeps that history on the device instead (ssa_ukf_rollout_*).                                                                       */
 int ssa_ukf_env_reduce(ssa_ukf* h, const double M[9], int step_index, void* stream);
 /* reward.py score terms from the current covariances: out double[N][6] =
  * [score_scaled_trace_P, score_trace_P, score_scaled_det_P(dt), score_det_P, score_det_pos_P, |dpos|] */

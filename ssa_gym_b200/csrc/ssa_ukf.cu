@@ -1034,6 +1034,10 @@ struct EnvParams {
   double* det_last;           // [N]
   int32_t* det_step;          // [E] step index det_last belongs to (< 0: no history, ssa_ukf_reset)
   const uint8_t* reset_mask;  // episodic refresh after an auto-reset: only these environments are re-evaluated
+  // episodic mode with the 'shaped' reward (null otherwise: the host finishes that reward from env_stats)
+  double* rew_hist;           // [E][n_steps] rewards of the running episode, entry 0 = 0 (np.sum(rewards[:i]), SS2:345)
+  int32_t* spos_prev;         // [E] argmax sigma_pos of the environment's previous step (SS2:348)
+  const int32_t* act_in;      // [E] REQUESTED actions (SS2:348 compares them also on steps update_interval skips)
 };
 
 
@@ -1124,7 +1128,9 @@ __device__ __forceinline__ void env_reduce_body(const EnvParams& p, const int e)
       a_vshan = am_better(a_vshan, ArgMax{sh, j});
     }
     a_trace = am_better(a_trace, ArgMax{tr, j});
-    a_spos = am_better(a_spos, ArgMax{sp, j});
+    // sigma_pos = sqrt of a sum of covariance diagonal entries: NaN if update() left a negative one (only x is checked
+    // for NaN there); np.argmax (the 'shaped' reward, SS2:348) orders a NaN first, as the Shannon column does
+    a_spos = am_better(a_spos, ArgMax{(sp == sp) ? sp : ssa_from_hilo(0x7ff00000, 0), j});
     a_dpos = am_better(a_dpos, ArgMax{dp, j});
     if (vis) {
       a_vtrace = am_better(a_vtrace, ArgMax{tr, j});
@@ -1190,6 +1196,16 @@ __device__ __forceinline__ void env_reduce_body(const EnvParams& p, const int e)
       else if (step_i + 1 >= p.n_steps) { done = 1; reward = 0.0; }
     } else if (p.reward_type == SSA_REWARD_TRINARY) {  // SS2:337-338
       reward = trinary;
+    } else if (p.rew_hist) {  // 'shaped' in the episodic mode (SS2:339-351, episode.py step_reward)
+      double* hist = p.rew_hist + (long)e * p.n_steps;
+      if (max_dpos > 5e6) { done = 1; reward = 0.0; }
+      else if (max_dpos < 3e4) { done = 1; reward = 1.0 - ssa_pairwise_sum(hist, step_i < p.n_steps ? step_i : p.n_steps); }
+      else {
+        const double r = ssa_div(1.0, (double)p.n_steps);
+        reward = (p.act_in[e] == p.spos_prev[e]) ? r : -r;
+      }
+      if (step_i < p.n_steps) hist[step_i] = reward;  // (without auto-reset an episode may run past its last step)
+      p.spos_prev[e] = sm[4][c0].i;
     } else {  // 'shaped' needs the reward history: finished on the host from env_stats (SS2:339-351)
       if (max_dpos > 5e6) { done = 1; reward = 0.0; }
       else if (max_dpos < 3e4) { done = 1; reward = 1.0; }
@@ -1212,7 +1228,8 @@ struct RolloutParams {
   const int32_t* actions; int32_t* act_eff;   // [E] requested / effective (update_interval) actions
   const uint8_t* done;                        // [E] reset mask (null: every environment)
   const double* sig;                          // x_sigma[6], z_sigma[3], packed P0[21]
-  int E, m, update_interval;
+  double* rew_hist; int32_t* spos_prev;       // 'shaped' reward state (EnvParams), null for the other rewards
+  int E, m, update_interval, n_steps;
 };
 
 // start of a step: measurement noise of step i+1 for every object, effective action of every environment
@@ -1257,6 +1274,10 @@ __device__ __forceinline__ void env_reset_body(const RolloutParams& p, const int
   if (threadIdx.x == 0) {
     p.episode[e] = ep + 1u;
     p.step_idx[e] = 0;
+    if (p.rew_hist) {  // a new episode: rewards[0] = 0 (entries 1 .. i-1 are written by its steps before any read) and
+      p.rew_hist[(long)e * p.n_steps] = 0.0;  // the argmax of its all-equal sigma_pos[0] (vec_env.py host mode: 0)
+      p.spos_prev[e] = 0;
+    }
   }
 }
 
@@ -1729,8 +1750,11 @@ struct ssa_ukf {
     int32_t* hin;        // pinned host actions [E]
     size_t out_bytes;
     float *dobs32, *hobs32;    // SSA_ROLLOUT_OBS_F32: obs [N][12] as floats (device block, pinned host mirror)
-    cudaGraphExec_t gexec[4];  // [auto_reset + 2 * obs_f32]
-    int gkernels[4];
+    double *daer, *haer;       // SSA_ROLLOUT_OBS_AER: the 'aer' observation [N][4] (device block, pinned host mirror)
+    double* rew_hist;          // 'shaped' only: [E][n_steps] reward history, then spos_prev [E] int32
+    int32_t* spos_prev;
+    cudaGraphExec_t gexec[6];  // [auto_reset + 2 * (obs_f32 ? 1 : obs_aer ? 2 : 0)]
+    int gkernels[6];
   } ro;
   int32_t *status, *infl, *actions, *greedy;
   uint8_t *visible, *updated, *innov_flags, *done;
@@ -1897,8 +1921,9 @@ int ssa_ukf_destroy(ssa_ukf* h) {
   for (int i = 0; i < h->sg.n; ++i) { cudaGraphExecDestroy(h->sg.gexec[i]); cudaGraphDestroy(h->sg.graph[i]); }
   if (h->ro.init) {
     cudaFree(h->ro.dbuf); cudaFree(h->ro.ibuf); cudaFree(h->ro.dout); cudaFree(h->ro.dobs32);
-    cudaFreeHost(h->ro.hout); cudaFreeHost(h->ro.hin); cudaFreeHost(h->ro.hobs32);
-    for (int i = 0; i < 4; ++i) if (h->ro.gexec[i]) cudaGraphExecDestroy(h->ro.gexec[i]);
+    cudaFree(h->ro.daer); cudaFree(h->ro.rew_hist);
+    cudaFreeHost(h->ro.hout); cudaFreeHost(h->ro.hin); cudaFreeHost(h->ro.hobs32); cudaFreeHost(h->ro.haer);
+    for (int i = 0; i < 6; ++i) if (h->ro.gexec[i]) cudaGraphExecDestroy(h->ro.gexec[i]);
   }
   cudaFree(h->snap);
   cudaFree(h->cat_part);
@@ -1997,6 +2022,9 @@ static int field_info(ssa_ukf* h, int field, void** p, size_t* bytes, int* soa_c
       if (!h->ro.init) { snprintf(g_err, sizeof(g_err), "episodic mode not configured"); return SSA_EINVAL; }
       *p = (uint8_t*)((int32_t*)(h->ro.dout + 12 * N + E) + SSA_N_TASKERS * E); *bytes = E; break;
     case SSA_F_INNOV_FLAGS: *p = h->innov_flags; *bytes = N; break;
+    case SSA_F_ROLLOUT_OBS_AER:
+      if (!h->ro.init) { snprintf(g_err, sizeof(g_err), "episodic mode not configured"); return SSA_EINVAL; }
+      *p = h->ro.daer; *bytes = N * 4 * 8; break;
     default: snprintf(g_err, sizeof(g_err), "unknown field %d", field); return SSA_EINVAL;
   }
   return SSA_OK;
@@ -2449,7 +2477,8 @@ static void rollout_params(ssa_ukf* h, RolloutParams* p, int only_done) {
   const size_t N = h->cfg.n_objects, E = h->cfg.n_envs;
   p->done = only_done ? (const uint8_t*)((int32_t*)(h->ro.dout + 12 * N + E) + SSA_N_TASKERS * E) : nullptr;
   p->sig = h->ro.sig;
-  p->E = h->cfg.n_envs; p->m = h->cfg.m; p->update_interval = h->ro.update_interval;
+  p->rew_hist = h->ro.rew_hist; p->spos_prev = h->ro.spos_prev;
+  p->E = h->cfg.n_envs; p->m = h->cfg.m; p->update_interval = h->ro.update_interval; p->n_steps = h->cfg.n_steps;
 }
 
 static void rollout_env_params(ssa_ukf* h, EnvParams* p, int increment, int greedy_only) {
@@ -2463,6 +2492,7 @@ static void rollout_env_params(ssa_ukf* h, EnvParams* p, int increment, int gree
   p->step_index = -1; p->step_idx = h->step_idx; p->increment = increment; p->greedy_only = greedy_only;
   p->P = h->P; p->ld = h->ld; p->det_prev = h->det_prev; p->det_last = h->det_last; p->det_step = h->det_step;
   p->det_cur = h->det_cur; p->reset_mask = nullptr;
+  p->rew_hist = h->ro.rew_hist; p->spos_prev = h->ro.spos_prev; p->act_in = h->ro.act_in;
 }
 
 static void launch_env_reduce(ssa_ukf* h, const EnvParams& ep, cudaStream_t st) {
@@ -2498,17 +2528,14 @@ int ssa_ukf_rollout_config(ssa_ukf* h, const double* orbits, int n_orbits, const
                            int update_interval) {
   if (!h || !orbits || n_orbits < 1 || !trans_table || n_table < 1 || !seeds || !x_sigma || !z_sigma || !P0 || update_interval < 1)
     return SSA_EINVAL;
-  if (h->cfg.reward_type == SSA_REWARD_SHAPED) {
-    snprintf(g_err, sizeof(g_err), "episodic device mode: the 'shaped' reward needs the host-side reward history");
-    return SSA_EINVAL;
-  }
   CK(cudaSetDevice(h->device));
   const size_t N = h->cfg.n_objects, E = h->cfg.n_envs;
   // (the cached graphs of ssa_ukf_step stay valid: every pointer they captured belongs to the handle)
   if (h->ro.init) {
     cudaFree(h->ro.dbuf); cudaFree(h->ro.ibuf); cudaFree(h->ro.dout); cudaFreeHost(h->ro.hout); cudaFreeHost(h->ro.hin);
     cudaFree(h->ro.dobs32); cudaFreeHost(h->ro.hobs32);
-    for (int i = 0; i < 4; ++i) if (h->ro.gexec[i]) { cudaGraphExecDestroy(h->ro.gexec[i]); h->ro.gexec[i] = nullptr; }
+    cudaFree(h->ro.daer); cudaFreeHost(h->ro.haer); cudaFree(h->ro.rew_hist);
+    for (int i = 0; i < 6; ++i) if (h->ro.gexec[i]) { cudaGraphExecDestroy(h->ro.gexec[i]); h->ro.gexec[i] = nullptr; }
     h->ro.init = 0;
   }
   h->ro.n_orbits = n_orbits; h->ro.n_table = n_table; h->ro.update_interval = update_interval;
@@ -2537,7 +2564,18 @@ int ssa_ukf_rollout_config(ssa_ukf* h, const double* orbits, int n_orbits, const
   CK(cudaMemset(h->ro.dobs32, 0, sizeof(float) * 12 * N));
   CK(cudaHostAlloc(&h->ro.hobs32, sizeof(float) * 12 * N, cudaHostAllocDefault));
   memset(h->ro.hobs32, 0, sizeof(float) * 12 * N);
-  for (int i = 0; i < 4; ++i) h->ro.gexec[i] = nullptr;
+  CK(cudaMalloc(&h->ro.daer, sizeof(double) * 4 * N));
+  CK(cudaMemset(h->ro.daer, 0, sizeof(double) * 4 * N));
+  CK(cudaHostAlloc(&h->ro.haer, sizeof(double) * 4 * N, cudaHostAllocDefault));
+  memset(h->ro.haer, 0, sizeof(double) * 4 * N);
+  h->ro.rew_hist = nullptr; h->ro.spos_prev = nullptr;
+  if (h->cfg.reward_type == SSA_REWARD_SHAPED) {  // the reward history lives on the device (env_reset_body clears it)
+    const size_t hist = sizeof(double) * E * (size_t)h->cfg.n_steps;
+    CK(cudaMalloc(&h->ro.rew_hist, hist + sizeof(int32_t) * E));
+    CK(cudaMemset(h->ro.rew_hist, 0, hist + sizeof(int32_t) * E));
+    h->ro.spos_prev = (int32_t*)((char*)h->ro.rew_hist + hist);
+  }
+  for (int i = 0; i < 6; ++i) h->ro.gexec[i] = nullptr;
   h->ro.init = 1;
   return SSA_OK;
 }
@@ -2553,6 +2591,8 @@ int ssa_ukf_rollout_io(ssa_ukf* h, int32_t** actions, double** obs, double** rew
   return SSA_OK;
 }
 
+static void launch_obs_aer(ssa_ukf* h, cudaStream_t st);
+
 int ssa_ukf_rollout_reset(ssa_ukf* h, void* stream) {
   if (!h || !h->ro.init) return SSA_EINVAL;
   CK(cudaSetDevice(h->device));
@@ -2563,7 +2603,9 @@ int ssa_ukf_rollout_reset(ssa_ukf* h, void* stream) {
   h->launches++;
   int rc = rollout_refresh(h, st, 0);
   if (rc) return rc;
+  launch_obs_aer(h, st);  // (the 'aer' rows of the fresh episodes, whichever layout the steps will use)
   CK(cudaMemcpyAsync(h->ro.hout, h->ro.dout, h->ro.out_bytes, cudaMemcpyDeviceToHost, st));
+  CK(cudaMemcpyAsync(h->ro.haer, h->ro.daer, sizeof(double) * 4 * h->cfg.n_objects, cudaMemcpyDeviceToHost, st));
   CK(cudaGetLastError());
   return SSA_OK;
 }
@@ -2603,7 +2645,37 @@ __global__ void __launch_bounds__(256) k_obs_to_f32(const double2* __restrict__ 
   }
 }
 
-static int rollout_chain(ssa_ukf* h, cudaStream_t st, int auto_reset, int obs_f32) {
+// SSA_ROLLOUT_OBS_AER: the 'aer' observation of every object (SS2:834-840, vec_env.py _format_obs), one thread per object:
+// az / el / range of the filter mean x[0..2] through the environment's trans_matrix row min(step_idx, n_table - 1) (its
+// row of the step just taken, step 0 after a re-draw), np.trace's left-to-right sum of the diag P columns, and
+// nan_to_num(nan = +-inf = 0.001) of the four values.
+__global__ void __launch_bounds__(128) k_obs_aer(const double* __restrict__ obs, const int32_t* __restrict__ step_idx,
+                                                 const double* __restrict__ table, int n_table, const ssa_obs ob, int m, long N,
+                                                 double* __restrict__ out) {
+  const long n = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (n >= N) return;
+  const int i = step_idx[n / m];
+  const double* o = obs + n * 12;
+  double x[3], v[4];
+#pragma unroll
+  for (int k = 0; k < 3; ++k) x[k] = o[k];
+  ssa_hx_aer_m<false>(x, table + (long)(i < n_table - 1 ? i : n_table - 1) * 9, ob.obs_itrs, ob.T, v);
+  v[3] = ((((o[6] + o[7]) + o[8]) + o[9]) + o[10]) + o[11];
+#pragma unroll
+  for (int k = 0; k < 4; ++k) out[n * 4 + k] = (v[k] - v[k] == 0.0) ? v[k] : 0.001;
+}
+
+static void launch_obs_aer(ssa_ukf* h, cudaStream_t st) {
+  ssa_obs ob;
+  memcpy(ob.obs_itrs, h->cfg.obs_itrs, sizeof(ob.obs_itrs));
+  memcpy(ob.T, h->cfg.T, sizeof(ob.T));
+  const long N = h->cfg.n_objects;
+  k_obs_aer<<<(unsigned)((N + 127) / 128), 128, 0, st>>>(h->ro.dout, h->step_idx, h->ro.table, h->ro.n_table, ob, h->cfg.m, N,
+                                                         h->ro.daer);
+  h->launches++;
+}
+
+static int rollout_chain(ssa_ukf* h, cudaStream_t st, int auto_reset, int obs_f32, int obs_aer) {
   RolloutParams rp;
   rollout_params(h, &rp, 1);
   const long N = h->cfg.n_objects;
@@ -2637,6 +2709,14 @@ static int rollout_chain(ssa_ukf* h, cudaStream_t st, int auto_reset, int obs_f3
     k_obs_to_f32<<<(unsigned)((n2 + 255) / 256), 256, 0, st>>>((const double2*)h->ro.dout, (float2*)h->ro.dobs32, n2);
     h->launches++;
   }
+  if (obs_aer) launch_obs_aer(h, st);
+  return SSA_OK;
+}
+
+int ssa_ukf_rollout_obs_aer(ssa_ukf* h, double** host, double** device) {
+  if (!h || !h->ro.init) return SSA_EINVAL;
+  if (host) *host = h->ro.haer;
+  if (device) *device = h->ro.daer;
   return SSA_OK;
 }
 
@@ -2652,9 +2732,13 @@ int ssa_ukf_rollout_step(ssa_ukf* h, int auto_reset, void* stream) {
   CK(cudaSetDevice(h->device));
   cudaStream_t st = (cudaStream_t)stream;
   const size_t E = h->cfg.n_envs;
-  const bool obs_f32 = (auto_reset & SSA_ROLLOUT_OBS_F32) != 0;
+  const bool obs_f32 = (auto_reset & SSA_ROLLOUT_OBS_F32) != 0, obs_aer = (auto_reset & SSA_ROLLOUT_OBS_AER) != 0;
+  if (obs_f32 && obs_aer) {
+    snprintf(g_err, sizeof(g_err), "SSA_ROLLOUT_OBS_F32 and SSA_ROLLOUT_OBS_AER exclude each other");
+    return SSA_EINVAL;
+  }
   const int ar = (auto_reset & 1) ? 1 : 0;
-  const int a = ar + (obs_f32 ? 2 : 0);
+  const int a = ar + (obs_f32 ? 2 : obs_aer ? 4 : 0);
   const bool device_io = (auto_reset & SSA_ROLLOUT_DEVICE_IO) != 0;
   if (!device_io) CK(cudaMemcpyAsync(h->ro.act_in, h->ro.hin, sizeof(int32_t) * E, cudaMemcpyHostToDevice, st));
   const char* gv = getenv("SSA_UKF_GRAPH");
@@ -2664,7 +2748,7 @@ int ssa_ukf_rollout_step(ssa_ukf* h, int auto_reset, void* stream) {
       CK(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
       const long l0 = h->launches;
       CK(cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal));
-      const int rc = rollout_chain(h, cs, ar, obs_f32);
+      const int rc = rollout_chain(h, cs, ar, obs_f32, obs_aer);
       cudaGraph_t g = nullptr;
       const cudaError_t ce = cudaStreamEndCapture(cs, &g);
       h->ro.gkernels[a] = (int)(h->launches - l0);
@@ -2679,13 +2763,17 @@ int ssa_ukf_rollout_step(ssa_ukf* h, int auto_reset, void* stream) {
     CK(cudaGraphLaunch(h->ro.gexec[a], st));
     h->launches += h->ro.gkernels[a];
   } else {
-    const int rc = rollout_chain(h, st, ar, obs_f32);
+    const int rc = rollout_chain(h, st, ar, obs_f32, obs_aer);
     if (rc) return rc;
   }
   if (!device_io) {
     if (obs_f32) {  // float observations + the reward / greedy / done tail of the double block
       const size_t N = h->cfg.n_objects;
       CK(cudaMemcpyAsync(h->ro.hobs32, h->ro.dobs32, sizeof(float) * 12 * N, cudaMemcpyDeviceToHost, st));
+      CK(cudaMemcpyAsync(h->ro.hout + 12 * N, h->ro.dout + 12 * N, h->ro.out_bytes - sizeof(double) * 12 * N, cudaMemcpyDeviceToHost, st));
+    } else if (obs_aer) {  // the 'aer' observations + the same tail
+      const size_t N = h->cfg.n_objects;
+      CK(cudaMemcpyAsync(h->ro.haer, h->ro.daer, sizeof(double) * 4 * N, cudaMemcpyDeviceToHost, st));
       CK(cudaMemcpyAsync(h->ro.hout + 12 * N, h->ro.dout + 12 * N, h->ro.out_bytes - sizeof(double) * 12 * N, cudaMemcpyDeviceToHost, st));
     } else {
       CK(cudaMemcpyAsync(h->ro.hout, h->ro.dout, h->ro.out_bytes, cudaMemcpyDeviceToHost, st));
@@ -2733,6 +2821,7 @@ int ssa_ukf_env_reduce(ssa_ukf* h, const double M[9], int step_index, void* stre
   p.increment = 0; p.greedy_only = 0;
   p.P = h->P; p.ld = h->ld; p.det_prev = h->det_prev; p.det_last = h->det_last; p.det_step = h->det_step;
   p.det_cur = h->det_cur; p.reset_mask = nullptr;
+  p.rew_hist = nullptr; p.spos_prev = nullptr; p.act_in = nullptr;  // 'shaped': finished on the host
   launch_env_reduce(h, p, st);
   CK(cudaGetLastError());
   return SSA_OK;

@@ -274,6 +274,57 @@ SSA_HD double ssa_det6_sym(const double* P, long stride) {
   return zero ? 0.0 : det;
 }
 
+// np.sum of a[0 .. n) (contiguous float64) in numpy's order: the 'shaped' reward's 1 - np.sum(rewards[:i]) (SS2:345),
+// where a sequential sum differs in the last bits for most prefix lengths.  numpy's pairwise_sum: a block of n < 8 is
+// summed sequentially from 0.0; a block of 8 <= n <= 128 in eight accumulators seeded with a[0..7] and advanced in
+// strides of 8, combined ((r0+r1)+(r2+r3))+((r4+r5)+(r6+r7)), its remainder added in order; a longer block is split at
+// n2 = n/2 - (n/2) % 8 and its two halves summed the same way and added.  The reduction adds the result to its 0.0
+// identity.  The recursion is walked with an explicit stack (no device recursion): a block of n <= 2^31 elements is
+// split at most 24 times before its halves reach 128.
+SSA_HD double ssa_pairwise_block(const double* a, long n) {
+  if (n < 8) {
+    double s = 0.0;
+    for (long i = 0; i < n; ++i) s = s + a[i];
+    return s;
+  }
+  double r[8];
+#pragma unroll
+  for (int j = 0; j < 8; ++j) r[j] = a[j];
+  long i = 8;
+  for (; i < n - (n % 8); i += 8) {
+#pragma unroll
+    for (int j = 0; j < 8; ++j) r[j] = r[j] + a[i + j];
+  }
+  double s = ((r[0] + r[1]) + (r[2] + r[3])) + ((r[4] + r[5]) + (r[6] + r[7]));
+  for (; i < n; ++i) s = s + a[i];
+  return s;
+}
+SSA_HD double ssa_pairwise_sum(const double* a, long n) {
+  double left[32];   // sum of the left half of each open split whose right half is being summed
+  long right[32];    // length of the right half of each open split (0 once it is being summed)
+  int top = 0;
+  long off = 0, len = n;
+  for (;;) {
+    while (len > 128) {  // descend into left halves
+      long n2 = len / 2;
+      n2 -= n2 % 8;
+      right[top] = len - n2;
+      ++top;
+      len = n2;
+    }
+    double s = ssa_pairwise_block(a + off, len);
+    off += len;
+    while (top > 0 && right[top - 1] == 0) {  // both halves of the innermost split are done
+      --top;
+      s = left[top] + s;
+    }
+    if (top == 0) return 0.0 + s;
+    left[top - 1] = s;  // a left half is done: sum the right one
+    len = right[top - 1];
+    right[top - 1] = 0;
+  }
+}
+
 // np.trace(P) over the packed diagonal, numpy's left-to-right order (agents.py:8,40)
 SSA_HD double ssa_trace6(const double* P, long stride) {
   double t = P[0];

@@ -105,6 +105,7 @@ class BatchedUKF:
             _lib.F_CATALOG_STATS: ((5,), np.float64), _lib.F_ROLLOUT_OBS: ((self.N, 12), np.float64),
             _lib.F_ROLLOUT_REWARD: ((self.n_envs,), np.float64), _lib.F_ROLLOUT_ACTIONS: ((self.n_envs,), np.int32),
             _lib.F_ROLLOUT_DONE: ((self.n_envs,), np.uint8), _lib.F_ROLLOUT_GREEDY: ((self.n_envs, _lib.N_TASKERS), np.int32),
+            _lib.F_ROLLOUT_OBS_AER: ((self.N, 4), np.float64),
         }
 
     # -- lifetime ---------------------------------------------------------------------------------
@@ -268,14 +269,20 @@ class BatchedUKF:
         _lib.check(self.lib.ssa_ukf_rollout_obs_f32(self.h, ctypes.byref(h32), ctypes.byref(d32)), "ssa_ukf_rollout_obs_f32")
         self.rollout_io["obs_f32"] = view(h32, ctypes.c_float, (N, 12))  # filled by rollout_step(obs_f32=True)
         self.rollout_obs_f32_device = d32.value
+        ha, da = ctypes.c_void_p(), ctypes.c_void_p()
+        _lib.check(self.lib.ssa_ukf_rollout_obs_aer(self.h, ctypes.byref(ha), ctypes.byref(da)), "ssa_ukf_rollout_obs_aer")
+        self.rollout_io["obs_aer"] = view(ha, ctypes.c_double, (N, 4))  # filled by rollout_reset and rollout_step(obs_aer=True)
         return self.rollout_io
 
     def rollout_reset(self, stream=None):
         _lib.check(self.lib.ssa_ukf_rollout_reset(self.h, stream), "ssa_ukf_rollout_reset")
 
-    def rollout_step(self, auto_reset=True, stream=None, device_io=False, obs_f32=False):
-        """obs_f32: the observations leave the device as float32 (rollout_io['obs_f32']; the float64 block is not copied)."""
-        mode = (1 if auto_reset else 0) | (_lib.ROLLOUT_DEVICE_IO if device_io else 0) | (_lib.ROLLOUT_OBS_F32 if obs_f32 else 0)
+    def rollout_step(self, auto_reset=True, stream=None, device_io=False, obs_f32=False, obs_aer=False):
+        """obs_f32: the observations leave the device as float32 (rollout_io['obs_f32']; the float64 block is not copied).
+        obs_aer: the step also computes the 'aer' observation [N, 4] (rollout_io['obs_aer'], device field F_ROLLOUT_OBS_AER),
+        which leaves the device instead of the float64 block.  The two exclude each other."""
+        mode = (1 if auto_reset else 0) | (_lib.ROLLOUT_DEVICE_IO if device_io else 0) | (_lib.ROLLOUT_OBS_F32 if obs_f32 else 0) | \
+            (_lib.ROLLOUT_OBS_AER if obs_aer else 0)
         _lib.check(self.lib.ssa_ukf_rollout_step(self.h, mode, stream), "ssa_ukf_rollout_step")
 
     @property

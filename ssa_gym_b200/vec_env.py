@@ -15,7 +15,10 @@ of finished episodes.  A vector_step is then one 4*E-byte upload, one CUDA-graph
 obs / reward / done / greedy (ssa_ukf_rollout_step).  Same distributions as the reference, NOT the same random
 streams: seed-for-seed episode parity with `SSA_Tasker_Env` holds only for `rng='host'`, whose reset has to draw
 n*m*3 + 7m numbers per environment from a sequential MT19937 stream on the host (measured at E = 4096: 102 ms per
-vector_step in host mode against 0.45 ms in device mode).
+vector_step in host mode against 0.45 ms in device mode).  The device mode covers the reference's whole configuration
+matrix: the 'shaped' reward keeps its per-environment reward history on the device (the episode's own 1 - np.sum(
+rewards[:i]) in numpy's summation order), and the 'aer' layout is computed by the last kernel of the step's graph, so
+only its [E, m*4] rows (32 B per object instead of 96) cross PCIe and the host formats nothing.
 """
 import numpy as np
 
@@ -89,9 +92,9 @@ class VecSSATaskerEnv:
         self._P0_packed = self.P_0[np.triu_indices(6)]
         self._views = None
         self.seed(seeds)
+        # device mode, 'aer': the observation rows are computed on the device (SSA_ROLLOUT_OBS_AER), not by _format_obs
+        self._obs_aer = rng == 'device' and self.obs_returned == 'aer'
         if self.rng == 'device':
-            if self.reward_type == 'shaped':
-                raise ValueError("rng='device' does not support the 'shaped' reward (host-side history); use rng='host'")
             keys = np.array([int(s_) & 0xFFFFFFFFFFFFFFFF for s_ in self.init_seeds], dtype=np.uint64)
             self._io = self.ukf.rollout_config(self.orbits, self.trans_matrix, keys, self.x_sigma, self.z_sigma, self.P_0,
                                                self.update_interval)
@@ -124,7 +127,8 @@ class VecSSATaskerEnv:
         """The per-env observation in the layout config['obs_returned'] asks for (SS2:355-361).  obs12 = [E', m*12] rows
         (x [6], diag P [6] per RSO) of the environments `idx` (default: all); 'aer' evaluates az / el / range of every
         filter mean on the device with the env's own trans_matrix[i] (SS2:834-840) — environments at the same step index
-        share one launch — and replaces NaN / inf by 0.001 as the reference does."""
+        share one launch — and replaces NaN / inf by 0.001 as the reference does.  (rng='device' computes the 'aer' rows
+        inside the step instead, k_obs_aer.)"""
         if self.obs_returned == 'flatten':
             return obs12
         o = np.asarray(obs12).reshape(-1, self.m, 12)
@@ -157,6 +161,8 @@ class VecSSATaskerEnv:
             self.ukf.rollout_reset()
             self.ukf.sync()
             self.i[:] = 0
+            if self._obs_aer:
+                return self._io["obs_aer"].reshape(self.E, self.m * 4)
             return self._format_obs(self._io["obs"].reshape(self.E, self.m * 12).astype(self.obs_dtype, copy=False))
         for e in range(self.E):
             self._draw(e)
@@ -244,7 +250,7 @@ class VecSSATaskerEnv:
         io = self._io
         io["actions"][:] = actions
         f32 = self.obs_dtype == np.float32
-        self.ukf.rollout_step(self.auto_reset, obs_f32=f32)
+        self.ukf.rollout_step(self.auto_reset, obs_f32=f32, obs_aer=self._obs_aer)
         self.ukf.sync()
         dones = io["done"].astype(bool)
         rewards = io["reward"].copy()
@@ -252,18 +258,24 @@ class VecSSATaskerEnv:
         if self.auto_reset:
             self.i[dones] = 0
             self.episodes[dones] += 1
-        self.obs = self._format_obs(io["obs_f32" if f32 else "obs"].reshape(self.E, self.m * 12))
+        if self._obs_aer:
+            self.obs = io["obs_aer"].reshape(self.E, self.m * 4)
+        else:
+            self.obs = self._format_obs(io["obs_f32" if f32 else "obs"].reshape(self.E, self.m * 12))
         return self.obs, self._format_reward(rewards), dones, self._infos  # E empty dicts, allocated once (4096 dict constructions cost 100 us)
 
     # -- device-resident consumer (a policy on the same GPU): no host copies, nothing synchronises -------------------
     def device_views(self):
         """Zero-copy torch tensors over the episodic mode's device buffers: 'actions' int32 [E] (INPUT of
-        vector_step_device), 'obs' float64 [E, m*12], 'reward' float64 [E], 'done' uint8 [E], 'greedy' int32 [E, taskers].
+        vector_step_device), 'obs' float64 [E, m*12] ([E, m*4] for obs_returned='aer'), 'reward' float64 [E], 'done' uint8
+        [E], 'greedy' int32 [E, taskers].
         The outputs are overwritten by every step; they are valid in stream order on the stream the step runs on."""
         assert self.rng == 'device', "device views exist in the device-resident episodic mode (rng='device')"
         if getattr(self, "_views", None) is None:
             u = self.ukf
-            self._views = {"actions": u.torch_view(F.F_ROLLOUT_ACTIONS), "obs": u.torch_view(F.F_ROLLOUT_OBS).view(self.E, self.m * 12),
+            obs = (u.torch_view(F.F_ROLLOUT_OBS_AER).view(self.E, self.m * 4) if self._obs_aer else
+                   u.torch_view(F.F_ROLLOUT_OBS).view(self.E, self.m * 12))
+            self._views = {"actions": u.torch_view(F.F_ROLLOUT_ACTIONS), "obs": obs,
                            "reward": u.torch_view(F.F_ROLLOUT_REWARD), "done": u.torch_view(F.F_ROLLOUT_DONE),
                            "greedy": u.torch_view(F.F_ROLLOUT_GREEDY)}
         return self._views
@@ -274,7 +286,7 @@ class VecSSATaskerEnv:
         no synchronisation (the reference hands every observation to the learner process through the host, SURVEY 3.4).
         The host mirrors (self.i, self.episodes) are not maintained in this mode."""
         assert self.rng == 'device'
-        self.ukf.rollout_step(self.auto_reset, stream=stream, device_io=True)
+        self.ukf.rollout_step(self.auto_reset, stream=stream, device_io=True, obs_aer=self._obs_aer)
         return self.device_views()
 
     # -- device taskers --------------------------------------------------------------------------------------
