@@ -105,6 +105,7 @@ enum ssa_field {
   SSA_F_ROLLOUT_DONE = 32,    /* uint8 [E]  and                                                                    */
   SSA_F_ROLLOUT_GREEDY = 33,  /* int32 [E][SSA_N_TASKERS] of the episodic output block                             */
   SSA_F_ROLLOUT_OBS_AER = 34, /* double [N][4]: the episodic mode's 'aer' observation block (SSA_ROLLOUT_OBS_AER)     */
+  SSA_F_ROLLOUT_EPISODE_STATS = 35, /* double [E][SSA_EPISODE_STATS_DOUBLES]: episode records (ssa_ukf_rollout_episode_stats_*) */
   SSA_F_COUNT_
 };
 
@@ -248,6 +249,32 @@ int ssa_ukf_rollout_step(ssa_ukf* h, int auto_reset, void* stream);
 int ssa_ukf_rollout_obs_f32(ssa_ukf* h, float** host, float** device);
 /* the 'aer' observation blocks of SSA_ROLLOUT_OBS_AER: pinned host mirror and device block, [N][4] doubles           */
 int ssa_ukf_rollout_obs_aer(ssa_ukf* h, double** host, double** device);
+/* Per-episode statistics of the episodic mode: each environment's return, length and filter-consistency figures
+ * (SS2:436-446 anees, SS2:564-569 NIS, SS2:598-604 innovation bounds, SS2:782-832 innovation_dw_test) accumulated inside
+ * the step graph, a few doubles per object instead of per-step histories.  Per environment over rows 0 .. L of an
+ * episode (L = the step index at which done is raised; row 0 = the fresh draw, before the first predict):
+ *   every row, every object: NEES of (x_true - x, P) as ssa_ukf_diagnostics evaluates it, NaN values left out;
+ *   steps 1 .. L, the tasked object when update_interval lets the step update it and it was updated: NIS (NaN left out),
+ *   the innovation-bound flags, and the Durbin-Watson state of the overall innovation series and of the object's own;
+ *   the sum of the step rewards of steps 1 .. L (the float64 reward of the output block).
+ * On a step whose done flag is set the environment's record is written; with auto-reset its accumulators are then
+ * cleared for the next episode, without auto-reset they keep running (the record of a finished environment is rewritten
+ * every step, covering the episode so far).  Record, SSA_EPISODE_STATS_DOUBLES doubles:
+ *   0 L | 1 return | 2 sum of the NEES values (per object in row order, then over objects in index order) | 3 their count
+ *   | 4 sum of the NIS values | 5 their count | 6 observations | 7-9 innovations inside 1 sigma per component | 10-12
+ *   inside 2 sigmas | 13-15 Durbin-Watson statistic of the overall series (NaN without an entry) | 16-18 minimum and
+ *   19-21 maximum of the per-object statistics over the objects with >= 2 entries (NaN if one of them is NaN or none
+ *   qualifies) | 22 objects in the failed state at the end.
+ *   enable    after ssa_ukf_rollout_config (which turns the statistics off again); allocates and clears the buffers, drops
+ *             the cached step graphs; accumulation starts with the next ssa_ukf_rollout_reset.  Each step then also
+ *             records y / S of the updated objects (SSA_STEP_RECORD) and runs two small kernels; without enable the step
+ *             graphs are unchanged.
+ *   download  the records of n environments envs[0..n) into out[n][SSA_EPISODE_STATS_DOUBLES]; blocks until copied.
+ *             SSA_EINVAL before enable.  The device block is SSA_F_ROLLOUT_EPISODE_STATS: the row of an environment is
+ *             valid, in stream order, after a step whose done flag is set for it.                                     */
+#define SSA_EPISODE_STATS_DOUBLES 23
+int ssa_ukf_rollout_episode_stats_enable(ssa_ukf* h);
+int ssa_ukf_rollout_episode_stats_download(ssa_ukf* h, const int32_t* envs, int n, double* out, void* stream);
 /* make `stream` wait for every outstanding internal copy of ssa_ukf_step_host / ssa_ukf_step_pinned */
 int ssa_ukf_host_join(ssa_ukf* h, void* stream);
 /* Convenience wrappers with the reference's call structure */

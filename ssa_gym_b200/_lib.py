@@ -27,10 +27,12 @@ N_TASKERS = 6
 (F_X_TRUE, F_X_FILTER, F_P_FILTER, F_OBS, F_DELTA_POS, F_DELTA_VEL, F_SIGMA_POS, F_SIGMA_VEL, F_TRACE,
  F_Z_TRUE, F_Y, F_S, F_SIGMAS_H, F_Z_NOISE, F_VISIBLE, F_STATUS, F_INFLATIONS, F_ACTIONS, F_REWARD, F_DONE,
  F_GREEDY, F_SCORES, F_UPDATED, F_TRANS_ENV, F_STEP_INDEX, F_ENV_STATS, F_DIAG, F_INNOV_FLAGS, F_CATALOG_STATS,
- F_ROLLOUT_OBS, F_ROLLOUT_REWARD, F_ROLLOUT_ACTIONS, F_ROLLOUT_DONE, F_ROLLOUT_GREEDY, F_ROLLOUT_OBS_AER) = range(35)
+ F_ROLLOUT_OBS, F_ROLLOUT_REWARD, F_ROLLOUT_ACTIONS, F_ROLLOUT_DONE, F_ROLLOUT_GREEDY, F_ROLLOUT_OBS_AER,
+ F_ROLLOUT_EPISODE_STATS) = range(36)
 ROLLOUT_DEVICE_IO = 2
 ROLLOUT_OBS_F32 = 4
 ROLLOUT_OBS_AER = 8
+EPISODE_STATS_DOUBLES = 23
 
 
 class SsaUkfCfg(ctypes.Structure):
@@ -73,6 +75,8 @@ PROTOTYPES = {
     "ssa_ukf_rollout_step": (_I, [c_void_p, _I, c_void_p]),
     "ssa_ukf_rollout_obs_f32": (_I, [c_void_p, c_void_p, c_void_p]),
     "ssa_ukf_rollout_obs_aer": (_I, [c_void_p, c_void_p, c_void_p]),
+    "ssa_ukf_rollout_episode_stats_enable": (_I, [c_void_p]),
+    "ssa_ukf_rollout_episode_stats_download": (_I, [c_void_p, c_void_p, _I, c_void_p, c_void_p]),
     "ssa_trans_matrix_table": (_I, [_I, _I, _I, _D, _D, _I, c_void_p, _I, c_void_p]),
     "ssa_ukf_predict": (_I, [c_void_p, c_void_p]),
     "ssa_ukf_update": (_I, [c_void_p, c_void_p, _I, c_void_p]),

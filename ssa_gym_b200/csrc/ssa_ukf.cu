@@ -1756,6 +1756,16 @@ struct ssa_ukf {
     cudaGraphExec_t gexec[6];  // [auto_reset + 2 * (obs_f32 ? 1 : obs_aer ? 2 : 0)]
     int gkernels[6];
   } ro;
+  // per-episode statistics of the episodic mode (ssa_ukf_rollout_episode_stats_*)
+  struct {
+    int on;              // buffers allocated (ssa_ukf_rollout_episode_stats_enable)
+    int live;            // accumulating: the step graphs carry k_ep_row0 / k_ep_step (from the next rollout_reset on)
+    double* buf;         // device: obj [N][SSA_EPO], env [E][SSA_EPE], rec [E][SSA_EPR], gathered [E][SSA_EPR], idx [E]
+    double *obj, *env, *rec, *gath;
+    int32_t* didx;
+    double* hbuf;        // pinned: gathered records [E][SSA_EPR], then idx [E] int32
+    int32_t* hidx;
+  } es;
   int32_t *status, *infl, *actions, *greedy;
   uint8_t *visible, *updated, *innov_flags, *done;
   double* diag;     // [N][2] NEES, NIS of the last ssa_ukf_diagnostics call
@@ -1925,6 +1935,7 @@ int ssa_ukf_destroy(ssa_ukf* h) {
     cudaFreeHost(h->ro.hout); cudaFreeHost(h->ro.hin); cudaFreeHost(h->ro.hobs32); cudaFreeHost(h->ro.haer);
     for (int i = 0; i < 6; ++i) if (h->ro.gexec[i]) cudaGraphExecDestroy(h->ro.gexec[i]);
   }
+  if (h->es.on) { cudaFree(h->es.buf); cudaFreeHost(h->es.hbuf); }
   cudaFree(h->snap);
   cudaFree(h->cat_part);
   cudaFree(h->stage);
@@ -2025,6 +2036,9 @@ static int field_info(ssa_ukf* h, int field, void** p, size_t* bytes, int* soa_c
     case SSA_F_ROLLOUT_OBS_AER:
       if (!h->ro.init) { snprintf(g_err, sizeof(g_err), "episodic mode not configured"); return SSA_EINVAL; }
       *p = h->ro.daer; *bytes = N * 4 * 8; break;
+    case SSA_F_ROLLOUT_EPISODE_STATS:
+      if (!h->es.on) { snprintf(g_err, sizeof(g_err), "episode statistics not enabled"); return SSA_EINVAL; }
+      *p = h->es.rec; *bytes = E * SSA_EPR * 8; break;
     default: snprintf(g_err, sizeof(g_err), "unknown field %d", field); return SSA_EINVAL;
   }
   return SSA_OK;
@@ -2538,6 +2552,10 @@ int ssa_ukf_rollout_config(ssa_ukf* h, const double* orbits, int n_orbits, const
     for (int i = 0; i < 6; ++i) if (h->ro.gexec[i]) { cudaGraphExecDestroy(h->ro.gexec[i]); h->ro.gexec[i] = nullptr; }
     h->ro.init = 0;
   }
+  if (h->es.on) {  // (a new configuration runs without episode statistics until they are enabled again)
+    cudaFree(h->es.buf); cudaFreeHost(h->es.hbuf);
+    memset(&h->es, 0, sizeof(h->es));
+  }
   h->ro.n_orbits = n_orbits; h->ro.n_table = n_table; h->ro.update_interval = update_interval;
   CK(cudaMalloc(&h->ro.dbuf, sizeof(double) * ((size_t)n_orbits * 6 + (size_t)n_table * 9 + 32)));
   h->ro.orbits = h->ro.dbuf; h->ro.table = h->ro.orbits + (size_t)n_orbits * 6; h->ro.sig = h->ro.table + (size_t)n_table * 9;
@@ -2593,10 +2611,20 @@ int ssa_ukf_rollout_io(ssa_ukf* h, int32_t** actions, double** obs, double** rew
 
 static void launch_obs_aer(ssa_ukf* h, cudaStream_t st);
 
+// the captured step graphs of the episodic mode (re-captured on the next ssa_ukf_rollout_step)
+static void rollout_drop_graphs(ssa_ukf* h) {
+  for (int i = 0; i < 6; ++i) if (h->ro.gexec[i]) { cudaGraphExecDestroy(h->ro.gexec[i]); h->ro.gexec[i] = nullptr; }
+}
+
 int ssa_ukf_rollout_reset(ssa_ukf* h, void* stream) {
   if (!h || !h->ro.init) return SSA_EINVAL;
   CK(cudaSetDevice(h->device));
   cudaStream_t st = (cudaStream_t)stream;
+  if (h->es.on) {  // every environment starts an episode: accumulators and records cleared, accumulation from here on
+    const size_t N = h->cfg.n_objects, E = h->cfg.n_envs;
+    CK(cudaMemsetAsync(h->es.buf, 0, sizeof(double) * (N * SSA_EPO + E * (SSA_EPE + SSA_EPR)), st));
+    if (!h->es.live) { rollout_drop_graphs(h); h->es.live = 1; }
+  }
   RolloutParams rp;
   rollout_params(h, &rp, 0);
   k_env_reset<<<(unsigned)rp.E, 128, 0, st>>>(rp);
@@ -2675,18 +2703,90 @@ static void launch_obs_aer(ssa_ukf* h, cudaStream_t st) {
   h->launches++;
 }
 
+// ---- per-episode statistics (ssa_ukf_rollout_episode_stats_*; accumulator layouts in ssa_ukf_core.h) ---------------
+struct EpParams {
+  const double* xt; const double* x; const double* P; long ld;   // state (SoA)
+  const int32_t* step_idx; const int32_t* act_eff;                // [E]
+  const uint8_t* updated; const double* y; const double* S;       // [N], [N][3], [N][9] (SSA_STEP_RECORD)
+  const double* reward; const uint8_t* done;                      // [E] of the output block
+  const int32_t* status;                                          // [N]
+  double* obj; double* env; double* rec;                          // [N][SSA_EPO], [E][SSA_EPE], [E][SSA_EPR]
+  int E, m, auto_reset;
+};
+static_assert(SSA_EPR == SSA_EPISODE_STATS_DOUBLES, "episode record layout");
+
+static void ep_params(ssa_ukf* h, EpParams* p, int auto_reset) {
+  const size_t N = h->cfg.n_objects, E = h->cfg.n_envs;
+  p->xt = h->xt; p->x = h->x; p->P = h->P; p->ld = h->ld;
+  p->step_idx = h->step_idx; p->act_eff = h->ro.act_eff;
+  p->updated = h->updated; p->y = h->y; p->S = h->S;
+  p->reward = h->ro.dout + 12 * N;
+  p->done = (const uint8_t*)((const int32_t*)(p->reward + E) + SSA_N_TASKERS * E);
+  p->status = h->status;
+  p->obj = h->es.obj; p->env = h->es.env; p->rec = h->es.rec;
+  p->E = (int)E; p->m = h->cfg.m; p->auto_reset = auto_reset;
+}
+
+// head of an episodic step: row 0 (the fresh draw, before the first predict) of the environments at step index 0, one
+// thread per object
+__global__ void __launch_bounds__(128) k_ep_row0(const EpParams p) {
+  const long n = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (n >= (long)p.E * p.m || p.step_idx[n / p.m] != 0) return;
+  ssa_ep_nees_row(p.obj + n * SSA_EPO, p.xt + n, p.x + n, p.ld, p.P + n, p.ld);
+}
+
+// after the reward / done reduction, before a finished environment is re-drawn: one warp per environment, four per CTA.
+// The lanes add the NEES of the step's row of every object; lane 0 then adds the tasked object's innovation terms and
+// the step reward, and for a finished environment writes the record (and clears the accumulators with auto-reset).
+__global__ void __launch_bounds__(128) k_ep_step(const EpParams p) {
+  const int e = (int)(blockIdx.x * 4 + (threadIdx.x >> 5)), lane = threadIdx.x & 31;
+  if (e >= p.E) return;  // (warp-uniform)
+  const long b = (long)e * p.m;
+  for (int j = lane; j < p.m; j += 32)
+    ssa_ep_nees_row(p.obj + (b + j) * SSA_EPO, p.xt + b + j, p.x + b + j, p.ld, p.P + b + j, p.ld);
+  __syncwarp();  // (lane 0 reads the object accumulators of the other lanes below)
+  if (lane) return;
+  double* env = p.env + (long)e * SSA_EPE;
+  double* obj = p.obj + b * SSA_EPO;
+  const int a = p.act_eff[e];
+  if (a >= 0 && a < p.m && p.updated[b + a]) ssa_ep_observe(env, obj + (long)a * SSA_EPO, p.y + (b + a) * 3, p.S + (b + a) * 9);
+  env[SSA_EPE_RET] = env[SSA_EPE_RET] + p.reward[e];
+  if (p.done[e]) {
+    ssa_ep_finalise(env, obj, p.status + b, p.m, (double)p.step_idx[e], p.rec + (long)e * SSA_EPR);
+    if (p.auto_reset) ssa_ep_clear(env, obj, p.m);
+  }
+}
+
+__global__ void __launch_bounds__(256) k_ep_gather(const double* __restrict__ rec, const int32_t* __restrict__ idx, int n,
+                                                   double* __restrict__ out) {
+  const int t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t < n * SSA_EPR) out[t] = rec[(long)idx[t / SSA_EPR] * SSA_EPR + t % SSA_EPR];
+}
+
 static int rollout_chain(ssa_ukf* h, cudaStream_t st, int auto_reset, int obs_f32, int obs_aer) {
   RolloutParams rp;
   rollout_params(h, &rp, 1);
   const long N = h->cfg.n_objects;
+  const bool stats = h->es.live != 0;
+  EpParams sp;
+  if (stats) {
+    ep_params(h, &sp, auto_reset);
+    k_ep_row0<<<(unsigned)((N + 127) / 128), 128, 0, st>>>(sp);
+    h->launches++;
+  }
   k_env_begin<<<(unsigned)((N + 127) / 128), 128, 0, st>>>(rp);
   h->launches++;
   StepOverride ov{h->ro.dout, h->ro.act_eff, h->ro.table, h->step_idx, 1, h->ro.n_table, nullptr};
-  int rc = step_impl(h, nullptr, SSA_STEP_TRUTH | SSA_STEP_PREDICT | SSA_STEP_UPDATE_ACT | SSA_STEP_EPILOGUE, st, nullptr, -1, &ov);
+  int rc = step_impl(h, nullptr, SSA_STEP_TRUTH | SSA_STEP_PREDICT | SSA_STEP_UPDATE_ACT | SSA_STEP_EPILOGUE | (stats ? SSA_STEP_RECORD : 0),
+                     st, nullptr, -1, &ov);
   if (rc) return rc;
   EnvParams ep;
   rollout_env_params(h, &ep, 1, 0);
   launch_env_reduce(h, ep, st);
+  if (stats) {
+    k_ep_step<<<(unsigned)((rp.E + 3) / 4), 128, 0, st>>>(sp);
+    h->launches++;
+  }
   if (auto_reset && !h->use_team && !getenv("SSA_UKF_REFRESH_CHAIN")) {  // one launch (k_env_refresh)
     EnvParams rep;
     rollout_env_params(h, &rep, 0, 1);
@@ -2724,6 +2824,45 @@ int ssa_ukf_rollout_obs_f32(ssa_ukf* h, float** host, float** device) {
   if (!h || !h->ro.init) return SSA_EINVAL;
   if (host) *host = h->ro.hobs32;
   if (device) *device = h->ro.dobs32;
+  return SSA_OK;
+}
+
+int ssa_ukf_rollout_episode_stats_enable(ssa_ukf* h) {
+  if (!h || !h->ro.init) { snprintf(g_err, sizeof(g_err), "episodic mode not configured"); return SSA_EINVAL; }
+  CK(cudaSetDevice(h->device));
+  const size_t N = h->cfg.n_objects, E = h->cfg.n_envs;
+  if (h->es.on) { CK(cudaDeviceSynchronize()); cudaFree(h->es.buf); cudaFreeHost(h->es.hbuf); memset(&h->es, 0, sizeof(h->es)); }
+  const size_t acc = N * SSA_EPO + E * (SSA_EPE + SSA_EPR);
+  CK(cudaMalloc(&h->es.buf, sizeof(double) * (acc + E * SSA_EPR) + sizeof(int32_t) * E));
+  CK(cudaMemset(h->es.buf, 0, sizeof(double) * (acc + E * SSA_EPR) + sizeof(int32_t) * E));
+  h->es.obj = h->es.buf; h->es.env = h->es.obj + N * SSA_EPO; h->es.rec = h->es.env + E * SSA_EPE;
+  h->es.gath = h->es.rec + E * SSA_EPR; h->es.didx = (int32_t*)(h->es.gath + E * SSA_EPR);
+  CK(cudaHostAlloc(&h->es.hbuf, sizeof(double) * E * SSA_EPR + sizeof(int32_t) * E, cudaHostAllocDefault));
+  h->es.hidx = (int32_t*)(h->es.hbuf + E * SSA_EPR);
+  h->es.on = 1;
+  h->es.live = 0;  // (from the next ssa_ukf_rollout_reset)
+  rollout_drop_graphs(h);
+  return SSA_OK;
+}
+
+int ssa_ukf_rollout_episode_stats_download(ssa_ukf* h, const int32_t* envs, int n, double* out, void* stream) {
+  if (!h) return SSA_EINVAL;
+  if (!h->es.on) { snprintf(g_err, sizeof(g_err), "episode statistics not enabled"); return SSA_EINVAL; }
+  const int E = h->cfg.n_envs;
+  if (n < 0 || n > E || (n > 0 && (!envs || !out))) { snprintf(g_err, sizeof(g_err), "bad environment list"); return SSA_EINVAL; }
+  for (int k = 0; k < n; ++k)
+    if (envs[k] < 0 || envs[k] >= E) { snprintf(g_err, sizeof(g_err), "environment index %d out of range", envs[k]); return SSA_EINVAL; }
+  if (n == 0) return SSA_OK;
+  CK(cudaSetDevice(h->device));
+  cudaStream_t st = (cudaStream_t)stream;
+  memcpy(h->es.hidx, envs, sizeof(int32_t) * n);
+  CK(cudaMemcpyAsync(h->es.didx, h->es.hidx, sizeof(int32_t) * n, cudaMemcpyHostToDevice, st));
+  k_ep_gather<<<(unsigned)((n * SSA_EPR + 255) / 256), 256, 0, st>>>(h->es.rec, h->es.didx, n, h->es.gath);
+  h->launches++;
+  CK(cudaGetLastError());
+  CK(cudaMemcpyAsync(h->es.hbuf, h->es.gath, sizeof(double) * n * SSA_EPR, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  memcpy(out, h->es.hbuf, sizeof(double) * n * SSA_EPR);
   return SSA_OK;
 }
 

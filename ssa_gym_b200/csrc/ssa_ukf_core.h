@@ -247,6 +247,113 @@ SSA_HD double ssa_nis3(const double* S, const double* y, int* flags) {
   return acc;
 }
 
+// Per-episode statistics of the device-resident episodic mode (ssa_ukf_rollout_episode_stats_*): running sums of the
+// diagnostics above over one episode, a few doubles per object and per environment instead of the per-step histories
+// of the drop-in env.  Counts are kept as doubles (exact up to 2^53).  Host layouts equal the device ones (AoS).
+// Object accumulator [SSA_EPO]: sum and count of the non-NaN NEES of its rows, Durbin-Watson state {num, den, prev} of
+// its own innovation series per component, and the number of entries of that series.
+#define SSA_EPO_S 0
+#define SSA_EPO_C 1
+#define SSA_EPO_DW 2
+#define SSA_EPO_DWN 11
+#define SSA_EPO 12
+// Environment accumulator [SSA_EPE]: return, observations, NIS sum / count, the six innovation-bound counters (inside
+// 1 sigma per component, then inside 2 sigmas), Durbin-Watson state of the overall innovation series and its entries.
+#define SSA_EPE_RET 0
+#define SSA_EPE_OBS 1
+#define SSA_EPE_NIS 2
+#define SSA_EPE_NISN 3
+#define SSA_EPE_BND 4
+#define SSA_EPE_DW 10
+#define SSA_EPE_DWN 19
+#define SSA_EPE 20
+// Record of a finished episode: SSA_EPISODE_STATS_DOUBLES (include/ssa_ukf.h) doubles, layout documented there.
+#define SSA_EPR 23
+
+// one row of an episode for one object: NEES of (x_true - x, P) as ssa_diag_kernel evaluates it, NaN left out
+SSA_HD void ssa_ep_nees_row(double* o, const double* xt, const double* x, long xs, const double* P, long ps) {
+  double d[6];
+#pragma unroll
+  for (int i = 0; i < 6; ++i) d[i] = xt[i * xs] - x[i * xs];
+  const double v = ssa_nees6(P, ps, d);
+  if (v == v) {
+    o[SSA_EPO_S] = o[SSA_EPO_S] + v;
+    o[SSA_EPO_C] = o[SSA_EPO_C] + 1.0;
+  }
+}
+// one entry of a Durbin-Watson series per component, in the order of ssa_innov_stats_kernel; dw = {num, den, prev} x 3,
+// n = entries before this one
+SSA_HD void ssa_dw_push(double* dw, double n, const double* y) {
+#pragma unroll
+  for (int c = 0; c < 3; ++c) {
+    const double e = y[c];
+    dw[3 * c + 1] = ssa_fma(e, e, dw[3 * c + 1]);
+    if (n > 0.0) {
+      const double d = e - dw[3 * c + 2];
+      dw[3 * c] = ssa_fma(d, d, dw[3 * c]);
+    }
+    dw[3 * c + 2] = e;
+  }
+}
+// an update of the tasked object: its innovation y and innovation covariance S (SSA_STEP_RECORD)
+SSA_HD void ssa_ep_observe(double* env, double* obj, const double* y, const double* S) {
+  env[SSA_EPE_OBS] = env[SSA_EPE_OBS] + 1.0;
+  int f = 0;
+  const double nis = ssa_nis3(S, y, &f);
+  if (nis == nis) {
+    env[SSA_EPE_NIS] = env[SSA_EPE_NIS] + nis;
+    env[SSA_EPE_NISN] = env[SSA_EPE_NISN] + 1.0;
+  }
+#pragma unroll
+  for (int b = 0; b < 6; ++b) env[SSA_EPE_BND + b] = env[SSA_EPE_BND + b] + (double)((f >> b) & 1);
+  ssa_dw_push(env + SSA_EPE_DW, env[SSA_EPE_DWN], y);
+  env[SSA_EPE_DWN] = env[SSA_EPE_DWN] + 1.0;
+  ssa_dw_push(obj + SSA_EPO_DW, obj[SSA_EPO_DWN], y);
+  obj[SSA_EPO_DWN] = obj[SSA_EPO_DWN] + 1.0;
+}
+// The record of an episode that ended at step L: env accumulator, the m object accumulators [m][SSA_EPO] and the m
+// status words of the environment.  Per-object Durbin-Watson min / max over the objects with >= 2 entries, NaN
+// propagating as in np.min / np.max, NaN when no object qualifies.
+SSA_HD void ssa_ep_finalise(const double* env, const double* obj, const int32_t* status, int m, double L, double* rec) {
+  rec[0] = L;
+  rec[1] = env[SSA_EPE_RET];
+  double s = 0.0, c = 0.0, failed = 0.0;
+  for (int j = 0; j < m; ++j) {
+    s = s + obj[j * SSA_EPO + SSA_EPO_S];
+    c = c + obj[j * SSA_EPO + SSA_EPO_C];
+    failed = failed + ((status[j] & SSA_ST_FAILED) ? 1.0 : 0.0);
+  }
+  rec[2] = s;
+  rec[3] = c;
+  rec[4] = env[SSA_EPE_NIS];
+  rec[5] = env[SSA_EPE_NISN];
+  rec[6] = env[SSA_EPE_OBS];
+#pragma unroll
+  for (int b = 0; b < 6; ++b) rec[7 + b] = env[SSA_EPE_BND + b];
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    rec[13 + k] = env[SSA_EPE_DWN] > 0.0 ? ssa_div(env[SSA_EPE_DW + 3 * k], env[SSA_EPE_DW + 3 * k + 1]) : ssa_nan();
+    double lo = ssa_nan(), hi = ssa_nan();
+    int any = 0, nan = 0;
+    for (int j = 0; j < m; ++j) {
+      const double* o = obj + j * SSA_EPO;
+      if (!(o[SSA_EPO_DWN] >= 2.0)) continue;
+      const double v = ssa_div(o[SSA_EPO_DW + 3 * k], o[SSA_EPO_DW + 3 * k + 1]);
+      nan |= (v != v);
+      lo = (!any || v < lo) ? v : lo;
+      hi = (!any || v > hi) ? v : hi;
+      any = 1;
+    }
+    rec[16 + k] = nan ? ssa_nan() : lo;
+    rec[19 + k] = nan ? ssa_nan() : hi;
+  }
+  rec[22] = failed;
+}
+SSA_HD void ssa_ep_clear(double* env, double* obj, int m) {
+  for (int q = 0; q < SSA_EPE; ++q) env[q] = 0.0;
+  for (int q = 0; q < m * SSA_EPO; ++q) obj[q] = 0.0;
+}
+
 // Determinant of a packed symmetric 6x6 (agent_shannon, agents.py:24: np.linalg.det(P)).  numpy factors with a pivoted
 // LU; for the symmetric (normally positive definite) covariances of the path the unpivoted symmetric elimination
 // P = L D L^T is just as stable, needs half the arithmetic and keeps its 21 entries in registers with static indices:

@@ -106,6 +106,7 @@ class BatchedUKF:
             _lib.F_ROLLOUT_REWARD: ((self.n_envs,), np.float64), _lib.F_ROLLOUT_ACTIONS: ((self.n_envs,), np.int32),
             _lib.F_ROLLOUT_DONE: ((self.n_envs,), np.uint8), _lib.F_ROLLOUT_GREEDY: ((self.n_envs, _lib.N_TASKERS), np.int32),
             _lib.F_ROLLOUT_OBS_AER: ((self.N, 4), np.float64),
+            _lib.F_ROLLOUT_EPISODE_STATS: ((self.n_envs, _lib.EPISODE_STATS_DOUBLES), np.float64),
         }
 
     # -- lifetime ---------------------------------------------------------------------------------
@@ -284,6 +285,20 @@ class BatchedUKF:
         mode = (1 if auto_reset else 0) | (_lib.ROLLOUT_DEVICE_IO if device_io else 0) | (_lib.ROLLOUT_OBS_F32 if obs_f32 else 0) | \
             (_lib.ROLLOUT_OBS_AER if obs_aer else 0)
         _lib.check(self.lib.ssa_ukf_rollout_step(self.h, mode, stream), "ssa_ukf_rollout_step")
+
+    def rollout_episode_stats_enable(self):
+        """Accumulate per-episode statistics inside the step graph from the next rollout_reset on (after rollout_config,
+        which turns them off again).  Records: rollout_episode_stats, or the device field F_ROLLOUT_EPISODE_STATS."""
+        _lib.check(self.lib.ssa_ukf_rollout_episode_stats_enable(self.h), "ssa_ukf_rollout_episode_stats_enable")
+
+    def rollout_episode_stats(self, envs, stream=None):
+        """The records [len(envs), EPISODE_STATS_DOUBLES] of the environments `envs` (layout: include/ssa_ukf.h); blocks
+        until copied.  A row is that of the episode that ended on the last step whose done flag was set for it."""
+        envs = np.ascontiguousarray(envs, dtype=np.int32).reshape(-1)
+        out = np.empty((len(envs), _lib.EPISODE_STATS_DOUBLES))
+        _lib.check(self.lib.ssa_ukf_rollout_episode_stats_download(self.h, _ptr(envs), len(envs), _ptr(out), stream),
+                   "ssa_ukf_rollout_episode_stats_download")
+        return out
 
     @property
     def next_parity(self):

@@ -18,7 +18,10 @@ n*m*3 + 7m numbers per environment from a sequential MT19937 stream on the host 
 vector_step in host mode against 0.45 ms in device mode).  The device mode covers the reference's whole configuration
 matrix: the 'shaped' reward keeps its per-environment reward history on the device (the episode's own 1 - np.sum(
 rewards[:i]) in numpy's summation order), and the 'aer' layout is computed by the last kernel of the step's graph, so
-only its [E, m*4] rows (32 B per object instead of 96) cross PCIe and the host formats nothing.
+only its [E, m*4] rows (32 B per object instead of 96) cross PCIe and the host formats nothing.  With
+`config['episode_stats'] = True` the step graph also accumulates every episode's return, length and the reference's
+filter-consistency figures (ANEES, NIS, innovation bounds, Durbin-Watson statistics) on the device; a finished
+environment reports them in `infos[e]['episode']` (see `episode_info`).
 """
 import numpy as np
 
@@ -29,6 +32,33 @@ from .transformations import arcsec2rad, default_eops, deg2rad, gcrs2irts_matrix
 from .ukf import BatchedUKF, Q_discrete_white_noise_block
 
 F = _lib
+
+
+def episode_info(rec):
+    """infos[e]['episode'] of a finished episode from its device record (include/ssa_ukf.h, SSA_EPISODE_STATS_DOUBLES):
+    'r' return and 'l' length (gymnasium's RecordEpisodeStatistics / SB3's Monitor keys), 'anees' (SS2:436-446, the mean
+    of the finite NEES values over rows 0 .. l and all objects), 'nis' (mean NIS of the tasked observations, SS2:564-569),
+    'observations', 'innovation_bounds' [2, 3] percentages inside 1 / 2 sigmas (SS2:598-604), 'durbin_watson' [3, 3]
+    rows all observations / min per object / max per object (SS2:782-832, rounded like innovation_dw_test) and 'failed'
+    (objects whose filter failed)."""
+    return episode_infos(np.asarray(rec).reshape(1, -1))[0]
+
+
+def episode_infos(recs):
+    """episode_info of the records [n, EPISODE_STATS_DOUBLES]: one numpy pass over all of them, then one dict each (a
+    step on which thousands of environments finish together builds its dicts in ~1 us each)."""
+    recs = np.asarray(recs, dtype=np.float64)
+    n_obs = recs[:, 6]
+    with np.errstate(invalid='ignore', divide='ignore'):
+        anees = np.where(recs[:, 3] > 0, recs[:, 2] / recs[:, 3], np.nan)
+        nis = np.where(recs[:, 5] > 0, recs[:, 4] / recs[:, 5], np.nan)
+        bounds = np.round(recs[:, 7:13].reshape(-1, 2, 3) / n_obs[:, None, None] * 100, 2)
+    bounds[n_obs == 0] = np.nan
+    dw = np.round(recs[:, 13:22].reshape(-1, 3, 3), 3)
+    scal = zip(recs[:, 1].tolist(), recs[:, 0].astype(np.int64).tolist(), anees.tolist(), nis.tolist(),
+               n_obs.astype(np.int64).tolist(), recs[:, 22].astype(np.int64).tolist())
+    return [{"r": r, "l": l, "anees": a, "nis": v, "observations": o, "innovation_bounds": b, "durbin_watson": d, "failed": f}
+            for (r, l, a, v, o, f), b, d in zip(scal, bounds, dw)]
 
 
 class VecSSATaskerEnv:
@@ -50,6 +80,10 @@ class VecSSATaskerEnv:
                 raise ValueError("obs_dtype='float32' needs rng='device' and a state-vector layout (obs_returned != 'aer')")
         elif self.obs_dtype != np.float64:
             raise ValueError("obs_dtype must be 'float64' or 'float32'")
+        # per-episode statistics accumulated inside the step graph (device mode only: the host mode has no device episodes)
+        self.episode_stats = bool(config.get('episode_stats', False))
+        if self.episode_stats and rng != 'device':
+            raise ValueError("episode_stats=True needs rng='device'")
         self.update_interval = config['update_interval']
         self.auto_reset = auto_reset
         if config.get('orbits') is not None:
@@ -100,6 +134,9 @@ class VecSSATaskerEnv:
                                                self.update_interval)
             self.z_noise = None  # drawn on the device, step by step
             self._infos = [{} for _ in range(self.E)]
+            self._infos_filled = []  # environments whose info dict holds the 'episode' entry of the previous step
+            if self.episode_stats:
+                self.ukf.rollout_episode_stats_enable()  # (accumulates from the rollout_reset of vector_reset on)
         self.obs = self.vector_reset()
 
     # -- seeding / reset --------------------------------------------------------------------------------
@@ -262,13 +299,26 @@ class VecSSATaskerEnv:
             self.obs = io["obs_aer"].reshape(self.E, self.m * 4)
         else:
             self.obs = self._format_obs(io["obs_f32" if f32 else "obs"].reshape(self.E, self.m * 12))
-        return self.obs, self._format_reward(rewards), dones, self._infos  # E empty dicts, allocated once (4096 dict constructions cost 100 us)
+        # E dicts allocated once (4096 dict constructions cost 100 us): empty, except on the step an episode finished
+        infos = self._infos
+        for e in self._infos_filled:
+            infos[e].clear()
+        self._infos_filled = []
+        if self.episode_stats and dones.any():
+            de = np.flatnonzero(dones).tolist()
+            for e, ep in zip(de, episode_infos(self.ukf.rollout_episode_stats(de))):
+                infos[e]["episode"] = ep
+            self._infos_filled = de
+        return self.obs, self._format_reward(rewards), dones, infos
 
     # -- device-resident consumer (a policy on the same GPU): no host copies, nothing synchronises -------------------
     def device_views(self):
         """Zero-copy torch tensors over the episodic mode's device buffers: 'actions' int32 [E] (INPUT of
         vector_step_device), 'obs' float64 [E, m*12] ([E, m*4] for obs_returned='aer'), 'reward' float64 [E], 'done' uint8
         [E], 'greedy' int32 [E, taskers].
+        With config['episode_stats']: 'episode_stats' float64 [E, EPISODE_STATS_DOUBLES], the record of each environment's
+        last finished episode (layout: include/ssa_ukf.h; episode_info turns a row into the infos entry), valid after a
+        step whose 'done' is set for it.
         The outputs are overwritten by every step; they are valid in stream order on the stream the step runs on."""
         assert self.rng == 'device', "device views exist in the device-resident episodic mode (rng='device')"
         if getattr(self, "_views", None) is None:
@@ -278,6 +328,8 @@ class VecSSATaskerEnv:
             self._views = {"actions": u.torch_view(F.F_ROLLOUT_ACTIONS), "obs": obs,
                            "reward": u.torch_view(F.F_ROLLOUT_REWARD), "done": u.torch_view(F.F_ROLLOUT_DONE),
                            "greedy": u.torch_view(F.F_ROLLOUT_GREEDY)}
+            if self.episode_stats:
+                self._views["episode_stats"] = u.torch_view(F.F_ROLLOUT_EPISODE_STATS)
         return self._views
 
     def vector_step_device(self, stream=None):
