@@ -12,6 +12,14 @@
 // Accuracy target: <= ~2 ulp on the argument ranges the path uses (measured against mpmath in
 // tests/test_math_accuracy.py).  Polynomial coefficients are the classic fdlibm minimax sets.
 //
+// Domain and special values (tests/test_math_domain.py, against numpy and mpmath): every function accepts every double
+// and keeps its ulp bound over its whole finite domain, with three stated exceptions: sinh / cosh on
+// (709.78, 710.48] (2.5 ulp: exp(|x|/2) squared), pow23 (1.5 + 1.5 |2/3 log x| ulp) and the subnormal results of exp
+// (counted in ulps of 2^-1074).  NaN in gives NaN out; results overflow and underflow where the true values do; odd
+// functions keep the sign of zero; atan2 follows C99 Annex F for signed zeros and infinities.  pow23 is NaN for every
+// x < 0, -inf included.  The inlined variants ssa_sincos_i and ssa_atan2_i are restricted to the ranges their hot
+// callers use (see there).
+//
 // No CUDA libdevice transcendental is called anywhere on the hot path.
 #pragma once
 #include <math.h>
@@ -239,16 +247,8 @@ SSA_HD double ssa_pymod(double a, double b) {
 #define SSA_RMAGIC  6755399441055744.0            /* 1.5 * 2^52 */
 
 typedef struct { double s, c; } ssa_sc;
-// Real (non-inlined) device functions for the big kernels below: the fused step kernel calls them
-// from ~60 sites and would otherwise exceed the instruction cache several times over.  Results are
-// returned by value so they travel in registers.
-SSA_HD ssa_sc ssa_sincos_i(double x) {
-  double t = ssa_fma(x, SSA_C(INVPIO2), SSA_C(RMAGIC));
-  int32_t q = ssa_lo32(t);
-  double n = t - SSA_C(RMAGIC);
-  double r = ssa_fma(-n, SSA_C(PIO2_A), x);
-  r = ssa_fma(-n, SSA_C(PIO2_B), r);
-  r = ssa_fma(-n, SSA_C(PIO2_C), r);
+// sin and cos of x = r + q pi/2, |r| <= ~pi/4: the fdlibm kernels, then the quadrant.
+SSA_HD ssa_sc ssa_sincos_kern(double r, int32_t q) {
   double z = ssa_mul(r, r);
   // sin kernel: r + r^3 (S1 + z S2 + ... )
   double ps = ssa_fma(z, SSA_C(S6), SSA_C(S5));
@@ -276,7 +276,133 @@ SSA_HD ssa_sc ssa_sincos_i(double x) {
   out.c = c_;
   return out;
 }
-SSA_HD_NOINLINE ssa_sc ssa_sincos_v(double x) { return ssa_sincos_i(x); }
+
+// 2/pi in binary, 32 bits a word, most significant first, after one word of zeros: table bit j is the bit of weight
+// 2^(31 - j), so that the reduction below can read windows that start before the binary point.
+#define SSA_TWO_OVER_PI_BITS(X)                                                                                      \
+  X(0x00000000) X(0xa2f9836e) X(0x4e441529) X(0xfc2757d1) X(0xf534ddc0) X(0xdb629599) X(0x3c439041) X(0xfe5163ab)    \
+  X(0xdebbc561) X(0xb7246e3a) X(0x424dd2e0) X(0x06492eea) X(0x09d1921c) X(0xfe1deb1c) X(0xb129a73e) X(0xe88235f5)    \
+  X(0x2ebb4484) X(0xe99c7026) X(0xb45f7e41) X(0x3991d639) X(0x835339f4) X(0x9c845f8b) X(0xbdf9283b) X(0x1ff897ff)    \
+  X(0xde05980f) X(0xef2f118b) X(0x5a0a6d1f) X(0x6d367ecf) X(0x27cb09b7) X(0x4f463f66) X(0x9e5fea2d) X(0x7527bac7)    \
+  X(0xebe5f17b) X(0x3d0739f7) X(0x8a5292ea) X(0x6bfb5fb1) X(0x1f8d5d08) X(0x56033046) X(0xfc7b6bab) X(0xf0cfbc20)    \
+  X(0x9af4361d)
+#define SSA_W32(v) v##u,
+#if defined(__CUDACC__)
+static __constant__ uint32_t ssa_2opi_dev[] = {SSA_TWO_OVER_PI_BITS(SSA_W32)};
+#endif
+static const uint32_t ssa_2opi_host[] = {SSA_TWO_OVER_PI_BITS(SSA_W32)};
+#undef SSA_W32
+SSA_HD uint64_t ssa_2opi_bits64(int j) {  // table bits j .. j+63
+#if defined(__CUDA_ARCH__)
+  const uint32_t* T = ssa_2opi_dev;
+#else
+  const uint32_t* T = ssa_2opi_host;
+#endif
+  const int w = j >> 5, s = j & 31;
+  const uint64_t a = ((uint64_t)T[w] << 32) | T[w + 1];
+  const uint64_t b = ((uint64_t)T[w + 2] << 32) | T[w + 3];
+  return s ? ((a << s) | (b >> (64 - s))) : a;
+}
+SSA_HD uint64_t ssa_umulhi64(uint64_t a, uint64_t b) {
+#if defined(__CUDA_ARCH__)
+  return __umul64hi(a, b);
+#else
+  return (uint64_t)(((unsigned __int128)a * b) >> 64);
+#endif
+}
+SSA_HD int ssa_clz64(uint64_t v) {  // v != 0
+#if defined(__CUDA_ARCH__)
+  return __clzll((long long)v);
+#else
+  return __builtin_clzll(v);
+#endif
+}
+
+// Arguments outside [2^-27, 2^30) in magnitude.  Tiny ones: sin x = x (this keeps the sign of -0), cos x = 1; the
+// polynomial path returns the same bits except for -0.  Non-finite ones: NaN.  Large ones: Payne-Hanek reduction in
+// integer arithmetic.  With x = M 2^E (M a 53-bit integer), the bits of 2/pi of weight 2^(1-E) and above multiply M
+// into multiples of 4 and drop out; a 192-bit window from there gives M 2/pi 2^E mod 4 = q + f to 2^-137, and the
+// closest double to a multiple of pi/2 keeps |f| above 2^-62.  f becomes a 106-bit double pair, r = f pi/2 one double.
+SSA_HD_NOINLINE ssa_sc ssa_sincos_edge(double x) {
+  const int32_t hx = ssa_hi32(x) & 0x7fffffff;
+  ssa_sc out;
+  if (hx < 0x3e400000) {
+    out.s = x;
+    out.c = 1.0;
+    return out;
+  }
+  if (hx >= 0x7ff00000) {
+    out.s = x - x;
+    out.c = out.s;
+    return out;
+  }
+  const int E = (hx >> 20) - 1075;  // >= -22
+  const uint64_t M = ((uint64_t)(hx & 0x000fffff) << 32 | (uint32_t)ssa_lo32(x)) | ((uint64_t)1 << 52);
+  const int j = E - 1 + 31;
+  const uint64_t w0 = ssa_2opi_bits64(j), w1 = ssa_2opi_bits64(j + 64), w2 = ssa_2opi_bits64(j + 128);
+  // P = M W mod 2^192, W = w0 w1 w2
+  const uint64_t p2 = M * w2;
+  const uint64_t h2 = ssa_umulhi64(M, w2);
+  const uint64_t l1 = M * w1;
+  const uint64_t p1 = l1 + h2;
+  const uint64_t p0 = M * w0 + ssa_umulhi64(M, w1) + (uint64_t)(p1 < l1);
+  int32_t q = (int32_t)(p0 >> 62);
+  uint64_t fh = (p0 << 2) | (p1 >> 62), fl = (p1 << 2) | (p2 >> 62);  // f in [0, 1), 128 bits
+  const bool neg = (fh >> 63) != 0;  // f >= 1/2: take f - 1 and the next quadrant
+  if (neg) {
+    q += 1;
+    fl = ~fl + 1;
+    fh = ~fh + (uint64_t)(fl == 0);
+  }
+  int sh = 0;
+  if (fh == 0) {
+    fh = fl;
+    fl = 0;
+    sh = 64;
+  }
+  const int lz = ssa_clz64(fh);
+  if (lz) {
+    fh = (fh << lz) | (fl >> (64 - lz));
+    fl <<= lz;
+  }
+  sh += lz;
+  // |f| = fh 2^-(64 + sh) + fl 2^-(128 + sh): a = the top 53 bits, b = the next 53
+  const double a = ssa_mul((double)(int64_t)(fh >> 11), ssa_from_hilo((int32_t)((1023 - 53 - sh) << 20), 0));
+  const double b = ssa_mul((double)(int64_t)(((fh & 0x7ff) << 42) | (fl >> 22)),
+                           ssa_from_hilo((int32_t)((1023 - 106 - sh) << 20), 0));
+  const double rh = ssa_mul(a, SSA_C(PIO2_A));
+  const double rl = ssa_fma(a, SSA_C(PIO2_B), ssa_fma(b, SSA_C(PIO2_A), ssa_fma(a, SSA_C(PIO2_A), -rh)));
+  double r = ssa_add(rh, rl);
+  if (neg) r = -r;
+  if (ssa_signbit(x)) {
+    r = -r;
+    q = -q;
+  }
+  return ssa_sincos_kern(r, q);
+}
+
+// Cody-Waite reduction, inlined into the propagation kernels.  Valid for 2^-27 <= |x| < 2^30: there the first step is
+// exact, and the pi/2 tail A + B + C keeps sin / cos within their bounds at the doubles nearest every multiple of pi/2
+// (tests/test_math_domain.py).  Its two callers stay inside that range without a test: ssa_fx's Newton iterates of
+// Kepler's equation (e < 0.99, started in [-pi, pi]) and the azimuth / elevation of ssa_aer2uvw_t.  Outside it
+// (beyond 2^51 pi/2 the quotient n is not even an integer) use ssa_sincos_v.
+SSA_HD ssa_sc ssa_sincos_i(double x) {
+  double t = ssa_fma(x, SSA_C(INVPIO2), SSA_C(RMAGIC));
+  int32_t q = ssa_lo32(t);
+  double n = t - SSA_C(RMAGIC);
+  double r = ssa_fma(-n, SSA_C(PIO2_A), x);
+  r = ssa_fma(-n, SSA_C(PIO2_B), r);
+  r = ssa_fma(-n, SSA_C(PIO2_C), r);
+  return ssa_sincos_kern(r, q);
+}
+// Every double: one unsigned compare of the high word sends |x| outside [2^-27, 2^30) to ssa_sincos_edge.  A real
+// (non-inlined) device function for the big kernels: the fused step kernel calls it from ~60 sites and would
+// otherwise exceed the instruction cache several times over.  Results are returned by value so they travel in
+// registers.
+SSA_HD_NOINLINE ssa_sc ssa_sincos_v(double x) {
+  if ((uint32_t)(ssa_hi32(x) & 0x7fffffff) - 0x3e400000u >= 0x41d00000u - 0x3e400000u) return ssa_sincos_edge(x);
+  return ssa_sincos_i(x);
+}
 SSA_HD void ssa_sincos(double x, double* sn, double* cs) {
   const ssa_sc r = ssa_sincos_v(x);
   *sn = r.s;
@@ -292,7 +418,11 @@ SSA_HD double ssa_tan(double x) { double s, c; ssa_sincos(x, &s, &c); return ssa
 // atan2 / atan  — one division: the fdlibm interval reduction (2t-1)/(2+t) etc. is applied to the
 // pair (|y|,|x|) directly, so t = |y|/|x| is never formed.
 // ---------------------------------------------------------------------------------------------
-SSA_HD double ssa_atan2_i(double y, double x) {
+SSA_HD_NOINLINE double ssa_atan2_big(double y, double x);
+// FULL: every argument pair.  |y| >= 2^1020 (where the interval tests below overflow) and inf go to ssa_atan2_big, and
+// atan2(+-0, NaN) is NaN.
+template <bool FULL>
+SSA_HD double ssa_atan2_t(double y, double x) {
   const double ax = ssa_fabs(x), ay = ssa_fabs(y);
   const double ay16 = ssa_mul(16.0, ay);
   double num, den, hi, lo;
@@ -308,12 +438,13 @@ SSA_HD double ssa_atan2_i(double y, double x) {
     num = ssa_fma(-1.5, ax, ay); den = ssa_fma(1.5, ay, ax);
     hi = SSA_C(ATHI2); lo = SSA_C(ATLO2);
   } else {
+    if (FULL && ssa_hi32(ay16) >= 0x7ff00000) return ssa_atan2_big(y, x);
     num = -ax; den = ay;
     hi = SSA_C(PIO2_A); lo = SSA_C(PIO2_B);
   }
   double z;
   if (den == 0.0) {
-    z = 0.0;  // atan2(+-0, +-0): fdlibm returns +-0 / +-pi through the quadrant logic below
+    z = FULL ? num - num : 0.0;  // atan2(+-0, +-0): fdlibm returns +-0 / +-pi through the quadrant logic below
   } else {
     const double t = ssa_div_i(num, den);
     const double t2 = ssa_mul(t, t);
@@ -335,7 +466,17 @@ SSA_HD double ssa_atan2_i(double y, double x) {
   if (ssa_signbit(x)) z = SSA_C(PI) - (z - SSA_C(PI_LO));
   return ssa_signbit(y) ? -z : z;
 }
-SSA_HD_NOINLINE double ssa_atan2(double y, double x) { return ssa_atan2_i(y, x); }
+// Both arguments scaled by 2^-6 keep the interval tests finite.  The scaling is exact for y (|y| >= 2^1020) and for
+// every x that does not make the result pi/2 to the last bit anyway.  Equal magnitudes, inf included, give the
+// octant bisectors: atan2(+-inf, +-inf) = +-pi/4, +-3pi/4.
+SSA_HD_NOINLINE double ssa_atan2_big(double y, double x) {
+  if (ssa_fabs(x) == ssa_fabs(y)) return ssa_atan2_t<false>(ssa_copysign(1.0, y), ssa_copysign(1.0, x));
+  return ssa_atan2_t<false>(ssa_mul(y, 0.015625), ssa_mul(x, 0.015625));
+}
+// Inlined variant for the hot kernels, without the two FULL cases: their arguments stay far below 2^1020 (ssa_fx:
+// e sin E0 and e cos E0 with e < 0.99; the azimuths of ssa_meas.h: coordinates in metres, 1e20 for a failed filter).
+SSA_HD double ssa_atan2_i(double y, double x) { return ssa_atan2_t<false>(y, x); }
+SSA_HD_NOINLINE double ssa_atan2(double y, double x) { return ssa_atan2_t<true>(y, x); }
 SSA_HD double ssa_atan(double x) { return ssa_atan2(x, 1.0); }
 
 // ---------------------------------------------------------------------------------------------
@@ -421,8 +562,9 @@ SSA_HD double ssa_scalbn_small(double x, int k) {  // x * 2^k for |k| < 1000, x 
 }
 SSA_HD_NOINLINE double ssa_exp(double x) {
   if (ssa_isnan(x)) return x;
-  if (x > 709.0) return ssa_from_hilo(0x7ff00000, 0);
-  if (x < -708.0) return 0.0;
+  // fdlibm's thresholds: exp(x) > DBL_MAX above o, < 2^-1075 (rounds to 0) below u
+  if (x > 7.09782712893383973096e+02) return ssa_from_hilo(0x7ff00000, 0);
+  if (x < -7.45133219101941108420e+02) return 0.0;
   const double t = ssa_fma(x, 1.44269504088896338700e+00, SSA_RMAGIC);
   const int32_t k = ssa_lo32(t);
   const double n = t - SSA_RMAGIC;
@@ -436,7 +578,7 @@ SSA_HD_NOINLINE double ssa_exp(double x) {
   c = ssa_fma(z, c, 1.66666666666666019037e-01);
   c = ssa_fma(-z, c, r);  // r - z*P(z)
   const double y = 1.0 - ((lo - ssa_div(ssa_mul(r, c), 2.0 - c)) - hi);
-  // scale by 2^k in two steps to stay in the normal range for k in [-1021, 1023]
+  // scale by 2^k, k in [-1075, 1024], in two steps: both factors are normal, so a subnormal result is y 2^k rounded once
   const int k1 = k / 2, k2 = k - k1;
   return ssa_mul(ssa_scalbn_small(y, k1), ssa_from_hilo((int32_t)((k2 + 1023) << 20), 0));
 }
@@ -477,6 +619,7 @@ SSA_HD_NOINLINE double ssa_log(double x) {
 SSA_HD double ssa_log1p(double y) {
   const double u = 1.0 + y;
   if (u == 1.0) return y;
+  if (u == ssa_from_hilo(0x7ff00000, 0)) return u;  // log1p(inf) = inf
   // log(u) * y/(u-1) corrects the rounding of 1+y (Kahan/HP-15C trick)
   return ssa_mul(ssa_log(u), ssa_div(y, u - 1.0));
 }
@@ -495,6 +638,9 @@ SSA_HD double ssa_sinh(double x) {
   if (ax < 22.0) {
     const double t = ssa_expm1(ax);
     r = ssa_mul(0.5, t + ssa_div(t, t + 1.0));
+  } else if (ax > 7.09782712893383973096e+02) {  // exp(ax) overflows, sinh(ax) up to 710.4758600739439
+    const double t = ssa_exp(ssa_mul(0.5, ax));
+    r = ssa_mul(ssa_mul(0.5, t), t);
   } else {
     r = ssa_mul(0.5, ssa_exp(ax));
   }
@@ -502,6 +648,10 @@ SSA_HD double ssa_sinh(double x) {
 }
 SSA_HD double ssa_cosh(double x) {
   const double ax = ssa_fabs(x);
+  if (ax > 7.09782712893383973096e+02) {  // as ssa_sinh
+    const double t = ssa_exp(ssa_mul(0.5, ax));
+    return ssa_mul(ssa_mul(0.5, t), t);
+  }
   const double t = ssa_exp(ax);
   return ssa_fma(0.5, t, ssa_div(0.5, t));
 }
@@ -511,8 +661,10 @@ SSA_HD double ssa_tanh(double x) {
   if (ax < 22.0) {
     const double t = ssa_expm1(ssa_mul(2.0, ax));
     r = ssa_div(t, t + 2.0);
-  } else {
+  } else if (ax >= 22.0) {
     r = 1.0;
+  } else {
+    return x;  // NaN
   }
   return ssa_signbit(x) ? -r : r;
 }
@@ -535,6 +687,7 @@ SSA_HD double ssa_asinh(double x) {
 }
 SSA_HD double ssa_acosh(double x) {
   if (!(x >= 1.0)) return ssa_nan();
+  if (x > 268435456.0) return ssa_log(x) + 6.93147180559945286227e-01;  // 2^28: t*t would overflow for large x
   const double t = x - 1.0;
   return ssa_log1p(t + ssa_sqrt(ssa_fma(t, t, ssa_mul(2.0, t))));
 }
