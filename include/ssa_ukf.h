@@ -125,6 +125,11 @@ enum ssa_field {
  * evaluated against the same previous determinant again and nothing moves, so repeated calls at one step give the
  * same picks; at i = 0, a smaller i, or with no history (after ssa_ukf_reset) the history restarts with ratio 1 and
  * the first visible object is picked.                                                                                */
+/* taskers that only the episodic mode runs (ssa_ukf_rollout_tasker): the random agents of agents.py                */
+#define SSA_TASKER_EXTERNAL (-1)             /* the caller's actions (default)                                       */
+#define SSA_TASKER_NAIVE_RANDOM 6            /* action_space.sample()                         agent_naive_random     */
+#define SSA_TASKER_VISIBLE_RANDOM 7          /* uniform among the visible objects             agent_visible_random   */
+#define SSA_TASKER_VISIBLE_GREEDY_SPOILED 8  /* visible greedy, a uniform action w.p. p    agent_visible_greedy_spoiled */
 
 /* flags for ssa_ukf_step */
 #define SSA_STEP_TRUTH 0x1        /* propagate the true states (SS2:265-266) */
@@ -245,6 +250,25 @@ int ssa_ukf_rollout_reset(ssa_ukf* h, void* stream);
  * (SSA_EINVAL).  The float64 rows stay valid on the device.                                                         */
 #define SSA_ROLLOUT_OBS_AER 8
 int ssa_ukf_rollout_step(ssa_ukf* h, int auto_reset, void* stream);
+/* Device taskers: the closed loop `a = agent(obs, env); env.step(a)` of the reference's agents inside the step graph.
+ * With a tasker set, each ssa_ukf_rollout_step first picks every environment's action from the state the previous step
+ * left (its greedy row, visibility flags, episode and step counters; ssa_tasker_pick in csrc/ssa_rng.h) and ignores
+ * the caller's: one Philox4x32-10 block per environment and step, counter (episode, 3, 0, step of the action).
+ *   SSA_TASKER_NAIVE_GREEDY .. SSA_TASKER_SHANNON   the greedy column; where it is -1, a uniform action
+ *   SSA_TASKER_NAIVE_RANDOM                          a uniform action
+ *   SSA_TASKER_VISIBLE_RANDOM                        uniform among the visible objects; without candidates (nothing,
+ *                                                    or only object 0 visible: agents.py:37) a uniform action
+ *   SSA_TASKER_VISIBLE_GREEDY_SPOILED                the visible-greedy column with probability 1 - spoil_p, else (and
+ *                                                    without candidates) a uniform action
+ * The distributions are the reference's, the streams are not (as for the reset and noise draws).  The pick is made on
+ * every step, also on steps update_interval skips, and is written to the requested-action buffer, so 'shaped' and the
+ * episode statistics see it as an external action.  The step skips the H2D of the actions; without
+ * SSA_ROLLOUT_DEVICE_IO it copies the taken actions into the pinned actions block of ssa_ukf_rollout_io, with it they
+ * are in SSA_F_ROLLOUT_ACTIONS.  A tasker step launches the kernels of an external-action step.
+ * tasker SSA_TASKER_EXTERNAL restores the caller's actions.  SSA_EINVAL before ssa_ukf_rollout_config (which returns
+ * the handle to external actions), for a tasker outside -1 .. 8, and for a spoil_p (used by
+ * SSA_TASKER_VISIBLE_GREEDY_SPOILED only) that is not in [0, 1].  A change drops the cached step graphs.            */
+int ssa_ukf_rollout_tasker(ssa_ukf* h, int tasker, double spoil_p);
 /* the float32 observation blocks of SSA_ROLLOUT_OBS_F32: pinned host mirror and device block, [N][12] floats          */
 int ssa_ukf_rollout_obs_f32(ssa_ukf* h, float** host, float** device);
 /* the 'aer' observation blocks of SSA_ROLLOUT_OBS_AER: pinned host mirror and device block, [N][4] doubles           */

@@ -23,6 +23,8 @@ STEP_CATALOG_STATS = 0x100
 N_TASKERS = 6
 (TASKER_NAIVE_GREEDY, TASKER_VISIBLE_GREEDY, TASKER_POS_ERROR_GREEDY, TASKER_VEL_ERROR_GREEDY, TASKER_VISIBLE_GREEDY_AER,
  TASKER_SHANNON) = range(6)
+TASKER_EXTERNAL = -1  # episodic mode only (ssa_ukf_rollout_tasker): the caller's actions, and the random agents
+TASKER_NAIVE_RANDOM, TASKER_VISIBLE_RANDOM, TASKER_VISIBLE_GREEDY_SPOILED = 6, 7, 8
 
 (F_X_TRUE, F_X_FILTER, F_P_FILTER, F_OBS, F_DELTA_POS, F_DELTA_VEL, F_SIGMA_POS, F_SIGMA_VEL, F_TRACE,
  F_Z_TRUE, F_Y, F_S, F_SIGMAS_H, F_Z_NOISE, F_VISIBLE, F_STATUS, F_INFLATIONS, F_ACTIONS, F_REWARD, F_DONE,
@@ -73,6 +75,7 @@ PROTOTYPES = {
     "ssa_ukf_rollout_io": (_I, [c_void_p] + [c_void_p] * 5),
     "ssa_ukf_rollout_reset": (_I, [c_void_p, c_void_p]),
     "ssa_ukf_rollout_step": (_I, [c_void_p, _I, c_void_p]),
+    "ssa_ukf_rollout_tasker": (_I, [c_void_p, _I, _D]),
     "ssa_ukf_rollout_obs_f32": (_I, [c_void_p, c_void_p, c_void_p]),
     "ssa_ukf_rollout_obs_aer": (_I, [c_void_p, c_void_p, c_void_p]),
     "ssa_ukf_rollout_episode_stats_enable": (_I, [c_void_p]),

@@ -14,6 +14,10 @@ The arrays read here (`env.P_filter[env.i]`, `env.delta_pos`, ...) were produced
 environments the argmax rules run on the device (`ssa_ukf_env_reduce`, SSA_TASKER_*), see vec_env.py; there
 agent_shannon's P_{i-1} is the covariance of the previous step index the reduction ran at, and a fresh episode (step 0)
 gets ratio 1 everywhere, as the reference's zeroed history row gives equal ratios.
+In the device-resident episodic mode all nine agents, the random ones included, also run inside the step graph
+(`VecSSATaskerEnv.set_tasker`, ssa_ukf_rollout_tasker): the device draws `action_space.sample()` and
+`np.random.choice` from counter-based Philox streams instead (same distributions, other streams; csrc/ssa_rng.h,
+ssa_tasker_pick).
 """
 import numpy as np
 

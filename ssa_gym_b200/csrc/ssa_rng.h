@@ -11,10 +11,12 @@
 #ifndef SSA_RNG_H
 #define SSA_RNG_H
 #include "ssa_math.h"
+#include "../../include/ssa_ukf.h"  // SSA_TASKER_*
 
 #define SSA_RNG_STREAM_ORBIT 0u
 #define SSA_RNG_STREAM_X 1u
 #define SSA_RNG_STREAM_Z 2u
+#define SSA_RNG_STREAM_ACT 3u
 
 struct ssa_u4 { uint32_t v[4]; };
 
@@ -72,6 +74,34 @@ SSA_HD void ssa_draw_z(uint32_t k0, uint32_t k1, uint32_t ep, uint32_t j, uint32
   ssa_normal2(ssa_philox4x32(ep, SSA_RNG_STREAM_Z | (1u << 8), j, step, k0, k1), &c, &d);
   (void)d;
   n3[0] = a; n3[1] = b; n3[2] = c;
+}
+
+// The action a device tasker (ssa_ukf_rollout_tasker) takes in environment (k0,k1), episode ep, for step `step`, from
+// the state the previous step left: greedy = the environment's row of the greedy block, vis = its m visibility flags.
+// One Philox block: v0 is action_space.sample() (uniform over m), v1 the choice among the visible objects, v2:v3 the
+// spoiled agent's uniform.  The candidates are empty where agents.py:37 `not np.any(idx)` holds: nothing visible, or
+// only object 0.  tasker: 0 .. SSA_TASKER_VISIBLE_GREEDY_SPOILED.
+SSA_HD int ssa_tasker_pick(uint32_t k0, uint32_t k1, uint32_t ep, uint32_t step, int m, int tasker, const int32_t* greedy,
+                           const uint8_t* vis, double spoil_p) {
+  const ssa_u4 r = ssa_philox4x32(ep, SSA_RNG_STREAM_ACT, 0u, step, k0, k1);
+  const int fallback = (int)ssa_mulhi32(r.v[0], (uint32_t)m);
+  if (tasker < SSA_N_TASKERS) return greedy[tasker] >= 0 ? greedy[tasker] : fallback;
+  if (tasker == SSA_TASKER_NAIVE_RANDOM) return fallback;
+  uint32_t n_vis = 0;
+  int any = 0;
+  for (int j = 0; j < m; ++j)
+    if (vis[j]) { n_vis += 1; any |= (j != 0); }
+  if (!any) return fallback;
+  if (tasker == SSA_TASKER_VISIBLE_RANDOM) {  // np.random.choice(idx): the k-th visible index in increasing order
+    uint32_t k = ssa_mulhi32(r.v[1], n_vis);
+    int j = 0;
+    for (;; ++j)
+      if (vis[j] && k-- == 0) break;
+    return j;
+  }
+  // SSA_TASKER_VISIBLE_GREEDY_SPOILED: np.random.choice([greedy, fallback], p=[1 - p, p]) is searchsorted(cdf, u,
+  // side='right'): the greedy pick for u < 1 - p
+  return ssa_u52(r.v[2], r.v[3]) < 1.0 - spoil_p ? greedy[SSA_TASKER_VISIBLE_GREEDY] : fallback;
 }
 
 #endif  // SSA_RNG_H

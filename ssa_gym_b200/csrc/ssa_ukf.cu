@@ -1225,14 +1225,17 @@ struct RolloutParams {
   const uint32_t* key;                        // [E][2] Philox key of each environment (from its seed)
   uint32_t* episode;                          // [E] resets performed so far
   int32_t* step_idx;                          // [E]
-  const int32_t* actions; int32_t* act_eff;   // [E] requested / effective (update_interval) actions
+  int32_t* actions; int32_t* act_eff;         // [E] requested / effective (update_interval) actions
   const uint8_t* done;                        // [E] reset mask (null: every environment)
   const double* sig;                          // x_sigma[6], z_sigma[3], packed P0[21]
   double* rew_hist; int32_t* spos_prev;       // 'shaped' reward state (EnvParams), null for the other rewards
+  const int32_t* greedy; const uint8_t* visible;  // greedy block [E][SSA_N_TASKERS], visibility [N] (device taskers)
+  int tasker; double spoil_p;                 // ssa_ukf_rollout_tasker (SSA_TASKER_EXTERNAL: the caller's actions)
   int E, m, update_interval, n_steps;
 };
 
-// start of a step: measurement noise of step i+1 for every object, effective action of every environment
+// start of a step: measurement noise of step i+1 for every object, the device tasker's pick (which replaces the
+// requested action) and the effective action of every environment
 __global__ void __launch_bounds__(128) k_env_begin(const RolloutParams p) {
   const long obj = (long)blockIdx.x * blockDim.x + threadIdx.x;
   if (obj >= (long)p.E * p.m) return;
@@ -1242,7 +1245,16 @@ __global__ void __launch_bounds__(128) k_env_begin(const RolloutParams p) {
   ssa_draw_z(p.key[2 * e], p.key[2 * e + 1], p.episode[e] - 1u, (uint32_t)j, (uint32_t)step, n3);
 #pragma unroll
   for (int a = 0; a < 3; ++a) p.z_noise[obj * 3 + a] = ssa_mul(n3[a], p.sig[6 + a]);
-  if (j == 0) p.act_eff[e] = (step % p.update_interval == 0) ? p.actions[e] : -1;  // SS2:292
+  if (j != 0) return;
+  int a;
+  if (p.tasker != SSA_TASKER_EXTERNAL) {
+    a = ssa_tasker_pick(p.key[2 * e], p.key[2 * e + 1], p.episode[e] - 1u, (uint32_t)step, p.m, p.tasker,
+                        p.greedy + (long)e * SSA_N_TASKERS, p.visible + obj, p.spoil_p);
+    p.actions[e] = a;
+  } else {
+    a = p.actions[e];
+  }
+  p.act_eff[e] = (step % p.update_interval == 0) ? a : -1;  // SS2:292
 }
 
 // (re)draw the environments whose done flag is set (all of them when p.done is null): SS2:193-221
@@ -1753,6 +1765,8 @@ struct ssa_ukf {
     double *daer, *haer;       // SSA_ROLLOUT_OBS_AER: the 'aer' observation [N][4] (device block, pinned host mirror)
     double* rew_hist;          // 'shaped' only: [E][n_steps] reward history, then spos_prev [E] int32
     int32_t* spos_prev;
+    int tasker;                // ssa_ukf_rollout_tasker
+    double spoil_p;
     cudaGraphExec_t gexec[6];  // [auto_reset + 2 * (obs_f32 ? 1 : obs_aer ? 2 : 0)]
     int gkernels[6];
   } ro;
@@ -2492,6 +2506,8 @@ static void rollout_params(ssa_ukf* h, RolloutParams* p, int only_done) {
   p->done = only_done ? (const uint8_t*)((int32_t*)(h->ro.dout + 12 * N + E) + SSA_N_TASKERS * E) : nullptr;
   p->sig = h->ro.sig;
   p->rew_hist = h->ro.rew_hist; p->spos_prev = h->ro.spos_prev;
+  p->greedy = (const int32_t*)(h->ro.dout + 12 * N + E); p->visible = h->visible;
+  p->tasker = h->ro.tasker; p->spoil_p = h->ro.spoil_p;
   p->E = h->cfg.n_envs; p->m = h->cfg.m; p->update_interval = h->ro.update_interval; p->n_steps = h->cfg.n_steps;
 }
 
@@ -2557,6 +2573,7 @@ int ssa_ukf_rollout_config(ssa_ukf* h, const double* orbits, int n_orbits, const
     memset(&h->es, 0, sizeof(h->es));
   }
   h->ro.n_orbits = n_orbits; h->ro.n_table = n_table; h->ro.update_interval = update_interval;
+  h->ro.tasker = SSA_TASKER_EXTERNAL; h->ro.spoil_p = 0.0;
   CK(cudaMalloc(&h->ro.dbuf, sizeof(double) * ((size_t)n_orbits * 6 + (size_t)n_table * 9 + 32)));
   h->ro.orbits = h->ro.dbuf; h->ro.table = h->ro.orbits + (size_t)n_orbits * 6; h->ro.sig = h->ro.table + (size_t)n_table * 9;
   CK(cudaMemcpy(h->ro.orbits, orbits, sizeof(double) * (size_t)n_orbits * 6, cudaMemcpyHostToDevice));
@@ -2878,8 +2895,8 @@ int ssa_ukf_rollout_step(ssa_ukf* h, int auto_reset, void* stream) {
   }
   const int ar = (auto_reset & 1) ? 1 : 0;
   const int a = ar + (obs_f32 ? 2 : obs_aer ? 4 : 0);
-  const bool device_io = (auto_reset & SSA_ROLLOUT_DEVICE_IO) != 0;
-  if (!device_io) CK(cudaMemcpyAsync(h->ro.act_in, h->ro.hin, sizeof(int32_t) * E, cudaMemcpyHostToDevice, st));
+  const bool device_io = (auto_reset & SSA_ROLLOUT_DEVICE_IO) != 0, tasked = h->ro.tasker != SSA_TASKER_EXTERNAL;
+  if (!device_io && !tasked) CK(cudaMemcpyAsync(h->ro.act_in, h->ro.hin, sizeof(int32_t) * E, cudaMemcpyHostToDevice, st));
   const char* gv = getenv("SSA_UKF_GRAPH");
   if (!(gv && strcmp(gv, "0") == 0) && !h->use_team) {
     if (!h->ro.gexec[a]) {
@@ -2917,7 +2934,24 @@ int ssa_ukf_rollout_step(ssa_ukf* h, int auto_reset, void* stream) {
     } else {
       CK(cudaMemcpyAsync(h->ro.hout, h->ro.dout, h->ro.out_bytes, cudaMemcpyDeviceToHost, st));
     }
+    if (tasked) CK(cudaMemcpyAsync(h->ro.hin, h->ro.act_in, sizeof(int32_t) * E, cudaMemcpyDeviceToHost, st));  // taken
   }
+  return SSA_OK;
+}
+
+int ssa_ukf_rollout_tasker(ssa_ukf* h, int tasker, double spoil_p) {
+  if (!h || !h->ro.init) { snprintf(g_err, sizeof(g_err), "episodic mode not configured"); return SSA_EINVAL; }
+  if (tasker < SSA_TASKER_EXTERNAL || tasker > SSA_TASKER_VISIBLE_GREEDY_SPOILED) {
+    snprintf(g_err, sizeof(g_err), "unknown tasker %d", tasker);
+    return SSA_EINVAL;
+  }
+  if (!(spoil_p >= 0.0 && spoil_p <= 1.0)) {  // (NaN fails both comparisons)
+    snprintf(g_err, sizeof(g_err), "spoil_p %g outside [0, 1]", spoil_p);
+    return SSA_EINVAL;
+  }
+  if (tasker != h->ro.tasker || spoil_p != h->ro.spoil_p) rollout_drop_graphs(h);  // (both are captured kernel parameters)
+  h->ro.tasker = tasker;
+  h->ro.spoil_p = spoil_p;
   return SSA_OK;
 }
 

@@ -286,6 +286,12 @@ class BatchedUKF:
             (_lib.ROLLOUT_OBS_AER if obs_aer else 0)
         _lib.check(self.lib.ssa_ukf_rollout_step(self.h, mode, stream), "ssa_ukf_rollout_step")
 
+    def rollout_tasker(self, tasker, spoil_p=0.25):
+        """Pick every environment's action inside the step graph (a TASKER_* id, include/ssa_ukf.h), TASKER_EXTERNAL for
+        the caller's actions.  spoil_p is TASKER_VISIBLE_GREEDY_SPOILED's probability of a random action.  After
+        rollout_config (which restores TASKER_EXTERNAL); the taken actions are in rollout_io['actions'] after a step."""
+        _lib.check(self.lib.ssa_ukf_rollout_tasker(self.h, int(tasker), float(spoil_p)), "ssa_ukf_rollout_tasker")
+
     def rollout_episode_stats_enable(self):
         """Accumulate per-episode statistics inside the step graph from the next rollout_reset on (after rollout_config,
         which turns them off again).  Records: rollout_episode_stats, or the device field F_ROLLOUT_EPISODE_STATS."""

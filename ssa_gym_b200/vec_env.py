@@ -21,17 +21,30 @@ rewards[:i]) in numpy's summation order), and the 'aer' layout is computed by th
 only its [E, m*4] rows (32 B per object instead of 96) cross PCIe and the host formats nothing.  With
 `config['episode_stats'] = True` the step graph also accumulates every episode's return, length and the reference's
 filter-consistency figures (ANEES, NIS, innovation bounds, Durbin-Watson statistics) on the device; a finished
-environment reports them in `infos[e]['episode']` (see `episode_info`).
+environment reports them in `infos[e]['episode']` (see `episode_info`).  `set_tasker(agent)` runs one of the nine
+agents of agents.py inside the step graph (device taskers, ssa_ukf_rollout_tasker): `vector_step()` then takes no
+actions, and a loop of `vector_step_device()` compares agents with no host round trip at all.
 """
 import numpy as np
 
-from . import _lib, dynamics
+from . import _lib, agents, dynamics
 from .episode import draw_episode
 from .gym_shim import seeding, spaces
 from .transformations import arcsec2rad, default_eops, deg2rad, gcrs2irts_matrix_b, lla2ecef, load_eop_c04, time_table
 from .ukf import BatchedUKF, Q_discrete_white_noise_block
 
 F = _lib
+
+
+# the agents of agents.py that the device runs (ssa_ukf_rollout_tasker), by function and by name
+_TASKERS = {
+    agents.agent_naive_greedy: F.TASKER_NAIVE_GREEDY, agents.agent_visible_greedy: F.TASKER_VISIBLE_GREEDY,
+    agents.agent_pos_error_greedy: F.TASKER_POS_ERROR_GREEDY, agents.agent_vel_error_greedy: F.TASKER_VEL_ERROR_GREEDY,
+    agents.agent_visible_greedy_aer: F.TASKER_VISIBLE_GREEDY_AER, agents.agent_shannon: F.TASKER_SHANNON,
+    agents.agent_naive_random: F.TASKER_NAIVE_RANDOM, agents.agent_visible_random: F.TASKER_VISIBLE_RANDOM,
+    agents.agent_visible_greedy_spoiled: F.TASKER_VISIBLE_GREEDY_SPOILED,
+}
+_TASKER_NAMES = {f.__name__[len("agent_"):]: k for f, k in _TASKERS.items()}
 
 
 def episode_info(rec):
@@ -125,6 +138,8 @@ class VecSSATaskerEnv:
         self.episodes = np.zeros(self.E, dtype=np.int64)
         self._P0_packed = self.P_0[np.triu_indices(6)]
         self._views = None
+        self.tasker = F.TASKER_EXTERNAL
+        self.last_actions = np.zeros(self.E, dtype=np.int64)  # the actions the last vector_step took
         self.seed(seeds)
         # device mode, 'aer': the observation rows are computed on the device (SSA_ROLLOUT_OBS_AER), not by _format_obs
         self._obs_aer = rng == 'device' and self.obs_returned == 'aer'
@@ -229,11 +244,42 @@ class VecSSATaskerEnv:
         self.episodes[e] += 1
 
     # -- step ---------------------------------------------------------------------------------------------
-    def vector_step(self, actions):
+    def set_tasker(self, agent, p=0.25):
+        """Run `agent` inside the step graph (rng='device'): one of the nine functions of agents.py, or its name without
+        the 'agent_' prefix ('visible_greedy', 'naive_random', ...); None returns to the caller's actions.  p is
+        agent_visible_greedy_spoiled's probability of a random action.  Each step then picks every environment's action
+        from the state the previous step left (the greedy block, the visibility flags), with the reference's
+        distributions and counter-based random streams (include/ssa_ukf.h, ssa_ukf_rollout_tasker).  Any other callable
+        raises ValueError: there is no host fallback."""
+        if self.rng != 'device':
+            raise ValueError("device taskers need rng='device'")
+        if agent is None:
+            tasker = F.TASKER_EXTERNAL
+        elif isinstance(agent, str):
+            if agent not in _TASKER_NAMES:
+                raise ValueError(f"unknown agent {agent!r}; device taskers: {sorted(_TASKER_NAMES)}")
+            tasker = _TASKER_NAMES[agent]
+        else:
+            tasker = next((k for f, k in _TASKERS.items() if f is agent), None)
+        if tasker is None:
+            raise ValueError(f"{agent!r} is not an agent of ssa_gym_b200.agents: the device runs only those")
+        self.ukf.rollout_tasker(tasker, p)
+        self.tasker = tasker
+
+    def vector_step(self, actions=None):
+        """One step of every environment with `actions` [E]; with a tasker set (set_tasker) the device picks them and
+        `actions` must be None.  `last_actions` holds the actions the step took."""
+        if self.tasker != F.TASKER_EXTERNAL:
+            if actions is not None:
+                raise ValueError("a device tasker is set (set_tasker): vector_step takes no actions")
+            return self._device_step(None)
+        if actions is None:
+            raise ValueError("vector_step needs actions (or a device tasker, set_tasker)")
         actions = np.ascontiguousarray(actions, dtype=np.int32).reshape(self.E)
         assert np.all((actions >= 0) & (actions < self.m)), "invalid action"
         if self.rng == 'device':
             return self._device_step(actions)
+        self.last_actions = actions.astype(np.int64)
         self.i += 1
         idx = self.i
         ar = np.arange(self.E)
@@ -283,12 +329,15 @@ class VecSSATaskerEnv:
     def _device_step(self, actions):
         """rng='device': the whole step (noise, UKF, reward / done, auto-reset, fresh obs, greedy taskers) is one
         H2D copy of the actions, one CUDA-graph launch and one D2H copy (ssa_ukf_rollout_step).  The returned obs
-        is a VIEW of the handle's pinned output block: it is overwritten by the next step."""
+        is a VIEW of the handle's pinned output block: it is overwritten by the next step.  actions None: a device
+        tasker picks them, and the step copies them back into the same block."""
         io = self._io
-        io["actions"][:] = actions
+        if actions is not None:
+            io["actions"][:] = actions
         f32 = self.obs_dtype == np.float32
         self.ukf.rollout_step(self.auto_reset, obs_f32=f32, obs_aer=self._obs_aer)
         self.ukf.sync()
+        self.last_actions = io["actions"].astype(np.int64)
         dones = io["done"].astype(bool)
         rewards = io["reward"].copy()
         self.i += 1
@@ -314,7 +363,7 @@ class VecSSATaskerEnv:
     # -- device-resident consumer (a policy on the same GPU): no host copies, nothing synchronises -------------------
     def device_views(self):
         """Zero-copy torch tensors over the episodic mode's device buffers: 'actions' int32 [E] (INPUT of
-        vector_step_device), 'obs' float64 [E, m*12] ([E, m*4] for obs_returned='aer'), 'reward' float64 [E], 'done' uint8
+        vector_step_device; with a device tasker its output, the actions the step took), 'obs' float64 [E, m*12] ([E, m*4] for obs_returned='aer'), 'reward' float64 [E], 'done' uint8
         [E], 'greedy' int32 [E, taskers].
         With config['episode_stats']: 'episode_stats' float64 [E, EPISODE_STATS_DOUBLES], the record of each environment's
         last finished episode (layout: include/ssa_ukf.h; episode_info turns a row into the infos entry), valid after a
