@@ -106,6 +106,8 @@ enum ssa_field {
   SSA_F_ROLLOUT_GREEDY = 33,  /* int32 [E][SSA_N_TASKERS] of the episodic output block                             */
   SSA_F_ROLLOUT_OBS_AER = 34, /* double [N][4]: the episodic mode's 'aer' observation block (SSA_ROLLOUT_OBS_AER)     */
   SSA_F_ROLLOUT_EPISODE_STATS = 35, /* double [E][SSA_EPISODE_STATS_DOUBLES]: episode records (ssa_ukf_rollout_episode_stats_*) */
+  SSA_F_ROLLOUT_TERMINAL_OBS = 36,  /* double: final observations of finished episodes (ssa_ukf_rollout_terminal_obs_download) */
+  SSA_F_ROLLOUT_TRUNCATED = 37,     /* uint8 [E]: done raised by the step limit alone (ssa_ukf_rollout_truncated)          */
   SSA_F_COUNT_
 };
 
@@ -220,7 +222,8 @@ int ssa_ukf_host_stats(ssa_ukf* h, int parity, double** stats_host, double** sta
  *   rollout_config  catalog [n_orbits][6], trans_matrix table [n_table][9] (row i = step i), one 64-bit seed per env,
  *                   x_sigma[6], z_sigma[3] (radians / metres), P0[36], update_interval
  *   rollout_io      pinned host blocks owned by the handle: actions [E] (in); obs [N][12], reward [E],
- *                   greedy [E][SSA_N_TASKERS], done [E] (out)
+ *                   greedy [E][SSA_N_TASKERS], done [E] (out); truncated [E] follows in the same block
+ *                   (ssa_ukf_rollout_truncated)
  *   rollout_reset   draw every environment, step index 0; outputs: obs, greedy, and the 'aer' block of
  *                   ssa_ukf_rollout_obs_aer
  *   rollout_step    one step of every environment with the actions in the pinned block: ONE H2D copy, ONE CUDA-graph
@@ -299,6 +302,33 @@ int ssa_ukf_rollout_obs_aer(ssa_ukf* h, double** host, double** device);
 #define SSA_EPISODE_STATS_DOUBLES 23
 int ssa_ukf_rollout_episode_stats_enable(ssa_ukf* h);
 int ssa_ukf_rollout_episode_stats_download(ssa_ukf* h, const int32_t* envs, int n, double* out, void* stream);
+/* Episode boundaries of the episodic mode: why an episode ended, its final observation, and the reset of chosen
+ * environments (the RLlib VectorEnv reset_at).
+ *   truncated        uint8 [E] written by every step next to done: 1 when done was raised by the step limit alone
+ *                    (i + 1 >= n_steps), 0 otherwise.  gym's TimeLimit rule: a lost (max delta_pos > 5e6) or successful
+ *                    (< 3e4) last step is a termination; with 'trinary', which ends at the step limit only, it equals
+ *                    done.  The block follows done in the output block, so the step's D2H copy carries it: pinned host
+ *                    mirror and device block (also SSA_F_ROLLOUT_TRUNCATED).
+ *   terminal_obs     with auto-reset, the step's observation rows of every finished environment before its re-draw, for a
+ *                    learner that bootstraps the value of a truncated episode: double [E][m][12], or [E][m][4] (the 'aer'
+ *                    rows of SSA_ROLLOUT_OBS_AER at the step index the episode ended on) when the step ran with
+ *                    SSA_ROLLOUT_OBS_AER.  Written inside the step graph (no extra launch); the row of an environment is
+ *                    valid, in stream order, after an auto-reset step whose done flag is set for it.  Without auto-reset
+ *                    it is not written: the step's own obs are the final ones.  The download copies the rows of n
+ *                    environments envs[0..n) into out[n][m * 12] (or [n][m * 4], the layout of the last auto-reset step)
+ *                    and blocks until copied; the device block is SSA_F_ROLLOUT_TERMINAL_OBS ([E][m][4] in its first
+ *                    4 N doubles in the 'aer' layout).
+ *   reset_envs       ssa_ukf_rollout_reset restricted to the n environments envs[0..n): each is re-drawn (episode counter
+ *                    + 1, step index 0, 'shaped' reward history cleared), its obs, errors, visibility, agent_shannon
+ *                    history and greedy columns refreshed, the 'aer' block recomputed; with live episode statistics its
+ *                    accumulators are cleared (its next record covers the new episode only).  The other environments keep
+ *                    their state and outputs.  Asynchronous like rollout_reset: the output and 'aer' blocks are copied to
+ *                    the host and valid after a synchronize.
+ * All three return SSA_EINVAL before ssa_ukf_rollout_config; the download and reset_envs also for n outside 0 .. E, a
+ * null list with n > 0, and an index outside 0 .. E - 1.                                                             */
+int ssa_ukf_rollout_truncated(ssa_ukf* h, uint8_t** host, uint8_t** device);
+int ssa_ukf_rollout_terminal_obs_download(ssa_ukf* h, const int32_t* envs, int n, double* out, void* stream);
+int ssa_ukf_rollout_reset_envs(ssa_ukf* h, const int32_t* envs, int n, void* stream);
 /* make `stream` wait for every outstanding internal copy of ssa_ukf_step_host / ssa_ukf_step_pinned */
 int ssa_ukf_host_join(ssa_ukf* h, void* stream);
 /* Convenience wrappers with the reference's call structure */

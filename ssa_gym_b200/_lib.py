@@ -30,7 +30,7 @@ TASKER_NAIVE_RANDOM, TASKER_VISIBLE_RANDOM, TASKER_VISIBLE_GREEDY_SPOILED = 6, 7
  F_Z_TRUE, F_Y, F_S, F_SIGMAS_H, F_Z_NOISE, F_VISIBLE, F_STATUS, F_INFLATIONS, F_ACTIONS, F_REWARD, F_DONE,
  F_GREEDY, F_SCORES, F_UPDATED, F_TRANS_ENV, F_STEP_INDEX, F_ENV_STATS, F_DIAG, F_INNOV_FLAGS, F_CATALOG_STATS,
  F_ROLLOUT_OBS, F_ROLLOUT_REWARD, F_ROLLOUT_ACTIONS, F_ROLLOUT_DONE, F_ROLLOUT_GREEDY, F_ROLLOUT_OBS_AER,
- F_ROLLOUT_EPISODE_STATS) = range(36)
+ F_ROLLOUT_EPISODE_STATS, F_ROLLOUT_TERMINAL_OBS, F_ROLLOUT_TRUNCATED) = range(38)
 ROLLOUT_DEVICE_IO = 2
 ROLLOUT_OBS_F32 = 4
 ROLLOUT_OBS_AER = 8
@@ -80,6 +80,9 @@ PROTOTYPES = {
     "ssa_ukf_rollout_obs_aer": (_I, [c_void_p, c_void_p, c_void_p]),
     "ssa_ukf_rollout_episode_stats_enable": (_I, [c_void_p]),
     "ssa_ukf_rollout_episode_stats_download": (_I, [c_void_p, c_void_p, _I, c_void_p, c_void_p]),
+    "ssa_ukf_rollout_truncated": (_I, [c_void_p, c_void_p, c_void_p]),
+    "ssa_ukf_rollout_terminal_obs_download": (_I, [c_void_p, c_void_p, _I, c_void_p, c_void_p]),
+    "ssa_ukf_rollout_reset_envs": (_I, [c_void_p, c_void_p, _I, c_void_p]),
     "ssa_trans_matrix_table": (_I, [_I, _I, _I, _D, _D, _I, c_void_p, _I, c_void_p]),
     "ssa_ukf_predict": (_I, [c_void_p, c_void_p]),
     "ssa_ukf_update": (_I, [c_void_p, c_void_p, _I, c_void_p]),

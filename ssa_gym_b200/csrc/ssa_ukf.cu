@@ -38,6 +38,7 @@
 #include <algorithm>
 #include <new>
 #include <numeric>
+#include <vector>
 
 #include <cuda.h>
 #include <utility>
@@ -1038,6 +1039,7 @@ struct EnvParams {
   double* rew_hist;           // [E][n_steps] rewards of the running episode, entry 0 = 0 (np.sum(rewards[:i]), SS2:345)
   int32_t* spos_prev;         // [E] argmax sigma_pos of the environment's previous step (SS2:348)
   const int32_t* act_in;      // [E] REQUESTED actions (SS2:348 compares them also on steps update_interval skips)
+  uint8_t* truncated;         // [E] episodic mode: done raised by the step limit alone (null outside that mode)
 };
 
 
@@ -1213,6 +1215,9 @@ __device__ __forceinline__ void env_reduce_body(const EnvParams& p, const int e)
     if (step_i + 1 >= p.n_steps) done = 1;  // SS2:353-354
     p.reward[e] = reward;
     p.done[e] = (uint8_t)done;
+    // gym's TimeLimit rule: a lost or successful last step is a termination; 'trinary' ends at the step limit only
+    if (p.truncated)
+      p.truncated[e] = (uint8_t)(done && (p.reward_type == SSA_REWARD_TRINARY || !(max_dpos > 5e6 || max_dpos < 3e4)));
   }
 }
 
@@ -1232,7 +1237,42 @@ struct RolloutParams {
   const int32_t* greedy; const uint8_t* visible;  // greedy block [E][SSA_N_TASKERS], visibility [N] (device taskers)
   int tasker; double spoil_p;                 // ssa_ukf_rollout_tasker (SSA_TASKER_EXTERNAL: the caller's actions)
   int E, m, update_interval, n_steps;
+  // final observations of the environments an auto-reset re-draws (env_terminal_rows); term null: not recorded
+  const double* obs;                          // [N][12] observation rows of the output block
+  double* term;                               // [E][m][12], or [E][m][4] with term_aer
+  int term_aer;
+  const double* table; int n_table;           // trans_matrix table (the 'aer' rows)
+  ssa_obs ob;                                 // observer constants (M unused)
 };
+
+// the 'aer' observation of one object (SS2:834-840, vec_env.py _format_obs) from its [12] observation row: az / el /
+// range of the filter mean x[0..2] through the trans_matrix M, np.trace's left-to-right sum of the diag P columns, and
+// nan_to_num(nan = +-inf = 0.001) of the four values
+__device__ __forceinline__ void obs_aer_row(const double* o, const double* M, const ssa_obs& ob, double* out) {
+  double x[3], v[4];
+#pragma unroll
+  for (int k = 0; k < 3; ++k) x[k] = o[k];
+  ssa_hx_aer_m<false>(x, M, ob.obs_itrs, ob.T, v);
+  v[3] = ((((o[6] + o[7]) + o[8]) + o[9]) + o[10]) + o[11];
+#pragma unroll
+  for (int k = 0; k < 4; ++k) out[k] = (v[k] - v[k] == 0.0) ? v[k] : 0.001;
+}
+
+// the final observation of finished environment e, in the layout of the step, before env_reset_body re-draws it: its
+// obs rows, or their 'aer' rows at the step index the episode ended on (read before env_reset_body zeroes it)
+__device__ __forceinline__ void env_terminal_rows(const RolloutParams& p, const int e) {
+  const int i = p.step_idx[e];
+  const double* M = p.table + (long)(i < p.n_table - 1 ? i : p.n_table - 1) * 9;
+  for (int j = threadIdx.x; j < p.m; j += blockDim.x) {
+    const long obj = (long)e * p.m + j;
+    if (p.term_aer) {
+      obs_aer_row(p.obs + obj * 12, M, p.ob, p.term + obj * 4);
+    } else {
+#pragma unroll
+      for (int k = 0; k < 12; ++k) p.term[obj * 12 + k] = p.obs[obj * 12 + k];
+    }
+  }
+}
 
 // start of a step: measurement noise of step i+1 for every object, the device tasker's pick (which replaces the
 // requested action) and the effective action of every environment
@@ -1262,6 +1302,7 @@ __device__ __forceinline__ void env_reset_body(const RolloutParams& p, const int
 __global__ void __launch_bounds__(128) k_env_reset(const RolloutParams p) {
   const int e = blockIdx.x;
   if (p.done && !p.done[e]) return;
+  if (p.term) env_terminal_rows(p, e);
   env_reset_body(p, e);
 }
 __device__ __forceinline__ void env_reset_body(const RolloutParams& p, const int e) {
@@ -1757,7 +1798,7 @@ struct ssa_ukf {
     uint32_t* ibuf;      // device: key [E][2], episode [E], act_in [E], act_eff [E]
     uint32_t *key, *episode;
     int32_t *act_in, *act_eff;
-    double* dout;        // device out block: [obs 12N][reward E][greedy 4E int32][done E uint8]
+    double* dout;        // device out block: [obs 12N][reward E][greedy 6E int32][done E uint8][truncated E uint8]
     double* hout;        // pinned host mirror
     int32_t* hin;        // pinned host actions [E]
     size_t out_bytes;
@@ -1767,6 +1808,14 @@ struct ssa_ukf {
     int32_t* spos_prev;
     int tasker;                // ssa_ukf_rollout_tasker
     double spoil_p;
+    // final observations (ssa_ukf_rollout_terminal_obs_download) and ssa_ukf_rollout_reset_envs
+    double* tbuf;              // device: terminal [12N], gathered rows [12N], then idx [E] int32, mask [E] uint8
+    double *term, *tgath;
+    int32_t* tidx;
+    uint8_t* mask;
+    double* htbuf;             // pinned: gathered rows [12N], then idx [E] int32
+    int32_t* htidx;
+    int term_w;                // doubles per object of the terminal rows: 12, 4 after an SSA_ROLLOUT_OBS_AER auto-reset step
     cudaGraphExec_t gexec[6];  // [auto_reset + 2 * (obs_f32 ? 1 : obs_aer ? 2 : 0)]
     int gkernels[6];
   } ro;
@@ -1945,8 +1994,9 @@ int ssa_ukf_destroy(ssa_ukf* h) {
   for (int i = 0; i < h->sg.n; ++i) { cudaGraphExecDestroy(h->sg.gexec[i]); cudaGraphDestroy(h->sg.graph[i]); }
   if (h->ro.init) {
     cudaFree(h->ro.dbuf); cudaFree(h->ro.ibuf); cudaFree(h->ro.dout); cudaFree(h->ro.dobs32);
-    cudaFree(h->ro.daer); cudaFree(h->ro.rew_hist);
+    cudaFree(h->ro.daer); cudaFree(h->ro.rew_hist); cudaFree(h->ro.tbuf);
     cudaFreeHost(h->ro.hout); cudaFreeHost(h->ro.hin); cudaFreeHost(h->ro.hobs32); cudaFreeHost(h->ro.haer);
+    cudaFreeHost(h->ro.htbuf);
     for (int i = 0; i < 6; ++i) if (h->ro.gexec[i]) cudaGraphExecDestroy(h->ro.gexec[i]);
   }
   if (h->es.on) { cudaFree(h->es.buf); cudaFreeHost(h->es.hbuf); }
@@ -2053,6 +2103,12 @@ static int field_info(ssa_ukf* h, int field, void** p, size_t* bytes, int* soa_c
     case SSA_F_ROLLOUT_EPISODE_STATS:
       if (!h->es.on) { snprintf(g_err, sizeof(g_err), "episode statistics not enabled"); return SSA_EINVAL; }
       *p = h->es.rec; *bytes = E * SSA_EPR * 8; break;
+    case SSA_F_ROLLOUT_TERMINAL_OBS:
+      if (!h->ro.init) { snprintf(g_err, sizeof(g_err), "episodic mode not configured"); return SSA_EINVAL; }
+      *p = h->ro.term; *bytes = N * 12 * 8; break;
+    case SSA_F_ROLLOUT_TRUNCATED:
+      if (!h->ro.init) { snprintf(g_err, sizeof(g_err), "episodic mode not configured"); return SSA_EINVAL; }
+      *p = (uint8_t*)((int32_t*)(h->ro.dout + 12 * N + E) + SSA_N_TASKERS * E) + ((E + 7) / 8) * 8; *bytes = E; break;
     default: snprintf(g_err, sizeof(g_err), "unknown field %d", field); return SSA_EINVAL;
   }
   return SSA_OK;
@@ -2509,6 +2565,11 @@ static void rollout_params(ssa_ukf* h, RolloutParams* p, int only_done) {
   p->greedy = (const int32_t*)(h->ro.dout + 12 * N + E); p->visible = h->visible;
   p->tasker = h->ro.tasker; p->spoil_p = h->ro.spoil_p;
   p->E = h->cfg.n_envs; p->m = h->cfg.m; p->update_interval = h->ro.update_interval; p->n_steps = h->cfg.n_steps;
+  p->obs = h->ro.dout; p->term = nullptr; p->term_aer = 0;
+  p->table = h->ro.table; p->n_table = h->ro.n_table;
+  memset(&p->ob, 0, sizeof(p->ob));
+  memcpy(p->ob.obs_itrs, h->cfg.obs_itrs, sizeof(p->ob.obs_itrs));
+  memcpy(p->ob.T, h->cfg.T, sizeof(p->ob.T));
 }
 
 static void rollout_env_params(ssa_ukf* h, EnvParams* p, int increment, int greedy_only) {
@@ -2523,6 +2584,7 @@ static void rollout_env_params(ssa_ukf* h, EnvParams* p, int increment, int gree
   p->P = h->P; p->ld = h->ld; p->det_prev = h->det_prev; p->det_last = h->det_last; p->det_step = h->det_step;
   p->det_cur = h->det_cur; p->reset_mask = nullptr;
   p->rew_hist = h->ro.rew_hist; p->spos_prev = h->ro.spos_prev; p->act_in = h->ro.act_in;
+  p->truncated = p->done + ((E + 7) / 8) * 8;
 }
 
 static void launch_env_reduce(ssa_ukf* h, const EnvParams& ep, cudaStream_t st) {
@@ -2540,13 +2602,14 @@ static void launch_env_reduce(ssa_ukf* h, const EnvParams& ep, cudaStream_t st) 
   h->launches += 2;
 }
 
-// obs / errors / visibility of the current states + greedy taskers (after a reset)
-static int rollout_refresh(ssa_ukf* h, cudaStream_t st, int only_done) {
+// obs / errors / visibility of the current states + greedy taskers (after a reset) of the environments in `mask` (the
+// ones k_env_reset has just re-drawn; null: every environment)
+static int rollout_refresh(ssa_ukf* h, cudaStream_t st, const uint8_t* mask) {
   EnvParams ep;
   rollout_env_params(h, &ep, 0, 1);
-  if (only_done) ep.reset_mask = ep.done;  // the environments k_env_reset has just re-drawn
+  ep.reset_mask = mask;
   // (observations, visibility, determinants and greedy actions of the other environments are this step's already)
-  StepOverride ov{h->ro.dout, h->ro.act_eff, h->ro.table, h->step_idx, 0, h->ro.n_table, only_done ? ep.done : nullptr};
+  StepOverride ov{h->ro.dout, h->ro.act_eff, h->ro.table, h->step_idx, 0, h->ro.n_table, mask};
   int rc = step_impl(h, nullptr, SSA_STEP_EPILOGUE, st, nullptr, -1, &ov);
   if (rc) return rc;
   launch_env_reduce(h, ep, st);
@@ -2565,6 +2628,7 @@ int ssa_ukf_rollout_config(ssa_ukf* h, const double* orbits, int n_orbits, const
     cudaFree(h->ro.dbuf); cudaFree(h->ro.ibuf); cudaFree(h->ro.dout); cudaFreeHost(h->ro.hout); cudaFreeHost(h->ro.hin);
     cudaFree(h->ro.dobs32); cudaFreeHost(h->ro.hobs32);
     cudaFree(h->ro.daer); cudaFreeHost(h->ro.haer); cudaFree(h->ro.rew_hist);
+    cudaFree(h->ro.tbuf); cudaFreeHost(h->ro.htbuf);
     for (int i = 0; i < 6; ++i) if (h->ro.gexec[i]) { cudaGraphExecDestroy(h->ro.gexec[i]); h->ro.gexec[i] = nullptr; }
     h->ro.init = 0;
   }
@@ -2588,7 +2652,7 @@ int ssa_ukf_rollout_config(ssa_ukf* h, const double* orbits, int n_orbits, const
   h->ro.key = h->ro.ibuf; h->ro.episode = h->ro.key + 2 * E;
   h->ro.act_in = (int32_t*)(h->ro.episode + E); h->ro.act_eff = h->ro.act_in + E;
   CK(cudaMemcpy(h->ro.key, seeds, sizeof(uint64_t) * E, cudaMemcpyHostToDevice));  // little-endian: key[2e] = low word
-  h->ro.out_bytes = sizeof(double) * (12 * N + E) + sizeof(int32_t) * SSA_N_TASKERS * E + ((E + 7) / 8) * 8;
+  h->ro.out_bytes = sizeof(double) * (12 * N + E) + sizeof(int32_t) * SSA_N_TASKERS * E + 2 * (((E + 7) / 8) * 8);
   CK(cudaMalloc(&h->ro.dout, h->ro.out_bytes));
   CK(cudaMemset(h->ro.dout, 0, h->ro.out_bytes));
   CK(cudaHostAlloc(&h->ro.hout, h->ro.out_bytes, cudaHostAllocDefault));
@@ -2610,6 +2674,14 @@ int ssa_ukf_rollout_config(ssa_ukf* h, const double* orbits, int n_orbits, const
     CK(cudaMemset(h->ro.rew_hist, 0, hist + sizeof(int32_t) * E));
     h->ro.spos_prev = (int32_t*)((char*)h->ro.rew_hist + hist);
   }
+  const size_t tbytes = sizeof(double) * 24 * N + sizeof(int32_t) * E + E;
+  CK(cudaMalloc(&h->ro.tbuf, tbytes));
+  CK(cudaMemset(h->ro.tbuf, 0, tbytes));
+  h->ro.term = h->ro.tbuf; h->ro.tgath = h->ro.term + 12 * N;
+  h->ro.tidx = (int32_t*)(h->ro.tgath + 12 * N); h->ro.mask = (uint8_t*)(h->ro.tidx + E);
+  CK(cudaHostAlloc(&h->ro.htbuf, sizeof(double) * 12 * N + sizeof(int32_t) * E, cudaHostAllocDefault));
+  h->ro.htidx = (int32_t*)(h->ro.htbuf + 12 * N);
+  h->ro.term_w = 12;
   for (int i = 0; i < 6; ++i) h->ro.gexec[i] = nullptr;
   h->ro.init = 1;
   return SSA_OK;
@@ -2646,7 +2718,7 @@ int ssa_ukf_rollout_reset(ssa_ukf* h, void* stream) {
   rollout_params(h, &rp, 0);
   k_env_reset<<<(unsigned)rp.E, 128, 0, st>>>(rp);
   h->launches++;
-  int rc = rollout_refresh(h, st, 0);
+  int rc = rollout_refresh(h, st, nullptr);
   if (rc) return rc;
   launch_obs_aer(h, st);  // (the 'aer' rows of the fresh episodes, whichever layout the steps will use)
   CK(cudaMemcpyAsync(h->ro.hout, h->ro.dout, h->ro.out_bytes, cudaMemcpyDeviceToHost, st));
@@ -2665,6 +2737,7 @@ int ssa_ukf_rollout_reset(ssa_ukf* h, void* stream) {
 __global__ void __launch_bounds__(128) k_env_refresh(const RolloutParams rp, const KParams p, const EnvParams ep) {
   const int e = blockIdx.x;
   if (!rp.done[e]) return;
+  env_terminal_rows(rp, e);  // (the step graphs with auto-reset always record the final observations)
   env_reset_body(rp, e);  // (ends with thread 0 advancing the episode counter and zeroing the step index)
   __syncthreads();
   for (int j = threadIdx.x; j < rp.m; j += blockDim.x) {
@@ -2690,24 +2763,15 @@ __global__ void __launch_bounds__(256) k_obs_to_f32(const double2* __restrict__ 
   }
 }
 
-// SSA_ROLLOUT_OBS_AER: the 'aer' observation of every object (SS2:834-840, vec_env.py _format_obs), one thread per object:
-// az / el / range of the filter mean x[0..2] through the environment's trans_matrix row min(step_idx, n_table - 1) (its
-// row of the step just taken, step 0 after a re-draw), np.trace's left-to-right sum of the diag P columns, and
-// nan_to_num(nan = +-inf = 0.001) of the four values.
+// SSA_ROLLOUT_OBS_AER: the 'aer' observation of every object (obs_aer_row), one thread per object, through the
+// environment's trans_matrix row min(step_idx, n_table - 1) (its row of the step just taken, step 0 after a re-draw).
 __global__ void __launch_bounds__(128) k_obs_aer(const double* __restrict__ obs, const int32_t* __restrict__ step_idx,
                                                  const double* __restrict__ table, int n_table, const ssa_obs ob, int m, long N,
                                                  double* __restrict__ out) {
   const long n = (long)blockIdx.x * blockDim.x + threadIdx.x;
   if (n >= N) return;
   const int i = step_idx[n / m];
-  const double* o = obs + n * 12;
-  double x[3], v[4];
-#pragma unroll
-  for (int k = 0; k < 3; ++k) x[k] = o[k];
-  ssa_hx_aer_m<false>(x, table + (long)(i < n_table - 1 ? i : n_table - 1) * 9, ob.obs_itrs, ob.T, v);
-  v[3] = ((((o[6] + o[7]) + o[8]) + o[9]) + o[10]) + o[11];
-#pragma unroll
-  for (int k = 0; k < 4; ++k) out[n * 4 + k] = (v[k] - v[k] == 0.0) ? v[k] : 0.001;
+  obs_aer_row(obs + n * 12, table + (long)(i < n_table - 1 ? i : n_table - 1) * 9, ob, out + n * 4);
 }
 
 static void launch_obs_aer(ssa_ukf* h, cudaStream_t st) {
@@ -2774,10 +2838,11 @@ __global__ void __launch_bounds__(128) k_ep_step(const EpParams p) {
   }
 }
 
-__global__ void __launch_bounds__(256) k_ep_gather(const double* __restrict__ rec, const int32_t* __restrict__ idx, int n,
-                                                   double* __restrict__ out) {
-  const int t = blockIdx.x * blockDim.x + threadIdx.x;
-  if (t < n * SSA_EPR) out[t] = rec[(long)idx[t / SSA_EPR] * SSA_EPR + t % SSA_EPR];
+// rows idx[0 .. n) of `row` doubles each, packed into out (the downloads of episode records and final observations)
+__global__ void __launch_bounds__(256) k_gather_rows(const double* __restrict__ src, const int32_t* __restrict__ idx, int n,
+                                                     long row, double* __restrict__ out) {
+  const long t = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t < n * row) out[t] = src[(long)idx[t / row] * row + t % row];
 }
 
 static int rollout_chain(ssa_ukf* h, cudaStream_t st, int auto_reset, int obs_f32, int obs_aer) {
@@ -2800,6 +2865,7 @@ static int rollout_chain(ssa_ukf* h, cudaStream_t st, int auto_reset, int obs_f3
   EnvParams ep;
   rollout_env_params(h, &ep, 1, 0);
   launch_env_reduce(h, ep, st);
+  if (auto_reset) { rp.term = h->ro.term; rp.term_aer = obs_aer; }  // (k_env_refresh / k_env_reset record them)
   if (stats) {
     k_ep_step<<<(unsigned)((rp.E + 3) / 4), 128, 0, st>>>(sp);
     h->launches++;
@@ -2818,7 +2884,7 @@ static int rollout_chain(ssa_ukf* h, cudaStream_t st, int auto_reset, int obs_f3
   } else if (auto_reset) {  // SSA_UKF_REFRESH_CHAIN=1 / team kernel: k_env_reset, then the gated refresh chain
     k_env_reset<<<(unsigned)rp.E, 128, 0, st>>>(rp);
     h->launches++;
-    rc = rollout_refresh(h, st, 1);
+    rc = rollout_refresh(h, st, rp.done);
     if (rc) return rc;
   }
   if (obs_f32) {
@@ -2862,24 +2928,92 @@ int ssa_ukf_rollout_episode_stats_enable(ssa_ukf* h) {
   return SSA_OK;
 }
 
-int ssa_ukf_rollout_episode_stats_download(ssa_ukf* h, const int32_t* envs, int n, double* out, void* stream) {
-  if (!h) return SSA_EINVAL;
-  if (!h->es.on) { snprintf(g_err, sizeof(g_err), "episode statistics not enabled"); return SSA_EINVAL; }
+// the environment list of a download / reset: 0 <= n <= E entries, each in [0, E) (and, for a download, an output)
+static int check_envs(const ssa_ukf* h, const int32_t* envs, int n, const void* out) {
   const int E = h->cfg.n_envs;
   if (n < 0 || n > E || (n > 0 && (!envs || !out))) { snprintf(g_err, sizeof(g_err), "bad environment list"); return SSA_EINVAL; }
   for (int k = 0; k < n; ++k)
     if (envs[k] < 0 || envs[k] >= E) { snprintf(g_err, sizeof(g_err), "environment index %d out of range", envs[k]); return SSA_EINVAL; }
+  return SSA_OK;
+}
+
+int ssa_ukf_rollout_episode_stats_download(ssa_ukf* h, const int32_t* envs, int n, double* out, void* stream) {
+  if (!h) return SSA_EINVAL;
+  if (!h->es.on) { snprintf(g_err, sizeof(g_err), "episode statistics not enabled"); return SSA_EINVAL; }
+  if (check_envs(h, envs, n, out)) return SSA_EINVAL;
   if (n == 0) return SSA_OK;
   CK(cudaSetDevice(h->device));
   cudaStream_t st = (cudaStream_t)stream;
   memcpy(h->es.hidx, envs, sizeof(int32_t) * n);
   CK(cudaMemcpyAsync(h->es.didx, h->es.hidx, sizeof(int32_t) * n, cudaMemcpyHostToDevice, st));
-  k_ep_gather<<<(unsigned)((n * SSA_EPR + 255) / 256), 256, 0, st>>>(h->es.rec, h->es.didx, n, h->es.gath);
+  k_gather_rows<<<(unsigned)((n * SSA_EPR + 255) / 256), 256, 0, st>>>(h->es.rec, h->es.didx, n, SSA_EPR, h->es.gath);
   h->launches++;
   CK(cudaGetLastError());
   CK(cudaMemcpyAsync(h->es.hbuf, h->es.gath, sizeof(double) * n * SSA_EPR, cudaMemcpyDeviceToHost, st));
   CK(cudaStreamSynchronize(st));
   memcpy(out, h->es.hbuf, sizeof(double) * n * SSA_EPR);
+  return SSA_OK;
+}
+
+int ssa_ukf_rollout_truncated(ssa_ukf* h, uint8_t** host, uint8_t** device) {
+  if (!h || !h->ro.init) { snprintf(g_err, sizeof(g_err), "episodic mode not configured"); return SSA_EINVAL; }
+  const size_t N = h->cfg.n_objects, E = h->cfg.n_envs, off = sizeof(double) * (12 * N + E) + sizeof(int32_t) * SSA_N_TASKERS * E +
+                                                               ((E + 7) / 8) * 8;
+  if (host) *host = (uint8_t*)h->ro.hout + off;
+  if (device) *device = (uint8_t*)h->ro.dout + off;
+  return SSA_OK;
+}
+
+int ssa_ukf_rollout_terminal_obs_download(ssa_ukf* h, const int32_t* envs, int n, double* out, void* stream) {
+  if (!h || !h->ro.init) { snprintf(g_err, sizeof(g_err), "episodic mode not configured"); return SSA_EINVAL; }
+  if (check_envs(h, envs, n, out)) return SSA_EINVAL;
+  if (n == 0) return SSA_OK;
+  CK(cudaSetDevice(h->device));
+  cudaStream_t st = (cudaStream_t)stream;
+  const long row = (long)h->ro.term_w * h->cfg.m;  // doubles per environment
+  memcpy(h->ro.htidx, envs, sizeof(int32_t) * n);
+  CK(cudaMemcpyAsync(h->ro.tidx, h->ro.htidx, sizeof(int32_t) * n, cudaMemcpyHostToDevice, st));
+  k_gather_rows<<<(unsigned)((n * row + 255) / 256), 256, 0, st>>>(h->ro.term, h->ro.tidx, n, row, h->ro.tgath);
+  h->launches++;
+  CK(cudaGetLastError());
+  CK(cudaMemcpyAsync(h->ro.htbuf, h->ro.tgath, sizeof(double) * n * row, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  memcpy(out, h->ro.htbuf, sizeof(double) * n * row);
+  return SSA_OK;
+}
+
+// ssa_ukf_rollout_reset_envs with episode statistics: the accumulators of the re-drawn environments start afresh
+__global__ void __launch_bounds__(128) k_ep_clear(double* env, double* obj, const uint8_t* __restrict__ mask, int E, int m) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e < E && mask[e]) ssa_ep_clear(env + (long)e * SSA_EPE, obj + (long)e * m * SSA_EPO, m);
+}
+
+int ssa_ukf_rollout_reset_envs(ssa_ukf* h, const int32_t* envs, int n, void* stream) {
+  if (!h || !h->ro.init) { snprintf(g_err, sizeof(g_err), "episodic mode not configured"); return SSA_EINVAL; }
+  if (check_envs(h, envs, n, envs)) return SSA_EINVAL;
+  if (n == 0) return SSA_OK;
+  CK(cudaSetDevice(h->device));
+  cudaStream_t st = (cudaStream_t)stream;
+  const int E = h->cfg.n_envs;
+  // (a pageable source: the copy has read it when cudaMemcpyAsync returns, so the vector may go out of scope)
+  std::vector<uint8_t> mask(E, 0);
+  for (int k = 0; k < n; ++k) mask[envs[k]] = 1;
+  CK(cudaMemcpyAsync(h->ro.mask, mask.data(), E, cudaMemcpyHostToDevice, st));
+  if (h->es.live) {
+    k_ep_clear<<<(unsigned)((E + 127) / 128), 128, 0, st>>>(h->es.env, h->es.obj, h->ro.mask, E, h->cfg.m);
+    h->launches++;
+  }
+  RolloutParams rp;
+  rollout_params(h, &rp, 0);
+  rp.done = h->ro.mask;
+  k_env_reset<<<(unsigned)E, 128, 0, st>>>(rp);
+  h->launches++;
+  int rc = rollout_refresh(h, st, h->ro.mask);
+  if (rc) return rc;
+  launch_obs_aer(h, st);
+  CK(cudaMemcpyAsync(h->ro.hout, h->ro.dout, h->ro.out_bytes, cudaMemcpyDeviceToHost, st));
+  CK(cudaMemcpyAsync(h->ro.haer, h->ro.daer, sizeof(double) * 4 * h->cfg.n_objects, cudaMemcpyDeviceToHost, st));
+  CK(cudaGetLastError());
   return SSA_OK;
 }
 
@@ -2895,6 +3029,7 @@ int ssa_ukf_rollout_step(ssa_ukf* h, int auto_reset, void* stream) {
   }
   const int ar = (auto_reset & 1) ? 1 : 0;
   const int a = ar + (obs_f32 ? 2 : obs_aer ? 4 : 0);
+  if (ar) h->ro.term_w = obs_aer ? 4 : 12;  // (the layout of the final observations this step records)
   const bool device_io = (auto_reset & SSA_ROLLOUT_DEVICE_IO) != 0, tasked = h->ro.tasker != SSA_TASKER_EXTERNAL;
   if (!device_io && !tasked) CK(cudaMemcpyAsync(h->ro.act_in, h->ro.hin, sizeof(int32_t) * E, cudaMemcpyHostToDevice, st));
   const char* gv = getenv("SSA_UKF_GRAPH");
@@ -2995,6 +3130,7 @@ int ssa_ukf_env_reduce(ssa_ukf* h, const double M[9], int step_index, void* stre
   p.P = h->P; p.ld = h->ld; p.det_prev = h->det_prev; p.det_last = h->det_last; p.det_step = h->det_step;
   p.det_cur = h->det_cur; p.reset_mask = nullptr;
   p.rew_hist = nullptr; p.spos_prev = nullptr; p.act_in = nullptr;  // 'shaped': finished on the host
+  p.truncated = nullptr;
   launch_env_reduce(h, p, st);
   CK(cudaGetLastError());
   return SSA_OK;

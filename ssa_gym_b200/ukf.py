@@ -107,6 +107,7 @@ class BatchedUKF:
             _lib.F_ROLLOUT_DONE: ((self.n_envs,), np.uint8), _lib.F_ROLLOUT_GREEDY: ((self.n_envs, _lib.N_TASKERS), np.int32),
             _lib.F_ROLLOUT_OBS_AER: ((self.N, 4), np.float64),
             _lib.F_ROLLOUT_EPISODE_STATS: ((self.n_envs, _lib.EPISODE_STATS_DOUBLES), np.float64),
+            _lib.F_ROLLOUT_TERMINAL_OBS: ((self.N, 12), np.float64), _lib.F_ROLLOUT_TRUNCATED: ((self.n_envs,), np.uint8),
         }
 
     # -- lifetime ---------------------------------------------------------------------------------
@@ -273,6 +274,10 @@ class BatchedUKF:
         ha, da = ctypes.c_void_p(), ctypes.c_void_p()
         _lib.check(self.lib.ssa_ukf_rollout_obs_aer(self.h, ctypes.byref(ha), ctypes.byref(da)), "ssa_ukf_rollout_obs_aer")
         self.rollout_io["obs_aer"] = view(ha, ctypes.c_double, (N, 4))  # filled by rollout_reset and rollout_step(obs_aer=True)
+        ht = ctypes.c_void_p()
+        _lib.check(self.lib.ssa_ukf_rollout_truncated(self.h, ctypes.byref(ht), None), "ssa_ukf_rollout_truncated")
+        self.rollout_io["truncated"] = view(ht, ctypes.c_uint8, (E,))  # done raised by the step limit alone
+        self._term_w = 12
         return self.rollout_io
 
     def rollout_reset(self, stream=None):
@@ -285,6 +290,8 @@ class BatchedUKF:
         mode = (1 if auto_reset else 0) | (_lib.ROLLOUT_DEVICE_IO if device_io else 0) | (_lib.ROLLOUT_OBS_F32 if obs_f32 else 0) | \
             (_lib.ROLLOUT_OBS_AER if obs_aer else 0)
         _lib.check(self.lib.ssa_ukf_rollout_step(self.h, mode, stream), "ssa_ukf_rollout_step")
+        if auto_reset:
+            self._term_w = 4 if obs_aer else 12  # the layout of the final observations this step records
 
     def rollout_tasker(self, tasker, spoil_p=0.25):
         """Pick every environment's action inside the step graph (a TASKER_* id, include/ssa_ukf.h), TASKER_EXTERNAL for
@@ -305,6 +312,22 @@ class BatchedUKF:
         _lib.check(self.lib.ssa_ukf_rollout_episode_stats_download(self.h, _ptr(envs), len(envs), _ptr(out), stream),
                    "ssa_ukf_rollout_episode_stats_download")
         return out
+
+    def rollout_terminal_obs(self, envs, stream=None):
+        """The final observations [len(envs), m*12] ([len(envs), m*4] after steps with obs_aer) of the environments
+        `envs`: their observation rows on the last auto-reset step whose done flag was set for them, before the re-draw
+        (include/ssa_ukf.h).  Blocks until copied."""
+        envs = np.ascontiguousarray(envs, dtype=np.int32).reshape(-1)
+        out = np.empty((len(envs), self.m * self._term_w))
+        _lib.check(self.lib.ssa_ukf_rollout_terminal_obs_download(self.h, _ptr(envs), len(envs), _ptr(out), stream),
+                   "ssa_ukf_rollout_terminal_obs_download")
+        return out
+
+    def rollout_reset_envs(self, envs, stream=None):
+        """rollout_reset of the environments `envs` only: re-drawn, refreshed, their episode statistics restarted; the
+        others keep their state and outputs.  rollout_io is valid after a sync."""
+        envs = np.ascontiguousarray(envs, dtype=np.int32).reshape(-1)
+        _lib.check(self.lib.ssa_ukf_rollout_reset_envs(self.h, _ptr(envs), len(envs), stream), "ssa_ukf_rollout_reset_envs")
 
     @property
     def next_parity(self):

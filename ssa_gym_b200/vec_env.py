@@ -24,6 +24,17 @@ filter-consistency figures (ANEES, NIS, innovation bounds, Durbin-Watson statist
 environment reports them in `infos[e]['episode']` (see `episode_info`).  `set_tasker(agent)` runs one of the nine
 agents of agents.py inside the step graph (device taskers, ssa_ukf_rollout_tasker): `vector_step()` then takes no
 actions, and a loop of `vector_step_device()` compares agents with no host round trip at all.
+
+At an episode boundary an RL learner needs to know why the episode ended and what its last observation was: PPO and A2C
+bootstrap the value of an episode cut by the step limit from its final observation (Stable-Baselines3's VecEnv keys
+'terminal_observation' and 'TimeLimit.truncated').  The device mode records both inside the step graph: `vec.truncated`
+([E] bool, every step) says which finished episodes ended at the step limit alone (a lost or successful last step is a
+termination, gym's TimeLimit rule), and with auto-reset the final observation rows of the finished environments are
+kept on the device before their re-draw (device_views()['terminal_obs'], `BatchedUKF.rollout_terminal_obs`).  With
+`config['terminal_observation'] = True` (either mode; off by default, since filling the dicts costs host time on every
+step where environments finish) every finished environment gets `infos[e]['TimeLimit.truncated']`, and in the device
+mode with auto-reset also `infos[e]['terminal_observation']` in the layout and dtype of the observations (the host mode
+always fills that key on its auto-resets).  `reset_at(e)` re-draws environment e alone in either mode.
 """
 import numpy as np
 
@@ -97,6 +108,8 @@ class VecSSATaskerEnv:
         self.episode_stats = bool(config.get('episode_stats', False))
         if self.episode_stats and rng != 'device':
             raise ValueError("episode_stats=True needs rng='device'")
+        # infos[e]['TimeLimit.truncated'] on every finished environment, and the device mode's terminal_observation
+        self.terminal_observation = bool(config.get('terminal_observation', False))
         self.update_interval = config['update_interval']
         self.auto_reset = auto_reset
         if config.get('orbits') is not None:
@@ -213,9 +226,8 @@ class VecSSATaskerEnv:
             self.ukf.rollout_reset()
             self.ukf.sync()
             self.i[:] = 0
-            if self._obs_aer:
-                return self._io["obs_aer"].reshape(self.E, self.m * 4)
-            return self._format_obs(self._io["obs"].reshape(self.E, self.m * 12).astype(self.obs_dtype, copy=False))
+            self.truncated = np.zeros(self.E, bool)
+            return self._device_obs()
         for e in range(self.E):
             self._draw(e)
         self.ukf.reset(self.x_true0.reshape(self.N, 6), self.x_filter0.reshape(self.N, 6), self.P_0)
@@ -229,8 +241,23 @@ class VecSSATaskerEnv:
         self.ukf.upload(F.F_STEP_INDEX, self.i)
         self.ukf.env_reduce(step_index=-1)
 
+    def _device_obs(self):
+        """rng='device': the observations of the output block after a (partial) reset, in the configured layout and dtype."""
+        if self._obs_aer:
+            return self._io["obs_aer"].reshape(self.E, self.m * 4)
+        return self._format_obs(self._io["obs"].reshape(self.E, self.m * 12).astype(self.obs_dtype, copy=False))
+
     def reset_at(self, e):
-        """Reset environment e only (device state of the other environments is untouched)."""
+        """Reset environment e only (device state of the other environments is untouched).  rng='device': one
+        ssa_ukf_rollout_reset_envs call (a new episode of the environment's own counter-based streams; with
+        episode_stats its accumulation starts afresh); self.obs is refreshed and returned."""
+        if self.rng == 'device':
+            self.ukf.rollout_reset_envs([e])
+            self.ukf.sync()
+            self.i[e] = 0
+            self.episodes[e] += 1
+            self.obs = self._device_obs()
+            return self.obs
         import torch
         self._draw(e)
         v = self._dev_views()
@@ -314,6 +341,10 @@ class VecSSATaskerEnv:
                 self.rewards_hist[e, idx[e]] = rewards[e]
             self.prev_spos_argmax = stats[:, 2].astype(np.int64)
         infos = [{} for _ in range(self.E)]
+        if self.terminal_observation and dones.any():
+            max_dpos = (stats if self.reward_type == 'shaped' else self.ukf.download(F.F_ENV_STATS))[:, 0]
+            for e, t in zip(np.flatnonzero(dones).tolist(), self._truncated(dones, max_dpos)[dones].tolist()):
+                infos[e]["TimeLimit.truncated"] = t
         if self.auto_reset and dones.any():
             de = np.where(dones)[0]
             term = self._format_obs(obs[de], de)   # in the layout the caller sees, at the step index the episode ended on
@@ -325,6 +356,13 @@ class VecSSATaskerEnv:
             obs[dones] = fresh[dones]
         self.obs = self._format_obs(obs)
         return self.obs, self._format_reward(rewards), dones, infos
+
+    def _truncated(self, dones, max_dpos):
+        """done raised by the step limit alone (gym's TimeLimit rule; the device's rule, include/ssa_ukf.h): a lost or
+        successful last step is a termination, 'trinary' ends at the step limit only."""
+        if self.reward_type == 'trinary':
+            return dones.copy()
+        return dones & ~((max_dpos > 5e6) | (max_dpos < 3e4))
 
     def _device_step(self, actions):
         """rng='device': the whole step (noise, UKF, reward / done, auto-reset, fresh obs, greedy taskers) is one
@@ -339,6 +377,7 @@ class VecSSATaskerEnv:
         self.ukf.sync()
         self.last_actions = io["actions"].astype(np.int64)
         dones = io["done"].astype(bool)
+        self.truncated = io["truncated"].astype(bool)
         rewards = io["reward"].copy()
         self.i += 1
         if self.auto_reset:
@@ -353,10 +392,19 @@ class VecSSATaskerEnv:
         for e in self._infos_filled:
             infos[e].clear()
         self._infos_filled = []
-        if self.episode_stats and dones.any():
+        if (self.episode_stats or self.terminal_observation) and dones.any():
             de = np.flatnonzero(dones).tolist()
-            for e, ep in zip(de, episode_infos(self.ukf.rollout_episode_stats(de))):
-                infos[e]["episode"] = ep
+            if self.episode_stats:
+                for e, ep in zip(de, episode_infos(self.ukf.rollout_episode_stats(de))):
+                    infos[e]["episode"] = ep
+            if self.terminal_observation:
+                for e, t in zip(de, self.truncated[de].tolist()):
+                    infos[e]["TimeLimit.truncated"] = t
+                if self.auto_reset:  # one download of the final rows, in the layout and dtype of the observations
+                    rows = self.ukf.rollout_terminal_obs(de)
+                    term = rows if self._obs_aer else self._format_obs(rows.astype(self.obs_dtype, copy=False))
+                    for k, e in enumerate(de):
+                        infos[e]["terminal_observation"] = term[k]
             self._infos_filled = de
         return self.obs, self._format_reward(rewards), dones, infos
 
@@ -364,7 +412,10 @@ class VecSSATaskerEnv:
     def device_views(self):
         """Zero-copy torch tensors over the episodic mode's device buffers: 'actions' int32 [E] (INPUT of
         vector_step_device; with a device tasker its output, the actions the step took), 'obs' float64 [E, m*12] ([E, m*4] for obs_returned='aer'), 'reward' float64 [E], 'done' uint8
-        [E], 'greedy' int32 [E, taskers].
+        [E], 'greedy' int32 [E, taskers], 'truncated' uint8 [E] (done raised by the step limit alone) and 'terminal_obs'
+        float64 [E, m*12] ([E, m*4] for 'aer'): with auto-reset, the final observation of each environment's last finished
+        episode, valid after a step whose 'done' is set for it (a PPO on the device bootstraps V(terminal_obs) where
+        done & truncated).
         With config['episode_stats']: 'episode_stats' float64 [E, EPISODE_STATS_DOUBLES], the record of each environment's
         last finished episode (layout: include/ssa_ukf.h; episode_info turns a row into the infos entry), valid after a
         step whose 'done' is set for it.
@@ -374,9 +425,12 @@ class VecSSATaskerEnv:
             u = self.ukf
             obs = (u.torch_view(F.F_ROLLOUT_OBS_AER).view(self.E, self.m * 4) if self._obs_aer else
                    u.torch_view(F.F_ROLLOUT_OBS).view(self.E, self.m * 12))
+            term = u.torch_view(F.F_ROLLOUT_TERMINAL_OBS).view(-1)
+            term = term[:self.N * 4].view(self.E, self.m * 4) if self._obs_aer else term.view(self.E, self.m * 12)
             self._views = {"actions": u.torch_view(F.F_ROLLOUT_ACTIONS), "obs": obs,
                            "reward": u.torch_view(F.F_ROLLOUT_REWARD), "done": u.torch_view(F.F_ROLLOUT_DONE),
-                           "greedy": u.torch_view(F.F_ROLLOUT_GREEDY)}
+                           "greedy": u.torch_view(F.F_ROLLOUT_GREEDY), "truncated": u.torch_view(F.F_ROLLOUT_TRUNCATED),
+                           "terminal_obs": term}
             if self.episode_stats:
                 self._views["episode_stats"] = u.torch_view(F.F_ROLLOUT_EPISODE_STATS)
         return self._views
