@@ -108,6 +108,10 @@ enum ssa_field {
   SSA_F_ROLLOUT_EPISODE_STATS = 35, /* double [E][SSA_EPISODE_STATS_DOUBLES]: episode records (ssa_ukf_rollout_episode_stats_*) */
   SSA_F_ROLLOUT_TERMINAL_OBS = 36,  /* double: final observations of finished episodes (ssa_ukf_rollout_terminal_obs_download) */
   SSA_F_ROLLOUT_TRUNCATED = 37,     /* uint8 [E]: done raised by the step limit alone (ssa_ukf_rollout_truncated)          */
+  SSA_F_ROLLOUT_OBS_NORM = 38,           /* float [E][F]: normalized observations (ssa_ukf_rollout_normalize)       */
+  SSA_F_ROLLOUT_REWARD_NORM = 39,        /* double [E]: normalized rewards                                            */
+  SSA_F_ROLLOUT_TERMINAL_OBS_NORM = 40,  /* float [E][F]: normalized final observations of finished episodes          */
+  SSA_F_ROLLOUT_NORM_STATE = 41,         /* double: running statistics and returns of the normalization (see there)   */
   SSA_F_COUNT_
 };
 
@@ -329,6 +333,61 @@ int ssa_ukf_rollout_episode_stats_download(ssa_ukf* h, const int32_t* envs, int 
 int ssa_ukf_rollout_truncated(ssa_ukf* h, uint8_t** host, uint8_t** device);
 int ssa_ukf_rollout_terminal_obs_download(ssa_ukf* h, const int32_t* envs, int n, double* out, void* stream);
 int ssa_ukf_rollout_reset_envs(ssa_ukf* h, const int32_t* envs, int n, void* stream);
+/* Running normalization of observations and returns in the episodic mode: Stable-Baselines3's VecNormalize (with
+ * RunningMeanStd) inside the step graph, so that a learner gets normalized float32 observations and normalized rewards
+ * without a per-step pass of its own over the [E][F] block.  F = 12 m for the [m][12] rows, 4 m for the 'aer' rows.
+ * Each step, after its observations are final (k_normalize, the last kernel of the step's graph), in VecNormalize's order:
+ *   1. with training and norm_obs, the observation statistics are updated from the step's rows (for finished environments
+ *      with auto-reset the fresh rows), taken as the caller would see them (float32-rounded for SSA_NORM_OBS_ROWS_F32;
+ *      their batch moments are still summed in float64, where numpy would accumulate a float32 array in float32);
+ *   2. the rows are normalized with the updated statistics, clip((x - mean) / sqrt(var + epsilon), +-clip_obs), as float32
+ *      (without norm_obs they are only converted to float32);
+ *   3. with training, returns = returns * gamma + r, then the return statistics are updated from the E returns
+ *      (r: the raw reward, NaN / +-inf replaced by 0.5 with reward_nan_to_num);
+ *   4. the rewards are normalized, clip(r / sqrt(ret var + epsilon), +-clip_reward) (without norm_reward: r);
+ *   5. with auto-reset the final rows of the finished environments are normalized with the same statistics;
+ *   6. returns[done] = 0 (with training off too, as VecNormalize does).
+ * Statistics start at mean 0, var 1, count 1e-4 (RunningMeanStd()); a batch of E rows is merged with
+ * RunningMeanStd.update_from_moments in its expression order.  The batch means and variances (np.mean, np.var) sum the E
+ * rows in one order that depends on E only (csrc/ssa_ukf_core.h, ssa_norm_moments), not numpy's sequential one.
+ * ssa_ukf_rollout_reset zeroes the returns and, with training and norm_obs, updates the observation statistics from the
+ * fresh rows (VecNormalize.reset); ssa_ukf_rollout_reset_envs zeroes the returns of its environments and normalizes their
+ * fresh rows with the current statistics, updating nothing.  The statistics are per handle: environments sharded over
+ * several GPUs keep one set per GPU.
+ *   normalize   after ssa_ukf_rollout_config (which turns normalization off again); NULL turns it off.  A first call, or
+ *               one that changes F, starts fresh statistics; otherwise they carry over.  training is a device flag (no
+ *               step graph is re-captured for it); any other change drops the cached step graphs.  The steps must then
+ *               run in obs_layout: SSA_ROLLOUT_OBS_F32 for SSA_NORM_OBS_ROWS_F32, SSA_ROLLOUT_OBS_AER for
+ *               SSA_NORM_OBS_AER, neither for SSA_NORM_OBS_ROWS (SSA_EINVAL otherwise).  A step or reset launches one
+ *               kernel more (an SSA_ROLLOUT_OBS_F32 step none: k_normalize also writes its float32 rows).  Without
+ *               SSA_ROLLOUT_DEVICE_IO a step copies the normalized rewards and rows to the pinned blocks of
+ *               ssa_ukf_rollout_norm_io, and the raw reward / greedy / done / truncated tail of ssa_ukf_rollout_io; the raw
+ *               rows stay on the device (SSA_F_ROLLOUT_OBS, SSA_F_ROLLOUT_OBS_AER).  SSA_EINVAL for gamma outside
+ *               [0, 1], clip_obs or clip_reward <= 0, epsilon < 0 or NaN, an unknown obs_layout.
+ *   norm_io     pinned host blocks: normalized obs float [E][F], normalized reward double [E].
+ *   norm_state  download / upload of the state, n = 2 F + 4 + E doubles: [obs mean F][obs var F][obs count][ret mean]
+ *               [ret var][ret count][returns E], for checkpoints and evaluation; both block.  (The device block
+ *               SSA_F_ROLLOUT_NORM_STATE is [ret mean, ret var, ret count, training][returns E][obs mean F][obs var F]
+ *               [obs count F].)
+ *   terminal_obs_norm_download   the normalized final rows of n environments envs[0..n) into out[n][F] (as
+ *               ssa_ukf_rollout_terminal_obs_download); blocks until copied.
+ * All but normalize return SSA_EINVAL while normalization is off, the state calls also for n != 2 F + 4 + E.         */
+#define SSA_NORM_OBS_ROWS 0      /* the [m][12] rows, float64                                                      */
+#define SSA_NORM_OBS_ROWS_F32 1  /* the [m][12] rows rounded to float32 (obs_dtype float32)                         */
+#define SSA_NORM_OBS_AER 2       /* the 'aer' rows [m][4]                                                           */
+typedef struct ssa_norm_cfg {
+  int32_t norm_obs;           /* 1: normalize the observations                                                      */
+  int32_t norm_reward;        /* 1: normalize the rewards                                                           */
+  int32_t training;           /* 1: update the statistics and the returns                                           */
+  int32_t obs_layout;         /* SSA_NORM_OBS_*                                                                     */
+  int32_t reward_nan_to_num;  /* 1: NaN / +-inf rewards count as 0.5 (the reference's layouts other than 'flatten')  */
+  double clip_obs, clip_reward, gamma, epsilon;  /* VecNormalize's defaults: 10, 10, 0.99, 1e-8                     */
+} ssa_norm_cfg;
+int ssa_ukf_rollout_normalize(ssa_ukf* h, const ssa_norm_cfg* cfg);
+int ssa_ukf_rollout_norm_io(ssa_ukf* h, float** obs, double** reward);
+int ssa_ukf_rollout_norm_state_download(ssa_ukf* h, double* out, size_t n, void* stream);
+int ssa_ukf_rollout_norm_state_upload(ssa_ukf* h, const double* in, size_t n, void* stream);
+int ssa_ukf_rollout_terminal_obs_norm_download(ssa_ukf* h, const int32_t* envs, int n, float* out, void* stream);
 /* make `stream` wait for every outstanding internal copy of ssa_ukf_step_host / ssa_ukf_step_pinned */
 int ssa_ukf_host_join(ssa_ukf* h, void* stream);
 /* Convenience wrappers with the reference's call structure */

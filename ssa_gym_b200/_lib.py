@@ -30,11 +30,13 @@ TASKER_NAIVE_RANDOM, TASKER_VISIBLE_RANDOM, TASKER_VISIBLE_GREEDY_SPOILED = 6, 7
  F_Z_TRUE, F_Y, F_S, F_SIGMAS_H, F_Z_NOISE, F_VISIBLE, F_STATUS, F_INFLATIONS, F_ACTIONS, F_REWARD, F_DONE,
  F_GREEDY, F_SCORES, F_UPDATED, F_TRANS_ENV, F_STEP_INDEX, F_ENV_STATS, F_DIAG, F_INNOV_FLAGS, F_CATALOG_STATS,
  F_ROLLOUT_OBS, F_ROLLOUT_REWARD, F_ROLLOUT_ACTIONS, F_ROLLOUT_DONE, F_ROLLOUT_GREEDY, F_ROLLOUT_OBS_AER,
- F_ROLLOUT_EPISODE_STATS, F_ROLLOUT_TERMINAL_OBS, F_ROLLOUT_TRUNCATED) = range(38)
+ F_ROLLOUT_EPISODE_STATS, F_ROLLOUT_TERMINAL_OBS, F_ROLLOUT_TRUNCATED, F_ROLLOUT_OBS_NORM, F_ROLLOUT_REWARD_NORM,
+ F_ROLLOUT_TERMINAL_OBS_NORM, F_ROLLOUT_NORM_STATE) = range(42)
 ROLLOUT_DEVICE_IO = 2
 ROLLOUT_OBS_F32 = 4
 ROLLOUT_OBS_AER = 8
 EPISODE_STATS_DOUBLES = 23
+NORM_OBS_ROWS, NORM_OBS_ROWS_F32, NORM_OBS_AER = 0, 1, 2
 
 
 class SsaUkfCfg(ctypes.Structure):
@@ -47,6 +49,15 @@ class SsaUkfCfg(ctypes.Structure):
         ("Wm", ctypes.c_double * 13), ("Wc", ctypes.c_double * 13),
         ("Q", ctypes.c_double * 36), ("R", ctypes.c_double * 9),
         ("obs_itrs", ctypes.c_double * 3), ("T", ctypes.c_double * 9), ("obs_limit", ctypes.c_double),
+    ]
+
+
+class SsaNormCfg(ctypes.Structure):
+    """Mirror of `struct ssa_norm_cfg` (include/ssa_ukf.h)."""
+    _fields_ = [
+        ("norm_obs", ctypes.c_int32), ("norm_reward", ctypes.c_int32), ("training", ctypes.c_int32),
+        ("obs_layout", ctypes.c_int32), ("reward_nan_to_num", ctypes.c_int32),
+        ("clip_obs", ctypes.c_double), ("clip_reward", ctypes.c_double), ("gamma", ctypes.c_double), ("epsilon", ctypes.c_double),
     ]
 
 
@@ -83,6 +94,11 @@ PROTOTYPES = {
     "ssa_ukf_rollout_truncated": (_I, [c_void_p, c_void_p, c_void_p]),
     "ssa_ukf_rollout_terminal_obs_download": (_I, [c_void_p, c_void_p, _I, c_void_p, c_void_p]),
     "ssa_ukf_rollout_reset_envs": (_I, [c_void_p, c_void_p, _I, c_void_p]),
+    "ssa_ukf_rollout_normalize": (_I, [c_void_p, ctypes.POINTER(SsaNormCfg)]),
+    "ssa_ukf_rollout_norm_io": (_I, [c_void_p, c_void_p, c_void_p]),
+    "ssa_ukf_rollout_norm_state_download": (_I, [c_void_p, c_void_p, _SZ, c_void_p]),
+    "ssa_ukf_rollout_norm_state_upload": (_I, [c_void_p, c_void_p, _SZ, c_void_p]),
+    "ssa_ukf_rollout_terminal_obs_norm_download": (_I, [c_void_p, c_void_p, _I, c_void_p, c_void_p]),
     "ssa_trans_matrix_table": (_I, [_I, _I, _I, _D, _D, _I, c_void_p, _I, c_void_p]),
     "ssa_ukf_predict": (_I, [c_void_p, c_void_p]),
     "ssa_ukf_update": (_I, [c_void_p, c_void_p, _I, c_void_p]),

@@ -1829,6 +1829,20 @@ struct ssa_ukf {
     double* hbuf;        // pinned: gathered records [E][SSA_EPR], then idx [E] int32
     int32_t* hidx;
   } es;
+  // running normalization of observations and returns in the episodic mode (ssa_ukf_rollout_normalize, k_normalize)
+  struct {
+    int on;
+    int F;               // normalized columns per environment: 12 m, or 4 m for SSA_NORM_OBS_AER
+    ssa_norm_cfg cfg;
+    double* buf;         // device: state [4 + E + 3F] (SSA_F_ROLLOUT_NORM_STATE), reward_norm [E], then floats obs_norm,
+                         // term_norm, gathered rows [E][F] each, then idx [E] int32
+    double *state, *reward;
+    float *obs, *term, *gath;
+    int32_t* didx;
+    double* hbuf;        // pinned: reward_norm [E], obs_norm [E][F] floats (the step copies both at once), gathered rows
+    float *hobs, *hgath; //         [E][F] floats, idx [E] int32
+    int32_t* hidx;
+  } nm;
   int32_t *status, *infl, *actions, *greedy;
   uint8_t *visible, *updated, *innov_flags, *done;
   double* diag;     // [N][2] NEES, NIS of the last ssa_ukf_diagnostics call
@@ -2000,6 +2014,7 @@ int ssa_ukf_destroy(ssa_ukf* h) {
     for (int i = 0; i < 6; ++i) if (h->ro.gexec[i]) cudaGraphExecDestroy(h->ro.gexec[i]);
   }
   if (h->es.on) { cudaFree(h->es.buf); cudaFreeHost(h->es.hbuf); }
+  if (h->nm.on) { cudaFree(h->nm.buf); cudaFreeHost(h->nm.hbuf); }
   cudaFree(h->snap);
   cudaFree(h->cat_part);
   cudaFree(h->stage);
@@ -2109,6 +2124,16 @@ static int field_info(ssa_ukf* h, int field, void** p, size_t* bytes, int* soa_c
     case SSA_F_ROLLOUT_TRUNCATED:
       if (!h->ro.init) { snprintf(g_err, sizeof(g_err), "episodic mode not configured"); return SSA_EINVAL; }
       *p = (uint8_t*)((int32_t*)(h->ro.dout + 12 * N + E) + SSA_N_TASKERS * E) + ((E + 7) / 8) * 8; *bytes = E; break;
+    case SSA_F_ROLLOUT_OBS_NORM: case SSA_F_ROLLOUT_REWARD_NORM: case SSA_F_ROLLOUT_TERMINAL_OBS_NORM:
+    case SSA_F_ROLLOUT_NORM_STATE: {
+      if (!h->nm.on) { snprintf(g_err, sizeof(g_err), "normalization not enabled"); return SSA_EINVAL; }
+      const size_t F = h->nm.F;
+      if (field == SSA_F_ROLLOUT_OBS_NORM) { *p = h->nm.obs; *bytes = E * F * 4; }
+      else if (field == SSA_F_ROLLOUT_REWARD_NORM) { *p = h->nm.reward; *bytes = E * 8; }
+      else if (field == SSA_F_ROLLOUT_TERMINAL_OBS_NORM) { *p = h->nm.term; *bytes = E * F * 4; }
+      else { *p = h->nm.state; *bytes = (4 + E + 3 * F) * 8; }
+      break;
+    }
     default: snprintf(g_err, sizeof(g_err), "unknown field %d", field); return SSA_EINVAL;
   }
   return SSA_OK;
@@ -2636,6 +2661,10 @@ int ssa_ukf_rollout_config(ssa_ukf* h, const double* orbits, int n_orbits, const
     cudaFree(h->es.buf); cudaFreeHost(h->es.hbuf);
     memset(&h->es, 0, sizeof(h->es));
   }
+  if (h->nm.on) {  // (nor normalization)
+    cudaFree(h->nm.buf); cudaFreeHost(h->nm.hbuf);
+    memset(&h->nm, 0, sizeof(h->nm));
+  }
   h->ro.n_orbits = n_orbits; h->ro.n_table = n_table; h->ro.update_interval = update_interval;
   h->ro.tasker = SSA_TASKER_EXTERNAL; h->ro.spoil_p = 0.0;
   CK(cudaMalloc(&h->ro.dbuf, sizeof(double) * ((size_t)n_orbits * 6 + (size_t)n_table * 9 + 32)));
@@ -2699,6 +2728,16 @@ int ssa_ukf_rollout_io(ssa_ukf* h, int32_t** actions, double** obs, double** rew
 }
 
 static void launch_obs_aer(ssa_ukf* h, cudaStream_t st);
+// k_normalize's modes
+#define SSA_NORM_STEP 0        // a step: statistics (training), normalized rows, rewards and final rows, returns[done] = 0
+#define SSA_NORM_RESET 1       // ssa_ukf_rollout_reset: returns = 0, observation statistics from the fresh rows (training)
+#define SSA_NORM_RESET_ENVS 2  // ssa_ukf_rollout_reset_envs: rows and returns of the masked environments, nothing updated
+static void launch_normalize(ssa_ukf* h, cudaStream_t st, int mode, int auto_reset, const uint8_t* mask);
+// normalized rewards and rows to their pinned host mirror (one copy: the two blocks are adjacent)
+static cudaError_t norm_copy_out(ssa_ukf* h, cudaStream_t st) {
+  const size_t E = h->cfg.n_envs;
+  return cudaMemcpyAsync(h->nm.hbuf, h->nm.reward, sizeof(double) * E + sizeof(float) * E * h->nm.F, cudaMemcpyDeviceToHost, st);
+}
 
 // the captured step graphs of the episodic mode (re-captured on the next ssa_ukf_rollout_step)
 static void rollout_drop_graphs(ssa_ukf* h) {
@@ -2723,6 +2762,10 @@ int ssa_ukf_rollout_reset(ssa_ukf* h, void* stream) {
   launch_obs_aer(h, st);  // (the 'aer' rows of the fresh episodes, whichever layout the steps will use)
   CK(cudaMemcpyAsync(h->ro.hout, h->ro.dout, h->ro.out_bytes, cudaMemcpyDeviceToHost, st));
   CK(cudaMemcpyAsync(h->ro.haer, h->ro.daer, sizeof(double) * 4 * h->cfg.n_objects, cudaMemcpyDeviceToHost, st));
+  if (h->nm.on) {
+    launch_normalize(h, st, SSA_NORM_RESET, 0, nullptr);
+    CK(norm_copy_out(h, st));
+  }
   CK(cudaGetLastError());
   return SSA_OK;
 }
@@ -2781,6 +2824,131 @@ static void launch_obs_aer(ssa_ukf* h, cudaStream_t st) {
   const long N = h->cfg.n_objects;
   k_obs_aer<<<(unsigned)((N + 127) / 128), 128, 0, st>>>(h->ro.dout, h->step_idx, h->ro.table, h->ro.n_table, ob, h->cfg.m, N,
                                                          h->ro.daer);
+  h->launches++;
+}
+
+// ---- running normalization of observations and returns (ssa_ukf_rollout_normalize; arithmetic: ssa_norm_* in
+// ssa_ukf_core.h) ------------------------------------------------------------------------------------------------
+// Device state (SSA_F_ROLLOUT_NORM_STATE): [ret mean, ret var, ret count, training][returns E][obs mean F][obs var F]
+// [obs count F].  Every column keeps its own copy of the (common) observation count, so the CTA of a column reads and
+// writes nothing another CTA writes and the kernel needs no grid-wide wait.
+static constexpr int kNormThreads = 128;
+static constexpr int kNormLeavesMax = 1024;  // ssa_norm_leaves(E) <= 1024 for every E (ssa_norm_leaf)
+struct NormParams {
+  const double* obs; int f32;        // rows [E][F] (the output block, or the 'aer' block); f32: float32-rounded values
+  const double* term;                // final rows [E][F] (auto-reset steps), or null
+  const uint8_t* done;               // [E]: the step's done flags, or the mask of SSA_NORM_RESET_ENVS
+  const double* reward;              // [E]: the step's raw reward
+  double* state;                     // SSA_F_ROLLOUT_NORM_STATE
+  float* out; float* term_out;       // [E][F] normalized rows, normalized final rows of the finished environments
+  double* reward_out;                // [E]
+  float* obs32;                      // SSA_ROLLOUT_OBS_F32 steps: the float32 rows of k_obs_to_f32, or null
+  int E, F, mode, norm_obs, norm_reward, reward_nan;
+  double clip_obs, clip_reward, gamma, eps;
+};
+
+// the sum over the E rows of the column x[r * stride] in the order of ssa_norm_moments: the leaves in parallel, then
+// every level of ssa_norm_tree in parallel over its pairs; sm holds ssa_norm_leaves(E) doubles
+__device__ double norm_sum(const double* x, long stride, int E, int f32, int sq, double mean, double* sm) {
+  const int L = ssa_norm_leaf(E), n = ssa_norm_leaves(E);
+  for (int k = threadIdx.x; k < n; k += blockDim.x) sm[k] = ssa_norm_leaf_sum(x, stride, k * L, min(k * L + L, E), f32, sq, mean);
+  __syncthreads();
+  for (int s = 1; s < n; s <<= 1) {
+    for (int i = 2 * s * threadIdx.x; i + s < n; i += 2 * s * blockDim.x) sm[i] = sm[i] + sm[i + s];
+    __syncthreads();
+  }
+  const double t = sm[0];
+  __syncthreads();  // (sm is reused by the next sum)
+  return t;
+}
+
+// The last kernel of a step (or of a reset) with normalization on.  CTA c < F owns observation column c: batch mean and
+// variance over the E rows (two passes, as np.var), merged into the column's running statistics, then the column of the
+// normalized rows and of the finished environments' normalized final rows.  CTA F owns the returns: returns * gamma +
+// reward, their batch moments merged into the return statistics, the normalized rewards, then returns[done] = 0.
+// A column's values are F doubles apart: every load takes one 32-byte sector that the neighbouring columns' CTAs read
+// too, so the rows cross from DRAM / L2 about once per pass.
+__global__ void __launch_bounds__(kNormThreads) k_normalize(const NormParams p) {
+  __shared__ double sm[kNormLeavesMax];
+  const int c = blockIdx.x, E = p.E, F = p.F;
+  double* rs = p.state;
+  double* ret = rs + 4;
+  const bool training = rs[3] != 0.0;
+  if (c == F) {
+    if (p.mode != SSA_NORM_STEP) {
+      for (int e = threadIdx.x; e < E; e += blockDim.x)
+        if (p.mode == SSA_NORM_RESET || p.done[e]) ret[e] = 0.0;
+      return;
+    }
+    double m = rs[0], v = rs[1], n = rs[2];
+    if (training) {
+      for (int e = threadIdx.x; e < E; e += blockDim.x)
+        ret[e] = ssa_norm_return(ret[e], p.gamma, ssa_norm_reward_in(p.reward[e], p.reward_nan));
+      __syncthreads();
+      const double bm = ssa_div(norm_sum(ret, 1, E, 0, 0, 0.0, sm), (double)E);
+      const double bv = ssa_div(norm_sum(ret, 1, E, 0, 1, bm, sm), (double)E);
+      ssa_norm_merge(&m, &v, &n, bm, bv, (double)E);
+      if (threadIdx.x == 0) { rs[0] = m; rs[1] = v; rs[2] = n; }
+    }
+    const double sd = ssa_norm_sd(v, p.eps);
+    for (int e = threadIdx.x; e < E; e += blockDim.x) {
+      const double r = ssa_norm_reward_in(p.reward[e], p.reward_nan);
+      p.reward_out[e] = p.norm_reward ? ssa_norm_reward(r, sd, p.clip_reward) : r;
+      if (p.done[e]) ret[e] = 0.0;
+    }
+    return;
+  }
+  double* mean = ret + E;
+  double* var = mean + F;
+  double* cnt = var + F;
+  double mu = mean[c], vr = var[c], n = cnt[c];
+  if (p.mode != SSA_NORM_RESET_ENVS && training && p.norm_obs) {
+    const double bm = ssa_div(norm_sum(p.obs + c, F, E, p.f32, 0, 0.0, sm), (double)E);
+    const double bv = ssa_div(norm_sum(p.obs + c, F, E, p.f32, 1, bm, sm), (double)E);
+    ssa_norm_merge(&mu, &vr, &n, bm, bv, (double)E);
+    if (threadIdx.x == 0) { mean[c] = mu; var[c] = vr; cnt[c] = n; }
+  }
+  const double sd = ssa_norm_sd(vr, p.eps);
+  constexpr int U = 8;  // rows per thread whose loads are issued together
+  for (int e0 = threadIdx.x; e0 < E; e0 += U * blockDim.x) {
+    double x[U];
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      const int e = e0 + u * blockDim.x;
+      x[u] = e < E ? p.obs[(long)e * F + c] : 0.0;
+    }
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      const int e = e0 + u * blockDim.x;
+      if (e >= E) break;
+      if (p.mode == SSA_NORM_RESET_ENVS && !p.done[e]) continue;
+      const long i = (long)e * F + c;
+      const double v = ssa_norm_in(x[u], p.f32);
+      p.out[i] = (float)(p.norm_obs ? ssa_norm_obs(v, mu, sd, p.clip_obs) : v);
+      if (p.obs32) p.obs32[i] = (float)x[u];
+      if (p.term && p.done[e]) {
+        const double t = ssa_norm_in(p.term[i], p.f32);
+        p.term_out[i] = (float)(p.norm_obs ? ssa_norm_obs(t, mu, sd, p.clip_obs) : t);
+      }
+    }
+  }
+}
+
+static void launch_normalize(ssa_ukf* h, cudaStream_t st, int mode, int auto_reset, const uint8_t* mask) {
+  const size_t N = h->cfg.n_objects, E = h->cfg.n_envs;
+  const ssa_norm_cfg& c = h->nm.cfg;
+  NormParams p;
+  p.obs = c.obs_layout == SSA_NORM_OBS_AER ? h->ro.daer : h->ro.dout;
+  p.f32 = c.obs_layout == SSA_NORM_OBS_ROWS_F32;
+  p.term = mode == SSA_NORM_STEP && auto_reset ? h->ro.term : nullptr;
+  p.reward = h->ro.dout + 12 * N;
+  p.done = mode == SSA_NORM_RESET_ENVS ? mask : (const uint8_t*)((const int32_t*)(p.reward + E) + SSA_N_TASKERS * E);
+  p.state = h->nm.state; p.out = h->nm.obs; p.term_out = h->nm.term; p.reward_out = h->nm.reward;
+  p.obs32 = mode == SSA_NORM_STEP && p.f32 ? h->ro.dobs32 : nullptr;
+  p.E = (int)E; p.F = h->nm.F; p.mode = mode;
+  p.norm_obs = c.norm_obs; p.norm_reward = c.norm_reward; p.reward_nan = c.reward_nan_to_num;
+  p.clip_obs = c.clip_obs; p.clip_reward = c.clip_reward; p.gamma = c.gamma; p.eps = c.epsilon;
+  k_normalize<<<(unsigned)(p.F + 1), kNormThreads, 0, st>>>(p);
   h->launches++;
 }
 
@@ -2887,12 +3055,14 @@ static int rollout_chain(ssa_ukf* h, cudaStream_t st, int auto_reset, int obs_f3
     rc = rollout_refresh(h, st, rp.done);
     if (rc) return rc;
   }
-  if (obs_f32) {
+  const bool norm = h->nm.on != 0;
+  if (obs_f32 && !norm) {  // (with normalization k_normalize writes the float32 rows)
     const long n2 = 6 * N;  // 12 N doubles, two at a time (the block is cudaMalloc-aligned)
     k_obs_to_f32<<<(unsigned)((n2 + 255) / 256), 256, 0, st>>>((const double2*)h->ro.dout, (float2*)h->ro.dobs32, n2);
     h->launches++;
   }
   if (obs_aer) launch_obs_aer(h, st);
+  if (norm) launch_normalize(h, st, SSA_NORM_STEP, auto_reset, nullptr);
   return SSA_OK;
 }
 
@@ -3013,6 +3183,10 @@ int ssa_ukf_rollout_reset_envs(ssa_ukf* h, const int32_t* envs, int n, void* str
   launch_obs_aer(h, st);
   CK(cudaMemcpyAsync(h->ro.hout, h->ro.dout, h->ro.out_bytes, cudaMemcpyDeviceToHost, st));
   CK(cudaMemcpyAsync(h->ro.haer, h->ro.daer, sizeof(double) * 4 * h->cfg.n_objects, cudaMemcpyDeviceToHost, st));
+  if (h->nm.on) {
+    launch_normalize(h, st, SSA_NORM_RESET_ENVS, 0, h->ro.mask);
+    CK(norm_copy_out(h, st));
+  }
   CK(cudaGetLastError());
   return SSA_OK;
 }
@@ -3025,6 +3199,10 @@ int ssa_ukf_rollout_step(ssa_ukf* h, int auto_reset, void* stream) {
   const bool obs_f32 = (auto_reset & SSA_ROLLOUT_OBS_F32) != 0, obs_aer = (auto_reset & SSA_ROLLOUT_OBS_AER) != 0;
   if (obs_f32 && obs_aer) {
     snprintf(g_err, sizeof(g_err), "SSA_ROLLOUT_OBS_F32 and SSA_ROLLOUT_OBS_AER exclude each other");
+    return SSA_EINVAL;
+  }
+  if (h->nm.on && (obs_aer ? SSA_NORM_OBS_AER : obs_f32 ? SSA_NORM_OBS_ROWS_F32 : SSA_NORM_OBS_ROWS) != h->nm.cfg.obs_layout) {
+    snprintf(g_err, sizeof(g_err), "the step's observation layout is not the one ssa_ukf_rollout_normalize was given");
     return SSA_EINVAL;
   }
   const int ar = (auto_reset & 1) ? 1 : 0;
@@ -3058,7 +3236,11 @@ int ssa_ukf_rollout_step(ssa_ukf* h, int auto_reset, void* stream) {
     if (rc) return rc;
   }
   if (!device_io) {
-    if (obs_f32) {  // float observations + the reward / greedy / done tail of the double block
+    if (h->nm.on) {  // normalized rewards and rows + the raw reward / greedy / done / truncated tail of the double block
+      const size_t N = h->cfg.n_objects;
+      CK(norm_copy_out(h, st));
+      CK(cudaMemcpyAsync(h->ro.hout + 12 * N, h->ro.dout + 12 * N, h->ro.out_bytes - sizeof(double) * 12 * N, cudaMemcpyDeviceToHost, st));
+    } else if (obs_f32) {  // float observations + the reward / greedy / done tail of the double block
       const size_t N = h->cfg.n_objects;
       CK(cudaMemcpyAsync(h->ro.hobs32, h->ro.dobs32, sizeof(float) * 12 * N, cudaMemcpyDeviceToHost, st));
       CK(cudaMemcpyAsync(h->ro.hout + 12 * N, h->ro.dout + 12 * N, h->ro.out_bytes - sizeof(double) * 12 * N, cudaMemcpyDeviceToHost, st));
@@ -3087,6 +3269,133 @@ int ssa_ukf_rollout_tasker(ssa_ukf* h, int tasker, double spoil_p) {
   if (tasker != h->ro.tasker || spoil_p != h->ro.spoil_p) rollout_drop_graphs(h);  // (both are captured kernel parameters)
   h->ro.tasker = tasker;
   h->ro.spoil_p = spoil_p;
+  return SSA_OK;
+}
+
+static void norm_free(ssa_ukf* h) {
+  cudaFree(h->nm.buf); cudaFreeHost(h->nm.hbuf);
+  memset(&h->nm, 0, sizeof(h->nm));
+}
+
+int ssa_ukf_rollout_normalize(ssa_ukf* h, const ssa_norm_cfg* cfg) {
+  if (!h || !h->ro.init) { snprintf(g_err, sizeof(g_err), "episodic mode not configured"); return SSA_EINVAL; }
+  CK(cudaSetDevice(h->device));
+  if (!cfg) {
+    if (h->nm.on) { CK(cudaDeviceSynchronize()); norm_free(h); rollout_drop_graphs(h); }
+    return SSA_OK;
+  }
+  if (!(cfg->gamma >= 0.0 && cfg->gamma <= 1.0)) { snprintf(g_err, sizeof(g_err), "gamma %g outside [0, 1]", cfg->gamma); return SSA_EINVAL; }
+  if (!(cfg->clip_obs > 0.0 && cfg->clip_reward > 0.0)) {
+    snprintf(g_err, sizeof(g_err), "clip_obs %g and clip_reward %g must be > 0", cfg->clip_obs, cfg->clip_reward);
+    return SSA_EINVAL;
+  }
+  if (!(cfg->epsilon >= 0.0)) { snprintf(g_err, sizeof(g_err), "epsilon %g must be >= 0", cfg->epsilon); return SSA_EINVAL; }
+  if (cfg->obs_layout < SSA_NORM_OBS_ROWS || cfg->obs_layout > SSA_NORM_OBS_AER) {
+    snprintf(g_err, sizeof(g_err), "unknown obs_layout %d", cfg->obs_layout);
+    return SSA_EINVAL;
+  }
+  ssa_norm_cfg c = *cfg;
+  c.norm_obs = c.norm_obs != 0; c.norm_reward = c.norm_reward != 0; c.training = c.training != 0;
+  c.reward_nan_to_num = c.reward_nan_to_num != 0;
+  const size_t E = h->cfg.n_envs, F = (size_t)(c.obs_layout == SSA_NORM_OBS_AER ? 4 : 12) * h->cfg.m;
+  if (h->nm.on && h->nm.F == (int)F) {  // the statistics carry over; only training is read from device memory
+    const ssa_norm_cfg& o = h->nm.cfg;
+    if (o.norm_obs != c.norm_obs || o.norm_reward != c.norm_reward || o.obs_layout != c.obs_layout ||
+        o.reward_nan_to_num != c.reward_nan_to_num || o.clip_obs != c.clip_obs || o.clip_reward != c.clip_reward ||
+        o.gamma != c.gamma || o.epsilon != c.epsilon)
+      rollout_drop_graphs(h);  // (captured kernel parameters)
+    if (o.training != c.training) {
+      const double t = c.training;
+      CK(cudaDeviceSynchronize());  // (no step in flight reads the flag while it changes)
+      CK(cudaMemcpy(h->nm.state + 3, &t, sizeof(double), cudaMemcpyHostToDevice));
+    }
+    h->nm.cfg = c;
+    return SSA_OK;
+  }
+  if (h->nm.on) { CK(cudaDeviceSynchronize()); norm_free(h); }
+  const size_t sd = 4 + E + 3 * F;  // state doubles
+  const size_t bytes = sizeof(double) * (sd + E) + sizeof(float) * 3 * E * F + sizeof(int32_t) * E;
+  CK(cudaMalloc(&h->nm.buf, bytes));
+  CK(cudaMemset(h->nm.buf, 0, bytes));
+  h->nm.state = h->nm.buf; h->nm.reward = h->nm.state + sd;
+  h->nm.obs = (float*)(h->nm.reward + E); h->nm.term = h->nm.obs + E * F; h->nm.gath = h->nm.term + E * F;
+  h->nm.didx = (int32_t*)(h->nm.gath + E * F);
+  // RunningMeanStd(): mean 0, var 1, count 1e-4; the returns 0
+  std::vector<double> st(sd, 0.0);
+  st[1] = 1.0; st[2] = 1e-4; st[3] = c.training;
+  for (size_t k = 0; k < F; ++k) { st[4 + E + F + k] = 1.0; st[4 + E + 2 * F + k] = 1e-4; }
+  CK(cudaMemcpy(h->nm.state, st.data(), sizeof(double) * sd, cudaMemcpyHostToDevice));
+  const size_t hbytes = sizeof(double) * E + sizeof(float) * 2 * E * F + sizeof(int32_t) * E;
+  CK(cudaHostAlloc(&h->nm.hbuf, hbytes, cudaHostAllocDefault));
+  memset(h->nm.hbuf, 0, hbytes);
+  h->nm.hobs = (float*)(h->nm.hbuf + E); h->nm.hgath = h->nm.hobs + E * F; h->nm.hidx = (int32_t*)(h->nm.hgath + E * F);
+  h->nm.cfg = c; h->nm.F = (int)F; h->nm.on = 1;
+  rollout_drop_graphs(h);
+  return SSA_OK;
+}
+
+int ssa_ukf_rollout_norm_io(ssa_ukf* h, float** obs, double** reward) {
+  if (!h || !h->nm.on) { snprintf(g_err, sizeof(g_err), "normalization not enabled"); return SSA_EINVAL; }
+  if (obs) *obs = h->nm.hobs;
+  if (reward) *reward = h->nm.hbuf;
+  return SSA_OK;
+}
+
+// the saved state [obs mean F][obs var F][obs count][ret mean][ret var][ret count][returns E] <-> the device state
+static int norm_state_check(ssa_ukf* h, const void* buf, size_t n) {
+  if (!h || !h->nm.on) { snprintf(g_err, sizeof(g_err), "normalization not enabled"); return SSA_EINVAL; }
+  const size_t want = 2 * (size_t)h->nm.F + 4 + h->cfg.n_envs;
+  if (!buf || n != want) { snprintf(g_err, sizeof(g_err), "state buffer of %zu doubles, want %zu", n, want); return SSA_EINVAL; }
+  return SSA_OK;
+}
+
+int ssa_ukf_rollout_norm_state_download(ssa_ukf* h, double* out, size_t n, void* stream) {
+  if (norm_state_check(h, out, n)) return SSA_EINVAL;
+  CK(cudaSetDevice(h->device));
+  const size_t E = h->cfg.n_envs, F = h->nm.F;
+  std::vector<double> d(4 + E + 3 * F);
+  cudaStream_t st = (cudaStream_t)stream;
+  CK(cudaMemcpyAsync(d.data(), h->nm.state, sizeof(double) * d.size(), cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  const double* col = d.data() + 4 + E;
+  memcpy(out, col, sizeof(double) * 2 * F);
+  out[2 * F] = col[2 * F];
+  memcpy(out + 2 * F + 1, d.data(), sizeof(double) * 3);
+  memcpy(out + 2 * F + 4, d.data() + 4, sizeof(double) * E);
+  return SSA_OK;
+}
+
+int ssa_ukf_rollout_norm_state_upload(ssa_ukf* h, const double* in, size_t n, void* stream) {
+  if (norm_state_check(h, in, n)) return SSA_EINVAL;
+  CK(cudaSetDevice(h->device));
+  const size_t E = h->cfg.n_envs, F = h->nm.F;
+  std::vector<double> d(4 + E + 3 * F);
+  memcpy(d.data(), in + 2 * F + 1, sizeof(double) * 3);
+  d[3] = h->nm.cfg.training;
+  memcpy(d.data() + 4, in + 2 * F + 4, sizeof(double) * E);
+  memcpy(d.data() + 4 + E, in, sizeof(double) * 2 * F);
+  for (size_t k = 0; k < F; ++k) d[4 + E + 2 * F + k] = in[2 * F];
+  cudaStream_t st = (cudaStream_t)stream;
+  CK(cudaMemcpyAsync(h->nm.state, d.data(), sizeof(double) * d.size(), cudaMemcpyHostToDevice, st));
+  CK(cudaStreamSynchronize(st));
+  return SSA_OK;
+}
+
+int ssa_ukf_rollout_terminal_obs_norm_download(ssa_ukf* h, const int32_t* envs, int n, float* out, void* stream) {
+  if (!h || !h->nm.on) { snprintf(g_err, sizeof(g_err), "normalization not enabled"); return SSA_EINVAL; }
+  if (check_envs(h, envs, n, out)) return SSA_EINVAL;
+  if (n == 0) return SSA_OK;
+  CK(cudaSetDevice(h->device));
+  cudaStream_t st = (cudaStream_t)stream;
+  const long row = h->nm.F / 2;  // a row of F floats as F / 2 doubles (F = 12 m or 4 m is even)
+  memcpy(h->nm.hidx, envs, sizeof(int32_t) * n);
+  CK(cudaMemcpyAsync(h->nm.didx, h->nm.hidx, sizeof(int32_t) * n, cudaMemcpyHostToDevice, st));
+  k_gather_rows<<<(unsigned)((n * row + 255) / 256), 256, 0, st>>>((const double*)h->nm.term, h->nm.didx, n, row, (double*)h->nm.gath);
+  h->launches++;
+  CK(cudaGetLastError());
+  CK(cudaMemcpyAsync(h->nm.hgath, h->nm.gath, sizeof(float) * n * h->nm.F, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  memcpy(out, h->nm.hgath, sizeof(float) * n * h->nm.F);
   return SSA_OK;
 }
 

@@ -442,3 +442,79 @@ SSA_HD double ssa_trace6(const double* P, long stride) {
   t = t + P[20 * stride];
   return t;
 }
+
+// ---- running normalization of observations and returns (episodic mode, k_normalize; ssa_ukf_rollout_normalize) -------
+// Stable-Baselines3's VecNormalize over RunningMeanStd, restated expression by expression so that a learner gets the
+// statistics it already uses.  Two deviations.  With obs_dtype float32 the batch moments are summed in float64 over the
+// float32-rounded rows, where np.mean / np.var of a float32 array would accumulate in float32.  And the order of the
+// batch sums over the E environments: numpy adds the
+// rows of a column in sequence, which a CTA cannot do quickly.  The sums here use ONE order that depends on E only (not
+// on the column, the layout, the launch path or the block shape): leaves of ssa_norm_leaf(E) consecutive rows, each
+// summed in row order from its first element, then the leaf sums combined by the fixed tree of ssa_norm_tree.
+// ssa_norm_leaf keeps the tree at most 1024 leaves wide (8 KB of shared memory per column).
+SSA_HD int ssa_norm_leaf(int E) { return E <= 32768 ? 32 : (E + 1023) / 1024; }
+SSA_HD int ssa_norm_leaves(int E) { return (E + ssa_norm_leaf(E) - 1) / ssa_norm_leaf(E); }
+// an observation value as the caller would see it un-normalized: float32-rounded for obs_dtype float32 (decltype(1.0)
+// names the built-in double also where the operation-counting build, oracle/opcount_twin.cpp, redefines `double`)
+SSA_HD double ssa_norm_in(double v, int f32) { return f32 ? (double)(float)(decltype(1.0))v : v; }
+// the reward that enters the returns: _format_reward's nan_to_num(nan = +-inf = 0.5) for the layouts other than 'flatten'
+SSA_HD double ssa_norm_reward_in(double r, int nan_to_num) { return (nan_to_num && !(r - r == 0.0)) ? 0.5 : r; }
+// one leaf: rows r0 .. r1 - 1 of the column x[r * stride]; sq: the squared deviations from `mean` instead of the values.
+// The rows are loaded 16 at a time before they are added in order: on the device a leaf's strided loads are then in
+// flight together instead of one L2 round trip per row.
+SSA_HD double ssa_norm_leaf_sum(const double* x, long stride, int r0, int r1, int f32, int sq, double mean) {
+  double s = 0.0;
+  for (int b = r0; b < r1; b += 16) {
+    double v[16];
+#pragma unroll
+    for (int j = 0; j < 16; ++j) v[j] = b + j < r1 ? x[(long)(b + j) * stride] : 0.0;
+#pragma unroll
+    for (int j = 0; j < 16; ++j) {
+      if (b + j >= r1) break;
+      double w = ssa_norm_in(v[j], f32);
+      if (sq) {
+        const double d = w - mean;
+        w = d * d;
+      }
+      s = b + j == r0 ? w : s + w;
+    }
+  }
+  return s;
+}
+// the leaf sums v[0 .. n) combined in place, level by level: at level s = 1, 2, 4, ... v[i] += v[i + s] for i = 0, 2s,
+// 4s, ... with i + s < n.  The sum ends in v[0].  (k_normalize runs each level's additions in parallel.)
+SSA_HD double ssa_norm_tree(double* v, int n) {
+  for (int s = 1; s < n; s <<= 1)
+    for (int i = 0; i + s < n; i += 2 * s) v[i] = v[i] + v[i + s];
+  return v[0];
+}
+// np.mean and np.var of a column of E rows (the sum over E, then that of the squared deviations from the mean over E),
+// in the fixed order; buf holds ssa_norm_leaves(E) doubles
+SSA_HD void ssa_norm_moments(const double* x, long stride, int E, int f32, double* buf, double* mean, double* var) {
+  const int L = ssa_norm_leaf(E), n = ssa_norm_leaves(E);
+  for (int k = 0; k < n; ++k) buf[k] = ssa_norm_leaf_sum(x, stride, k * L, k * L + L < E ? k * L + L : E, f32, 0, 0.0);
+  const double mu = ssa_div(ssa_norm_tree(buf, n), (double)E);
+  for (int k = 0; k < n; ++k) buf[k] = ssa_norm_leaf_sum(x, stride, k * L, k * L + L < E ? k * L + L : E, f32, 1, mu);
+  *mean = mu;
+  *var = ssa_div(ssa_norm_tree(buf, n), (double)E);
+}
+// RunningMeanStd.update_from_moments, in its expression order
+SSA_HD void ssa_norm_merge(double* mean, double* var, double* count, double bmean, double bvar, double bcount) {
+  const double delta = bmean - *mean;
+  const double tot = *count + bcount;
+  const double new_mean = *mean + ssa_div(delta * bcount, tot);
+  const double m_a = *var * *count, m_b = bvar * bcount;
+  const double m_2 = m_a + m_b + ssa_div(delta * delta * *count * bcount, tot);
+  *mean = new_mean;
+  *var = ssa_div(m_2, tot);
+  *count = bcount + *count;
+}
+// np.clip(v, -c, c): NaN stays NaN
+SSA_HD double ssa_norm_clip(double v, double c) { return v < -c ? -c : (v > c ? c : v); }
+// VecNormalize.normalize_obs / normalize_reward of one value, with sd = ssa_norm_sd(var, epsilon) of the statistic
+// (the division inlined: it runs once per element)
+SSA_HD double ssa_norm_sd(double var, double eps) { return ssa_sqrt(var + eps); }
+SSA_HD double ssa_norm_obs(double v, double mean, double sd, double clip) { return ssa_norm_clip(ssa_div_i(v - mean, sd), clip); }
+SSA_HD double ssa_norm_reward(double r, double sd, double clip) { return ssa_norm_clip(ssa_div_i(r, sd), clip); }
+// VecNormalize._update_reward: returns * gamma + reward
+SSA_HD double ssa_norm_return(double ret, double gamma, double r) { return ret * gamma + r; }

@@ -162,7 +162,8 @@ class BatchedUKF:
             shape = (6, self.ld)
         elif field == _lib.F_P_FILTER:
             shape = (21, self.ld)
-        typestr = {np.dtype(np.float64): "<f8", np.dtype(np.int32): "<i4", np.dtype(np.uint8): "|u1"}[np.dtype(dtype)]
+        typestr = {np.dtype(np.float64): "<f8", np.dtype(np.float32): "<f4", np.dtype(np.int32): "<i4",
+                   np.dtype(np.uint8): "|u1"}[np.dtype(dtype)]
 
         class _CAI:
             pass
@@ -278,6 +279,7 @@ class BatchedUKF:
         _lib.check(self.lib.ssa_ukf_rollout_truncated(self.h, ctypes.byref(ht), None), "ssa_ukf_rollout_truncated")
         self.rollout_io["truncated"] = view(ht, ctypes.c_uint8, (E,))  # done raised by the step limit alone
         self._term_w = 12
+        self.rollout_norm_io = None  # (a new configuration runs without normalization, rollout_normalize)
         return self.rollout_io
 
     def rollout_reset(self, stream=None):
@@ -328,6 +330,58 @@ class BatchedUKF:
         others keep their state and outputs.  rollout_io is valid after a sync."""
         envs = np.ascontiguousarray(envs, dtype=np.int32).reshape(-1)
         _lib.check(self.lib.ssa_ukf_rollout_reset_envs(self.h, _ptr(envs), len(envs), stream), "ssa_ukf_rollout_reset_envs")
+
+    def rollout_normalize(self, on=True, obs_layout=_lib.NORM_OBS_ROWS, reward_nan_to_num=False, training=True, norm_obs=True,
+                          norm_reward=True, clip_obs=10.0, clip_reward=10.0, gamma=0.99, epsilon=1e-8):
+        """Stable-Baselines3's VecNormalize inside the step graph (include/ssa_ukf.h, ssa_ukf_rollout_normalize); on=False
+        turns it off.  obs_layout (NORM_OBS_*) must match the steps' obs_f32 / obs_aer.  After rollout_config (which
+        turns it off).  rollout_norm_io: pinned host views of the normalized obs [E, F] float32 and rewards [E]."""
+        if not on:
+            _lib.check(self.lib.ssa_ukf_rollout_normalize(self.h, None), "ssa_ukf_rollout_normalize")
+            self.rollout_norm_io = None
+            return None
+        c = _lib.SsaNormCfg(int(bool(norm_obs)), int(bool(norm_reward)), int(bool(training)), int(obs_layout),
+                            int(bool(reward_nan_to_num)), float(clip_obs), float(clip_reward), float(gamma), float(epsilon))
+        _lib.check(self.lib.ssa_ukf_rollout_normalize(self.h, ctypes.byref(c)), "ssa_ukf_rollout_normalize")
+        F = self.m * (4 if obs_layout == _lib.NORM_OBS_AER else 12)
+        self.norm_F = F
+        E = self.n_envs
+        self._shapes[_lib.F_ROLLOUT_OBS_NORM] = ((E, F), np.float32)
+        self._shapes[_lib.F_ROLLOUT_TERMINAL_OBS_NORM] = ((E, F), np.float32)
+        self._shapes[_lib.F_ROLLOUT_REWARD_NORM] = ((E,), np.float64)
+        self._shapes[_lib.F_ROLLOUT_NORM_STATE] = ((4 + E + 3 * F,), np.float64)
+        ho, hr = ctypes.c_void_p(), ctypes.c_void_p()
+        _lib.check(self.lib.ssa_ukf_rollout_norm_io(self.h, ctypes.byref(ho), ctypes.byref(hr)), "ssa_ukf_rollout_norm_io")
+        self.rollout_norm_io = {
+            "obs": np.ctypeslib.as_array(ctypes.cast(ho, ctypes.POINTER(ctypes.c_float)), shape=(E * F,)).reshape(E, F),
+            "reward": np.ctypeslib.as_array(ctypes.cast(hr, ctypes.POINTER(ctypes.c_double)), shape=(E,))}
+        return self.rollout_norm_io
+
+    def rollout_norm_state(self, stream=None):
+        """The normalization state: {'obs_mean' [F], 'obs_var' [F], 'obs_count', 'ret_mean', 'ret_var', 'ret_count',
+        'returns' [E]} (VecNormalize's obs_rms, ret_rms and returns); blocks until copied."""
+        F, E = self.norm_F, self.n_envs
+        out = np.empty(2 * F + 4 + E)
+        _lib.check(self.lib.ssa_ukf_rollout_norm_state_download(self.h, _ptr(out), out.size, stream),
+                   "ssa_ukf_rollout_norm_state_download")
+        return {"obs_mean": out[:F], "obs_var": out[F:2 * F], "obs_count": float(out[2 * F]), "ret_mean": float(out[2 * F + 1]),
+                "ret_var": float(out[2 * F + 2]), "ret_count": float(out[2 * F + 3]), "returns": out[2 * F + 4:]}
+
+    def rollout_load_norm_state(self, state, stream=None):
+        """Restore a rollout_norm_state() dict (training keeps its current setting); blocks until copied."""
+        F, E = self.norm_F, self.n_envs
+        buf = np.concatenate([np.asarray(state["obs_mean"], np.float64).reshape(F), np.asarray(state["obs_var"], np.float64).reshape(F),
+                              [state["obs_count"], state["ret_mean"], state["ret_var"], state["ret_count"]],
+                              np.asarray(state["returns"], np.float64).reshape(E)])
+        _lib.check(self.lib.ssa_ukf_rollout_norm_state_upload(self.h, _ptr(buf), buf.size, stream), "ssa_ukf_rollout_norm_state_upload")
+
+    def rollout_terminal_obs_norm(self, envs, stream=None):
+        """The normalized final observations float32 [len(envs), F] of the environments `envs` (as rollout_terminal_obs)."""
+        envs = np.ascontiguousarray(envs, dtype=np.int32).reshape(-1)
+        out = np.empty((len(envs), self.norm_F), dtype=np.float32)
+        _lib.check(self.lib.ssa_ukf_rollout_terminal_obs_norm_download(self.h, _ptr(envs), len(envs), _ptr(out), stream),
+                   "ssa_ukf_rollout_terminal_obs_norm_download")
+        return out
 
     @property
     def next_parity(self):

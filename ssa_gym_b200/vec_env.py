@@ -35,6 +35,16 @@ kept on the device before their re-draw (device_views()['terminal_obs'], `Batche
 step where environments finish) every finished environment gets `infos[e]['TimeLimit.truncated']`, and in the device
 mode with auto-reset also `infos[e]['terminal_observation']` in the layout and dtype of the observations (the host mode
 always fills that key on its auto-resets).  `reset_at(e)` re-draws environment e alone in either mode.
+
+No policy learns from these observations raw (positions up to 4e7 m, covariance diagonals from 1e10 m^2 down by eight
+orders of magnitude), and the usual remedy, Stable-Baselines3's VecNormalize, is a numpy pass over the [E, F] block on
+every step.  With `config['normalize'] = True` (or a dict of VecNormalize's keyword arguments: training, norm_obs,
+norm_reward, clip_obs, clip_reward, gamma, epsilon) the device mode does the same inside the step graph
+(ssa_ukf_rollout_normalize, one kernel): observations and rewards come back normalized, the observations as float32,
+and the step copies those instead of the raw float64 rows.  VecNormalize's semantics, its order of updates and its
+defaults; infos[e]['terminal_observation'] is normalized as VecNormalize does, infos[e]['episode'] keeps the raw
+return.  get_original_obs() / get_original_reward(), normalizer_state() / load_normalizer_state() and `training` follow
+VecNormalize's names.
 """
 import numpy as np
 
@@ -56,6 +66,10 @@ _TASKERS = {
     agents.agent_visible_greedy_spoiled: F.TASKER_VISIBLE_GREEDY_SPOILED,
 }
 _TASKER_NAMES = {f.__name__[len("agent_"):]: k for f, k in _TASKERS.items()}
+
+# VecNormalize's keyword arguments and defaults (config['normalize'])
+_NORM_DEFAULTS = {"training": True, "norm_obs": True, "norm_reward": True, "clip_obs": 10.0, "clip_reward": 10.0,
+                  "gamma": 0.99, "epsilon": 1e-8}
 
 
 def episode_info(rec):
@@ -110,6 +124,20 @@ class VecSSATaskerEnv:
             raise ValueError("episode_stats=True needs rng='device'")
         # infos[e]['TimeLimit.truncated'] on every finished environment, and the device mode's terminal_observation
         self.terminal_observation = bool(config.get('terminal_observation', False))
+        # running normalization of observations and returns inside the step graph (VecNormalize; device mode only)
+        nz = config.get('normalize', False)
+        if nz is not True and not isinstance(nz, dict) and nz not in (False, None):
+            raise ValueError("normalize must be True, False or a dict of VecNormalize keyword arguments")
+        self.normalize = nz is True or isinstance(nz, dict)
+        if self.normalize:
+            if rng != 'device':
+                raise ValueError("normalize needs rng='device'")
+            kw = {} if nz is True else dict(nz)
+            unknown = sorted(set(kw) - set(_NORM_DEFAULTS))
+            if unknown:
+                raise ValueError(f"unknown normalize keys {unknown}; VecNormalize's are {sorted(_NORM_DEFAULTS)}")
+            self._norm_kw = dict(_NORM_DEFAULTS, **kw)
+            self._norm_kw["training"] = bool(self._norm_kw["training"])
         self.update_interval = config['update_interval']
         self.auto_reset = auto_reset
         if config.get('orbits') is not None:
@@ -165,6 +193,9 @@ class VecSSATaskerEnv:
             self._infos_filled = []  # environments whose info dict holds the 'episode' entry of the previous step
             if self.episode_stats:
                 self.ukf.rollout_episode_stats_enable()  # (accumulates from the rollout_reset of vector_reset on)
+            if self.normalize:
+                self._apply_normalize()  # (vector_reset below updates the observation statistics, VecNormalize.reset)
+            self._old_reward = np.zeros(self.E)
         self.obs = self.vector_reset()
 
     # -- seeding / reset --------------------------------------------------------------------------------
@@ -242,7 +273,11 @@ class VecSSATaskerEnv:
         self.ukf.env_reduce(step_index=-1)
 
     def _device_obs(self):
-        """rng='device': the observations of the output block after a (partial) reset, in the configured layout and dtype."""
+        """rng='device': the observations of the output block after a (partial) reset, in the configured layout and dtype
+        (normalized float32 with config['normalize'])."""
+        if self.normalize:
+            rows = self.ukf.rollout_norm_io["obs"]
+            return rows if self._obs_aer else self._format_obs(rows)
         if self._obs_aer:
             return self._io["obs_aer"].reshape(self.E, self.m * 4)
         return self._format_obs(self._io["obs"].reshape(self.E, self.m * 12).astype(self.obs_dtype, copy=False))
@@ -383,7 +418,11 @@ class VecSSATaskerEnv:
         if self.auto_reset:
             self.i[dones] = 0
             self.episodes[dones] += 1
-        if self._obs_aer:
+        if self.normalize:
+            self._old_reward = self._format_reward(rewards)
+            rewards = self.ukf.rollout_norm_io["reward"].copy()
+            self.obs = self._device_obs()
+        elif self._obs_aer:
             self.obs = io["obs_aer"].reshape(self.E, self.m * 4)
         else:
             self.obs = self._format_obs(io["obs_f32" if f32 else "obs"].reshape(self.E, self.m * 12))
@@ -401,12 +440,62 @@ class VecSSATaskerEnv:
                 for e, t in zip(de, self.truncated[de].tolist()):
                     infos[e]["TimeLimit.truncated"] = t
                 if self.auto_reset:  # one download of the final rows, in the layout and dtype of the observations
-                    rows = self.ukf.rollout_terminal_obs(de)
-                    term = rows if self._obs_aer else self._format_obs(rows.astype(self.obs_dtype, copy=False))
+                    if self.normalize:  # (normalized with the step's statistics, as VecNormalize does)
+                        rows = self.ukf.rollout_terminal_obs_norm(de)
+                        term = rows if self._obs_aer else self._format_obs(rows)
+                    else:
+                        rows = self.ukf.rollout_terminal_obs(de)
+                        term = rows if self._obs_aer else self._format_obs(rows.astype(self.obs_dtype, copy=False))
                     for k, e in enumerate(de):
                         infos[e]["terminal_observation"] = term[k]
             self._infos_filled = de
-        return self.obs, self._format_reward(rewards), dones, infos
+        return self.obs, (rewards if self.normalize else self._format_reward(rewards)), dones, infos
+
+    # -- running normalization (config['normalize']; Stable-Baselines3 VecNormalize's names) -------------------------
+    def _need_normalize(self):
+        if not self.normalize:
+            raise ValueError("normalization is off: construct with config['normalize'] = True (rng='device')")
+
+    def _apply_normalize(self):
+        layout = F.NORM_OBS_AER if self._obs_aer else F.NORM_OBS_ROWS_F32 if self.obs_dtype == np.float32 else F.NORM_OBS_ROWS
+        self.ukf.rollout_normalize(obs_layout=layout, reward_nan_to_num=self.obs_returned != 'flatten', **self._norm_kw)
+
+    @property
+    def training(self):
+        """VecNormalize.training: with False the statistics and the returns stay as they are (a device flag: setting it
+        re-captures nothing)."""
+        self._need_normalize()
+        return self._norm_kw["training"]
+
+    @training.setter
+    def training(self, value):
+        self._need_normalize()
+        self._norm_kw["training"] = bool(value)
+        self._apply_normalize()
+
+    def get_original_obs(self):
+        """The observations of the last step or reset before normalization, in the layout and dtype they would have without
+        it (downloaded from the device on demand)."""
+        self._need_normalize()
+        if self._obs_aer:
+            return self.ukf.download(F.F_ROLLOUT_OBS_AER).reshape(self.E, self.m * 4)
+        return self._format_obs(self.ukf.download(F.F_ROLLOUT_OBS).reshape(self.E, self.m * 12).astype(self.obs_dtype, copy=False))
+
+    def get_original_reward(self):
+        """The rewards of the last step before normalization (after the layout's nan_to_num)."""
+        self._need_normalize()
+        return self._old_reward.copy()
+
+    def normalizer_state(self):
+        """{'obs_mean' [F], 'obs_var' [F], 'obs_count', 'ret_mean', 'ret_var', 'ret_count', 'returns' [E]}: VecNormalize's
+        obs_rms, ret_rms and returns, for a checkpoint or an evaluation env (load_normalizer_state)."""
+        self._need_normalize()
+        return self.ukf.rollout_norm_state()
+
+    def load_normalizer_state(self, state):
+        """Restore a normalizer_state() dict; `training` keeps its setting.  The next step normalizes with it."""
+        self._need_normalize()
+        self.ukf.rollout_load_norm_state(state)
 
     # -- device-resident consumer (a policy on the same GPU): no host copies, nothing synchronises -------------------
     def device_views(self):
@@ -419,6 +508,8 @@ class VecSSATaskerEnv:
         With config['episode_stats']: 'episode_stats' float64 [E, EPISODE_STATS_DOUBLES], the record of each environment's
         last finished episode (layout: include/ssa_ukf.h; episode_info turns a row into the infos entry), valid after a
         step whose 'done' is set for it.
+        With config['normalize']: 'obs_norm' float32 [E, F] (F = m*12, or m*4 for 'aer'), 'reward_norm' float64 [E] and
+        'terminal_obs_norm' float32 [E, F] (with auto-reset, valid like 'terminal_obs').
         The outputs are overwritten by every step; they are valid in stream order on the stream the step runs on."""
         assert self.rng == 'device', "device views exist in the device-resident episodic mode (rng='device')"
         if getattr(self, "_views", None) is None:
@@ -433,6 +524,10 @@ class VecSSATaskerEnv:
                            "terminal_obs": term}
             if self.episode_stats:
                 self._views["episode_stats"] = u.torch_view(F.F_ROLLOUT_EPISODE_STATS)
+            if self.normalize:
+                self._views.update({"obs_norm": u.torch_view(F.F_ROLLOUT_OBS_NORM),
+                                    "reward_norm": u.torch_view(F.F_ROLLOUT_REWARD_NORM),
+                                    "terminal_obs_norm": u.torch_view(F.F_ROLLOUT_TERMINAL_OBS_NORM)})
         return self._views
 
     def vector_step_device(self, stream=None):
@@ -441,7 +536,8 @@ class VecSSATaskerEnv:
         no synchronisation (the reference hands every observation to the learner process through the host, SURVEY 3.4).
         The host mirrors (self.i, self.episodes) are not maintained in this mode."""
         assert self.rng == 'device'
-        self.ukf.rollout_step(self.auto_reset, stream=stream, device_io=True, obs_aer=self._obs_aer)
+        self.ukf.rollout_step(self.auto_reset, stream=stream, device_io=True, obs_aer=self._obs_aer,
+                              obs_f32=self.normalize and self.obs_dtype == np.float32)  # (the normalization's layout)
         return self.device_views()
 
     # -- device taskers --------------------------------------------------------------------------------------
