@@ -1733,6 +1733,29 @@ int set_err(const char* what, cudaError_t e) {
 // ---------------------------------------------------------------------------------------------------
 // C ABI
 // ---------------------------------------------------------------------------------------------------
+// The output block of the episodic mode (include/ssa_ukf.h), on the device and as its pinned host mirror:
+// [obs 12N doubles][reward E doubles][greedy 6E int32][done E bytes, padded to 8][truncated E bytes, padded to 8]
+struct RolloutBlock {
+  double* obs; double* reward; int32_t* greedy; uint8_t* done; uint8_t* truncated;
+  size_t bytes;  // of the whole block
+  size_t tail;   // byte offset of reward .. truncated (what follows the observation rows)
+};
+
+// the views of the block at base (null: only its sizes)
+static RolloutBlock rollout_block(void* base, size_t N, size_t E) {
+  RolloutBlock b = {};
+  const size_t flags = (E + 7) / 8 * 8;
+  b.tail = sizeof(double) * 12 * N;
+  b.bytes = sizeof(double) * (12 * N + E) + sizeof(int32_t) * SSA_N_TASKERS * E + 2 * flags;
+  if (!base) return b;
+  b.obs = (double*)base;
+  b.reward = b.obs + 12 * N;
+  b.greedy = (int32_t*)(b.reward + E);
+  b.done = (uint8_t*)(b.greedy + SSA_N_TASKERS * E);
+  b.truncated = b.done + flags;
+  return b;
+}
+
 struct ssa_ukf {
   ssa_ukf_cfg cfg;
   int device;
@@ -1758,6 +1781,9 @@ struct ssa_ukf {
   int use_fused;  // one launch per full catalog step (k_step_tile) instead of the four tile kernels
   int legacy_act; // SSA_UKF_ACT=split: the RL-mode update of the tasked objects runs as k_hx + k_update instead of k_update_tile
   int fold_factor;  // tile2: the two factorisations inside the tile kernels instead of k_factor / k_refactor
+  int use_graph;    // ssa_ukf_step_pinned / ssa_ukf_rollout_step as captured graphs (SSA_UKF_GRAPH=0: plain launches)
+  int det_kernel;   // SSA_UKF_DET_KERNEL set: ssa_det_kernel also for m <= 64, not the determinants inside the reduction
+  int refresh_chain;  // SSA_UKF_REFRESH_CHAIN set: an auto-reset step re-draws with k_env_reset + the refresh chain
   int sm_count;
   // double-buffered host pipeline (ssa_ukf_step_host)
   struct {
@@ -1775,7 +1801,6 @@ struct ssa_ukf {
     size_t out_doubles, in_off, in_doubles;
     cudaGraphExec_t gexec[2];  // the step's kernel chain captured per parity (ssa_ukf_step_pinned)
     int gflags[2], gkernels[2];
-    int use_graph;
   } hp;
   // ssa_ukf_step as one graph launch (SSA_UKF_STEP_GRAPH=0: five plain launches).  The only launch parameter that
   // changes from step to step is the trans_matrix, which only k_hx reads: its kernel node is re-parameterised
@@ -1798,23 +1823,22 @@ struct ssa_ukf {
     uint32_t* ibuf;      // device: key [E][2], episode [E], act_in [E], act_eff [E]
     uint32_t *key, *episode;
     int32_t *act_in, *act_eff;
-    double* dout;        // device out block: [obs 12N][reward E][greedy 6E int32][done E uint8][truncated E uint8]
-    double* hout;        // pinned host mirror
+    RolloutBlock dev, host;  // the output block and its pinned host mirror
     int32_t* hin;        // pinned host actions [E]
-    size_t out_bytes;
     float *dobs32, *hobs32;    // SSA_ROLLOUT_OBS_F32: obs [N][12] as floats (device block, pinned host mirror)
     double *daer, *haer;       // SSA_ROLLOUT_OBS_AER: the 'aer' observation [N][4] (device block, pinned host mirror)
     double* rew_hist;          // 'shaped' only: [E][n_steps] reward history, then spos_prev [E] int32
     int32_t* spos_prev;
     int tasker;                // ssa_ukf_rollout_tasker
     double spoil_p;
-    // final observations (ssa_ukf_rollout_terminal_obs_download) and ssa_ukf_rollout_reset_envs
-    double* tbuf;              // device: terminal [12N], gathered rows [12N], then idx [E] int32, mask [E] uint8
-    double *term, *tgath;
-    int32_t* tidx;
+    // final observations (ssa_ukf_rollout_terminal_obs_download), ssa_ukf_rollout_reset_envs, and the rows of every
+    // gathered download (gather_download: final observations, episode records, normalized final observations)
+    double* tbuf;              // device: terminal [12N], gathered rows [max(12N, SSA_EPR E)], then idx [E] int32, mask [E] uint8
+    double *term, *gath;
+    int32_t* gidx;
     uint8_t* mask;
-    double* htbuf;             // pinned: gathered rows [12N], then idx [E] int32
-    int32_t* htidx;
+    double* hgath;             // pinned: gathered rows [max(12N, SSA_EPR E)], then idx [E] int32
+    int32_t* hgidx;
     int term_w;                // doubles per object of the terminal rows: 12, 4 after an SSA_ROLLOUT_OBS_AER auto-reset step
     cudaGraphExec_t gexec[6];  // [auto_reset + 2 * (obs_f32 ? 1 : obs_aer ? 2 : 0)]
     int gkernels[6];
@@ -1823,11 +1847,8 @@ struct ssa_ukf {
   struct {
     int on;              // buffers allocated (ssa_ukf_rollout_episode_stats_enable)
     int live;            // accumulating: the step graphs carry k_ep_row0 / k_ep_step (from the next rollout_reset on)
-    double* buf;         // device: obj [N][SSA_EPO], env [E][SSA_EPE], rec [E][SSA_EPR], gathered [E][SSA_EPR], idx [E]
-    double *obj, *env, *rec, *gath;
-    int32_t* didx;
-    double* hbuf;        // pinned: gathered records [E][SSA_EPR], then idx [E] int32
-    int32_t* hidx;
+    double* buf;         // device: obj [N][SSA_EPO], env [E][SSA_EPE], rec [E][SSA_EPR]
+    double *obj, *env, *rec;
   } es;
   // running normalization of observations and returns in the episodic mode (ssa_ukf_rollout_normalize, k_normalize)
   struct {
@@ -1835,13 +1856,11 @@ struct ssa_ukf {
     int F;               // normalized columns per environment: 12 m, or 4 m for SSA_NORM_OBS_AER
     ssa_norm_cfg cfg;
     double* buf;         // device: state [4 + E + 3F] (SSA_F_ROLLOUT_NORM_STATE), reward_norm [E], then floats obs_norm,
-                         // term_norm, gathered rows [E][F] each, then idx [E] int32
+                         // term_norm [E][F] each
     double *state, *reward;
-    float *obs, *term, *gath;
-    int32_t* didx;
-    double* hbuf;        // pinned: reward_norm [E], obs_norm [E][F] floats (the step copies both at once), gathered rows
-    float *hobs, *hgath; //         [E][F] floats, idx [E] int32
-    int32_t* hidx;
+    float *obs, *term;
+    double* hbuf;        // pinned: reward_norm [E], obs_norm [E][F] floats (the step copies both at once)
+    float* hobs;
   } nm;
   int32_t *status, *infl, *actions, *greedy;
   uint8_t *visible, *updated, *innov_flags, *done;
@@ -1853,6 +1872,62 @@ struct ssa_ukf {
                                          // block of the double-buffered host pipeline)
   size_t stage_bytes;
 };
+
+// Captures the kernels that enqueue(stream) launches into *exec: a non-blocking stream in thread-local capture mode,
+// instantiated without flags.  *kernels: the launches it made (the handle's counter is left as it was; every launch of
+// the graph adds them).  keep: receives the captured graph, which the caller then owns; null: destroyed here.
+template <typename Enqueue>
+static int capture_chain(ssa_ukf* h, Enqueue&& enqueue, cudaGraph_t* keep, cudaGraphExec_t* exec, int* kernels) {
+  cudaStream_t cs;
+  CK(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
+  const long l0 = h->launches;
+  CK(cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal));
+  const int rc = enqueue(cs);
+  cudaGraph_t g = nullptr;
+  const cudaError_t ce = cudaStreamEndCapture(cs, &g);
+  *kernels = (int)(h->launches - l0);
+  h->launches = l0;
+  cudaStreamDestroy(cs);
+  if (rc) { if (g) cudaGraphDestroy(g); return rc; }
+  if (ce != cudaSuccess) return set_err("cudaStreamEndCapture", ce);
+  const cudaError_t ie = cudaGraphInstantiate(exec, g, 0);
+  if (ie == cudaSuccess && keep) { *keep = g; return SSA_OK; }
+  cudaGraphDestroy(g);
+  return ie == cudaSuccess ? SSA_OK : set_err("cudaGraphInstantiate", ie);
+}
+
+// the guard of the ssa_ukf_rollout_* entry points that need ssa_ukf_rollout_config
+static bool rollout_ready(const ssa_ukf* h) {
+  if (h && h->ro.init) return true;
+  snprintf(g_err, sizeof(g_err), "episodic mode not configured");
+  return false;
+}
+
+// the captured step graphs of the episodic mode (re-captured on the next ssa_ukf_rollout_step)
+static void rollout_drop_graphs(ssa_ukf* h) {
+  for (int i = 0; i < 6; ++i) if (h->ro.gexec[i]) { cudaGraphExecDestroy(h->ro.gexec[i]); h->ro.gexec[i] = nullptr; }
+}
+
+// The only code that frees the buffers of the episodic mode, of its episode statistics and of its normalization; each
+// leaves its part of the handle zeroed (not configured / not enabled).
+static void rollout_free(ssa_ukf* h) {
+  cudaFree(h->ro.dbuf); cudaFree(h->ro.ibuf); cudaFree(h->ro.dev.obs); cudaFree(h->ro.dobs32);
+  cudaFree(h->ro.daer); cudaFree(h->ro.rew_hist); cudaFree(h->ro.tbuf);
+  cudaFreeHost(h->ro.host.obs); cudaFreeHost(h->ro.hin); cudaFreeHost(h->ro.hobs32); cudaFreeHost(h->ro.haer);
+  cudaFreeHost(h->ro.hgath);
+  rollout_drop_graphs(h);
+  memset(&h->ro, 0, sizeof(h->ro));
+}
+
+static void episode_stats_free(ssa_ukf* h) {
+  cudaFree(h->es.buf);
+  memset(&h->es, 0, sizeof(h->es));
+}
+
+static void norm_free(ssa_ukf* h) {
+  cudaFree(h->nm.buf); cudaFreeHost(h->nm.hbuf);
+  memset(&h->nm, 0, sizeof(h->nm));
+}
 
 extern "C" {
 
@@ -1971,6 +2046,10 @@ int ssa_ukf_create(const ssa_ukf_cfg* cfg, int device, ssa_ukf** out) {
     cudaFuncSetAttribute(k_step_tile<SSA_TILE, kTileThreads>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(UpdateTile<SSA_TILE>));
     const char* gv = getenv("SSA_UKF_STEP_GRAPH");
     h->sg.on = (gv && strcmp(gv, "0") == 0) ? 0 : 1;
+    const char* cg = getenv("SSA_UKF_GRAPH");
+    h->use_graph = (cg && strcmp(cg, "0") == 0) ? 0 : 1;
+    h->det_kernel = getenv("SSA_UKF_DET_KERNEL") ? 1 : 0;
+    h->refresh_chain = getenv("SSA_UKF_REFRESH_CHAIN") ? 1 : 0;
     const char* pv = getenv("SSA_UKF_PDL");
     h->pdl = (pv && strcmp(pv, "0") == 0) ? 0 : 1;
     h->staged_max = kStagedMaxDefault;
@@ -2006,15 +2085,9 @@ int ssa_ukf_destroy(ssa_ukf* h) {
     cudaStreamDestroy(h->hp.up); cudaStreamDestroy(h->hp.dn);
   }
   for (int i = 0; i < h->sg.n; ++i) { cudaGraphExecDestroy(h->sg.gexec[i]); cudaGraphDestroy(h->sg.graph[i]); }
-  if (h->ro.init) {
-    cudaFree(h->ro.dbuf); cudaFree(h->ro.ibuf); cudaFree(h->ro.dout); cudaFree(h->ro.dobs32);
-    cudaFree(h->ro.daer); cudaFree(h->ro.rew_hist); cudaFree(h->ro.tbuf);
-    cudaFreeHost(h->ro.hout); cudaFreeHost(h->ro.hin); cudaFreeHost(h->ro.hobs32); cudaFreeHost(h->ro.haer);
-    cudaFreeHost(h->ro.htbuf);
-    for (int i = 0; i < 6; ++i) if (h->ro.gexec[i]) cudaGraphExecDestroy(h->ro.gexec[i]);
-  }
-  if (h->es.on) { cudaFree(h->es.buf); cudaFreeHost(h->es.hbuf); }
-  if (h->nm.on) { cudaFree(h->nm.buf); cudaFreeHost(h->nm.hbuf); }
+  rollout_free(h);
+  episode_stats_free(h);
+  norm_free(h);
   cudaFree(h->snap);
   cudaFree(h->cat_part);
   cudaFree(h->stage);
@@ -2096,34 +2169,26 @@ static int field_info(ssa_ukf* h, int field, void** p, size_t* bytes, int* soa_c
     case SSA_F_CATALOG_STATS:
       if (!h->cat_stats) { snprintf(g_err, sizeof(g_err), "call ssa_ukf_catalog_stats first"); return SSA_EINVAL; }
       *p = h->cat_stats; *bytes = 5 * 8; break;
-    case SSA_F_ROLLOUT_OBS:
-      if (!h->ro.init) { snprintf(g_err, sizeof(g_err), "episodic mode not configured"); return SSA_EINVAL; }
-      *p = h->ro.dout; *bytes = N * 12 * 8; break;
-    case SSA_F_ROLLOUT_REWARD:
-      if (!h->ro.init) { snprintf(g_err, sizeof(g_err), "episodic mode not configured"); return SSA_EINVAL; }
-      *p = h->ro.dout + 12 * N; *bytes = E * 8; break;
-    case SSA_F_ROLLOUT_ACTIONS:
-      if (!h->ro.init) { snprintf(g_err, sizeof(g_err), "episodic mode not configured"); return SSA_EINVAL; }
-      *p = h->ro.act_in; *bytes = E * 4; break;
-    case SSA_F_ROLLOUT_GREEDY:
-      if (!h->ro.init) { snprintf(g_err, sizeof(g_err), "episodic mode not configured"); return SSA_EINVAL; }
-      *p = (int32_t*)(h->ro.dout + 12 * N + E); *bytes = E * SSA_N_TASKERS * 4; break;
-    case SSA_F_ROLLOUT_DONE:
-      if (!h->ro.init) { snprintf(g_err, sizeof(g_err), "episodic mode not configured"); return SSA_EINVAL; }
-      *p = (uint8_t*)((int32_t*)(h->ro.dout + 12 * N + E) + SSA_N_TASKERS * E); *bytes = E; break;
     case SSA_F_INNOV_FLAGS: *p = h->innov_flags; *bytes = N; break;
-    case SSA_F_ROLLOUT_OBS_AER:
-      if (!h->ro.init) { snprintf(g_err, sizeof(g_err), "episodic mode not configured"); return SSA_EINVAL; }
-      *p = h->ro.daer; *bytes = N * 4 * 8; break;
+    case SSA_F_ROLLOUT_OBS: case SSA_F_ROLLOUT_REWARD: case SSA_F_ROLLOUT_ACTIONS: case SSA_F_ROLLOUT_GREEDY:
+    case SSA_F_ROLLOUT_DONE: case SSA_F_ROLLOUT_OBS_AER: case SSA_F_ROLLOUT_TERMINAL_OBS: case SSA_F_ROLLOUT_TRUNCATED: {
+      if (!rollout_ready(h)) return SSA_EINVAL;
+      const RolloutBlock& b = h->ro.dev;
+      switch (field) {
+        case SSA_F_ROLLOUT_OBS: *p = b.obs; *bytes = N * 12 * 8; break;
+        case SSA_F_ROLLOUT_REWARD: *p = b.reward; *bytes = E * 8; break;
+        case SSA_F_ROLLOUT_ACTIONS: *p = h->ro.act_in; *bytes = E * 4; break;
+        case SSA_F_ROLLOUT_GREEDY: *p = b.greedy; *bytes = E * SSA_N_TASKERS * 4; break;
+        case SSA_F_ROLLOUT_DONE: *p = b.done; *bytes = E; break;
+        case SSA_F_ROLLOUT_OBS_AER: *p = h->ro.daer; *bytes = N * 4 * 8; break;
+        case SSA_F_ROLLOUT_TERMINAL_OBS: *p = h->ro.term; *bytes = N * 12 * 8; break;
+        case SSA_F_ROLLOUT_TRUNCATED: *p = b.truncated; *bytes = E; break;
+      }
+      break;
+    }
     case SSA_F_ROLLOUT_EPISODE_STATS:
       if (!h->es.on) { snprintf(g_err, sizeof(g_err), "episode statistics not enabled"); return SSA_EINVAL; }
       *p = h->es.rec; *bytes = E * SSA_EPR * 8; break;
-    case SSA_F_ROLLOUT_TERMINAL_OBS:
-      if (!h->ro.init) { snprintf(g_err, sizeof(g_err), "episodic mode not configured"); return SSA_EINVAL; }
-      *p = h->ro.term; *bytes = N * 12 * 8; break;
-    case SSA_F_ROLLOUT_TRUNCATED:
-      if (!h->ro.init) { snprintf(g_err, sizeof(g_err), "episodic mode not configured"); return SSA_EINVAL; }
-      *p = (uint8_t*)((int32_t*)(h->ro.dout + 12 * N + E) + SSA_N_TASKERS * E) + ((E + 7) / 8) * 8; *bytes = E; break;
     case SSA_F_ROLLOUT_OBS_NORM: case SSA_F_ROLLOUT_REWARD_NORM: case SSA_F_ROLLOUT_TERMINAL_OBS_NORM:
     case SSA_F_ROLLOUT_NORM_STATE: {
       if (!h->nm.on) { snprintf(g_err, sizeof(g_err), "normalization not enabled"); return SSA_EINVAL; }
@@ -2363,24 +2428,15 @@ int ssa_ukf_step(ssa_ukf* h, const double M[9], int flags, void* stream) {
   if (gi < 0) {  // capture the chain for this flag combination (at most 4 are cached)
     if (h->sg.n == 4) { cudaGraphExecDestroy(h->sg.gexec[3]); cudaGraphDestroy(h->sg.graph[3]); h->sg.n = 3; }
     gi = h->sg.n;
-    cudaStream_t cs;
-    CK(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
-    const long l0 = h->launches;
-    CK(cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal));
-    const int rc = step_impl(h, M, flags, cs, nullptr, -1, nullptr, &h->sg.p[gi]);
-    cudaGraph_t g = nullptr;
-    const cudaError_t ce = cudaStreamEndCapture(cs, &g);
-    h->sg.gkernels[gi] = (int)(h->launches - l0);
-    h->launches = l0;
-    cudaStreamDestroy(cs);
-    if (rc) { if (g) cudaGraphDestroy(g); return rc; }
-    if (ce != cudaSuccess) return set_err("cudaStreamEndCapture", ce);
+    const int rc = capture_chain(h, [&](cudaStream_t cs) { return step_impl(h, M, flags, cs, nullptr, -1, nullptr, &h->sg.p[gi]); },
+                                 &h->sg.graph[gi], &h->sg.gexec[gi], &h->sg.gkernels[gi]);
+    if (rc) return rc;
     h->sg.hx_node[gi] = nullptr;
     size_t nn = 0;
-    cudaGraphGetNodes(g, nullptr, &nn);
+    cudaGraphGetNodes(h->sg.graph[gi], nullptr, &nn);
     cudaGraphNode_t nodes[16];
     if (nn > 16) nn = 16;
-    cudaGraphGetNodes(g, nodes, &nn);
+    cudaGraphGetNodes(h->sg.graph[gi], nodes, &nn);
     for (size_t i = 0; i < nn; ++i) {
       cudaGraphNodeType ty;
       cudaKernelNodeParams kp;
@@ -2393,9 +2449,6 @@ int ssa_ukf_step(ssa_ukf* h, const double M[9], int flags, void* stream) {
         h->sg.hx_params[gi] = kp;
       }
     }
-    const cudaError_t ie = cudaGraphInstantiate(&h->sg.gexec[gi], g, 0);
-    if (ie != cudaSuccess) { cudaGraphDestroy(g); return set_err("cudaGraphInstantiate", ie); }
-    h->sg.graph[gi] = g;
     h->sg.flags[gi] = flags;
     h->sg.n = gi + 1;
   }
@@ -2420,10 +2473,6 @@ static int hostpipe_init(ssa_ukf* h) {
   h->hp.out_doubles = 12 * N + ld + ld / 2;
   h->hp.in_off = h->hp.out_doubles + 4 * ld;
   h->hp.in_doubles = 3 * N + 10 + (E + 1) / 2;
-  {
-    const char* gv = getenv("SSA_UKF_GRAPH");
-    h->hp.use_graph = (gv && strcmp(gv, "0") == 0) ? 0 : 1;
-  }
   for (int b = 0; b < 2; ++b) {
     const size_t tot = h->hp.in_off + h->hp.in_doubles;
     CK(cudaMalloc(&h->hp.block[b], sizeof(double) * tot));
@@ -2536,24 +2585,12 @@ int ssa_ukf_step_pinned(ssa_ukf* h, int flags, void* stream, int* parity_used) {
   // compute on the caller's stream: needs this step's inputs and a drained output buffer
   CK(cudaStreamWaitEvent(st, h->hp.e_up[b], 0));
   if (h->hp.calls >= 2) CK(cudaStreamWaitEvent(st, h->hp.e_dn[b], 0));
-  if (h->hp.use_graph && !h->use_team) {
+  if (h->use_graph && !h->use_team) {
     if (!h->hp.gexec[b] || h->hp.gflags[b] != flags) {  // (re)capture the kernel chain of this parity
       if (h->hp.gexec[b]) { cudaGraphExecDestroy(h->hp.gexec[b]); h->hp.gexec[b] = nullptr; }
-      cudaStream_t cs;
-      CK(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
-      const long l0 = h->launches;
-      CK(cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal));
-      rc = step_impl(h, nullptr, flags, cs, nullptr, b);
-      cudaGraph_t g = nullptr;
-      const cudaError_t ce = cudaStreamEndCapture(cs, &g);
-      h->hp.gkernels[b] = (int)(h->launches - l0);
-      h->launches = l0;
-      cudaStreamDestroy(cs);
-      if (rc) { if (g) cudaGraphDestroy(g); return rc; }
-      if (ce != cudaSuccess) return set_err("cudaStreamEndCapture", ce);
-      const cudaError_t ie = cudaGraphInstantiate(&h->hp.gexec[b], g, 0);
-      cudaGraphDestroy(g);
-      if (ie != cudaSuccess) return set_err("cudaGraphInstantiate", ie);
+      rc = capture_chain(h, [&](cudaStream_t cs) { return step_impl(h, nullptr, flags, cs, nullptr, b); }, nullptr, &h->hp.gexec[b],
+                         &h->hp.gkernels[b]);
+      if (rc) return rc;
       h->hp.gflags[b] = flags;
     }
     CK(cudaGraphLaunch(h->hp.gexec[b], st));
@@ -2583,14 +2620,13 @@ static void rollout_params(ssa_ukf* h, RolloutParams* p, int only_done) {
   p->orbits = h->ro.orbits; p->n_orbits = h->ro.n_orbits;
   p->key = h->ro.key; p->episode = h->ro.episode; p->step_idx = h->step_idx;
   p->actions = h->ro.act_in; p->act_eff = h->ro.act_eff;
-  const size_t N = h->cfg.n_objects, E = h->cfg.n_envs;
-  p->done = only_done ? (const uint8_t*)((int32_t*)(h->ro.dout + 12 * N + E) + SSA_N_TASKERS * E) : nullptr;
+  p->done = only_done ? h->ro.dev.done : nullptr;
   p->sig = h->ro.sig;
   p->rew_hist = h->ro.rew_hist; p->spos_prev = h->ro.spos_prev;
-  p->greedy = (const int32_t*)(h->ro.dout + 12 * N + E); p->visible = h->visible;
+  p->greedy = h->ro.dev.greedy; p->visible = h->visible;
   p->tasker = h->ro.tasker; p->spoil_p = h->ro.spoil_p;
   p->E = h->cfg.n_envs; p->m = h->cfg.m; p->update_interval = h->ro.update_interval; p->n_steps = h->cfg.n_steps;
-  p->obs = h->ro.dout; p->term = nullptr; p->term_aer = 0;
+  p->obs = h->ro.dev.obs; p->term = nullptr; p->term_aer = 0;
   p->table = h->ro.table; p->n_table = h->ro.n_table;
   memset(&p->ob, 0, sizeof(p->ob));
   memcpy(p->ob.obs_itrs, h->cfg.obs_itrs, sizeof(p->ob.obs_itrs));
@@ -2598,23 +2634,19 @@ static void rollout_params(ssa_ukf* h, RolloutParams* p, int only_done) {
 }
 
 static void rollout_env_params(ssa_ukf* h, EnvParams* p, int increment, int greedy_only) {
-  const size_t N = h->cfg.n_objects, E = h->cfg.n_envs;
   p->dpos = h->dpos; p->dvel = h->dvel; p->spos = h->spos; p->trace = h->trace; p->visible = h->visible;
-  p->reward = h->ro.dout + 12 * N;
-  p->greedy = (int32_t*)(p->reward + E);
-  p->done = (uint8_t*)(p->greedy + SSA_N_TASKERS * E);
+  p->reward = h->ro.dev.reward; p->greedy = h->ro.dev.greedy; p->done = h->ro.dev.done; p->truncated = h->ro.dev.truncated;
   p->env_stats = h->env_stats;
   p->E = h->cfg.n_envs; p->m = h->cfg.m; p->reward_type = h->cfg.reward_type; p->n_steps = h->cfg.n_steps;
   p->step_index = -1; p->step_idx = h->step_idx; p->increment = increment; p->greedy_only = greedy_only;
   p->P = h->P; p->ld = h->ld; p->det_prev = h->det_prev; p->det_last = h->det_last; p->det_step = h->det_step;
   p->det_cur = h->det_cur; p->reset_mask = nullptr;
   p->rew_hist = h->ro.rew_hist; p->spos_prev = h->ro.spos_prev; p->act_in = h->ro.act_in;
-  p->truncated = p->done + ((E + 7) / 8) * 8;
 }
 
 static void launch_env_reduce(ssa_ukf* h, const EnvParams& ep, cudaStream_t st) {
   const int N = h->cfg.n_objects;
-  if (ep.m <= 64 && !getenv("SSA_UKF_DET_KERNEL")) {  // determinants inside the reduction
+  if (ep.m <= 64 && !h->det_kernel) {  // determinants inside the reduction
     EnvParams e2 = ep;
     e2.det_cur = nullptr;
     ssa_env_reduce_kernel<true><<<(unsigned)((ep.E + 3) / 4), 128, 0, st>>>(e2);
@@ -2634,7 +2666,7 @@ static int rollout_refresh(ssa_ukf* h, cudaStream_t st, const uint8_t* mask) {
   rollout_env_params(h, &ep, 0, 1);
   ep.reset_mask = mask;
   // (observations, visibility, determinants and greedy actions of the other environments are this step's already)
-  StepOverride ov{h->ro.dout, h->ro.act_eff, h->ro.table, h->step_idx, 0, h->ro.n_table, mask};
+  StepOverride ov{h->ro.dev.obs, h->ro.act_eff, h->ro.table, h->step_idx, 0, h->ro.n_table, mask};
   int rc = step_impl(h, nullptr, SSA_STEP_EPILOGUE, st, nullptr, -1, &ov);
   if (rc) return rc;
   launch_env_reduce(h, ep, st);
@@ -2649,22 +2681,9 @@ int ssa_ukf_rollout_config(ssa_ukf* h, const double* orbits, int n_orbits, const
   CK(cudaSetDevice(h->device));
   const size_t N = h->cfg.n_objects, E = h->cfg.n_envs;
   // (the cached graphs of ssa_ukf_step stay valid: every pointer they captured belongs to the handle)
-  if (h->ro.init) {
-    cudaFree(h->ro.dbuf); cudaFree(h->ro.ibuf); cudaFree(h->ro.dout); cudaFreeHost(h->ro.hout); cudaFreeHost(h->ro.hin);
-    cudaFree(h->ro.dobs32); cudaFreeHost(h->ro.hobs32);
-    cudaFree(h->ro.daer); cudaFreeHost(h->ro.haer); cudaFree(h->ro.rew_hist);
-    cudaFree(h->ro.tbuf); cudaFreeHost(h->ro.htbuf);
-    for (int i = 0; i < 6; ++i) if (h->ro.gexec[i]) { cudaGraphExecDestroy(h->ro.gexec[i]); h->ro.gexec[i] = nullptr; }
-    h->ro.init = 0;
-  }
-  if (h->es.on) {  // (a new configuration runs without episode statistics until they are enabled again)
-    cudaFree(h->es.buf); cudaFreeHost(h->es.hbuf);
-    memset(&h->es, 0, sizeof(h->es));
-  }
-  if (h->nm.on) {  // (nor normalization)
-    cudaFree(h->nm.buf); cudaFreeHost(h->nm.hbuf);
-    memset(&h->nm, 0, sizeof(h->nm));
-  }
+  rollout_free(h);
+  episode_stats_free(h);  // (a new configuration runs without episode statistics until they are enabled again)
+  norm_free(h);           // (nor normalization)
   h->ro.n_orbits = n_orbits; h->ro.n_table = n_table; h->ro.update_interval = update_interval;
   h->ro.tasker = SSA_TASKER_EXTERNAL; h->ro.spoil_p = 0.0;
   CK(cudaMalloc(&h->ro.dbuf, sizeof(double) * ((size_t)n_orbits * 6 + (size_t)n_table * 9 + 32)));
@@ -2681,12 +2700,15 @@ int ssa_ukf_rollout_config(ssa_ukf* h, const double* orbits, int n_orbits, const
   h->ro.key = h->ro.ibuf; h->ro.episode = h->ro.key + 2 * E;
   h->ro.act_in = (int32_t*)(h->ro.episode + E); h->ro.act_eff = h->ro.act_in + E;
   CK(cudaMemcpy(h->ro.key, seeds, sizeof(uint64_t) * E, cudaMemcpyHostToDevice));  // little-endian: key[2e] = low word
-  h->ro.out_bytes = sizeof(double) * (12 * N + E) + sizeof(int32_t) * SSA_N_TASKERS * E + 2 * (((E + 7) / 8) * 8);
-  CK(cudaMalloc(&h->ro.dout, h->ro.out_bytes));
-  CK(cudaMemset(h->ro.dout, 0, h->ro.out_bytes));
-  CK(cudaHostAlloc(&h->ro.hout, h->ro.out_bytes, cudaHostAllocDefault));
+  const size_t out_bytes = rollout_block(nullptr, N, E).bytes;
+  void *dout, *hout;
+  CK(cudaMalloc(&dout, out_bytes));
+  h->ro.dev = rollout_block(dout, N, E);
+  CK(cudaMemset(dout, 0, out_bytes));
+  CK(cudaHostAlloc(&hout, out_bytes, cudaHostAllocDefault));
+  h->ro.host = rollout_block(hout, N, E);
   CK(cudaHostAlloc(&h->ro.hin, sizeof(int32_t) * E, cudaHostAllocDefault));
-  memset(h->ro.hout, 0, h->ro.out_bytes);
+  memset(hout, 0, out_bytes);
   memset(h->ro.hin, 0, sizeof(int32_t) * E);
   CK(cudaMalloc(&h->ro.dobs32, sizeof(float) * 12 * N));
   CK(cudaMemset(h->ro.dobs32, 0, sizeof(float) * 12 * N));
@@ -2696,34 +2718,34 @@ int ssa_ukf_rollout_config(ssa_ukf* h, const double* orbits, int n_orbits, const
   CK(cudaMemset(h->ro.daer, 0, sizeof(double) * 4 * N));
   CK(cudaHostAlloc(&h->ro.haer, sizeof(double) * 4 * N, cudaHostAllocDefault));
   memset(h->ro.haer, 0, sizeof(double) * 4 * N);
-  h->ro.rew_hist = nullptr; h->ro.spos_prev = nullptr;
   if (h->cfg.reward_type == SSA_REWARD_SHAPED) {  // the reward history lives on the device (env_reset_body clears it)
     const size_t hist = sizeof(double) * E * (size_t)h->cfg.n_steps;
     CK(cudaMalloc(&h->ro.rew_hist, hist + sizeof(int32_t) * E));
     CK(cudaMemset(h->ro.rew_hist, 0, hist + sizeof(int32_t) * E));
     h->ro.spos_prev = (int32_t*)((char*)h->ro.rew_hist + hist);
   }
-  const size_t tbytes = sizeof(double) * 24 * N + sizeof(int32_t) * E + E;
+  // the rows of a gathered download: n <= E final observations (term_w m <= 12 m doubles each), episode records
+  // (SSA_EPR doubles) or normalized final observations (F / 2 <= 6 m doubles)
+  const size_t grows = std::max(12 * N, (size_t)SSA_EPR * E);
+  const size_t tbytes = sizeof(double) * (12 * N + grows) + sizeof(int32_t) * E + E;
   CK(cudaMalloc(&h->ro.tbuf, tbytes));
   CK(cudaMemset(h->ro.tbuf, 0, tbytes));
-  h->ro.term = h->ro.tbuf; h->ro.tgath = h->ro.term + 12 * N;
-  h->ro.tidx = (int32_t*)(h->ro.tgath + 12 * N); h->ro.mask = (uint8_t*)(h->ro.tidx + E);
-  CK(cudaHostAlloc(&h->ro.htbuf, sizeof(double) * 12 * N + sizeof(int32_t) * E, cudaHostAllocDefault));
-  h->ro.htidx = (int32_t*)(h->ro.htbuf + 12 * N);
+  h->ro.term = h->ro.tbuf; h->ro.gath = h->ro.term + 12 * N;
+  h->ro.gidx = (int32_t*)(h->ro.gath + grows); h->ro.mask = (uint8_t*)(h->ro.gidx + E);
+  CK(cudaHostAlloc(&h->ro.hgath, sizeof(double) * grows + sizeof(int32_t) * E, cudaHostAllocDefault));
+  h->ro.hgidx = (int32_t*)(h->ro.hgath + grows);
   h->ro.term_w = 12;
-  for (int i = 0; i < 6; ++i) h->ro.gexec[i] = nullptr;
   h->ro.init = 1;
   return SSA_OK;
 }
 
 int ssa_ukf_rollout_io(ssa_ukf* h, int32_t** actions, double** obs, double** reward, int32_t** greedy, uint8_t** done) {
-  if (!h || !h->ro.init) return SSA_EINVAL;
-  const size_t N = h->cfg.n_objects, E = h->cfg.n_envs;
+  if (!rollout_ready(h)) return SSA_EINVAL;
   if (actions) *actions = h->ro.hin;
-  if (obs) *obs = h->ro.hout;
-  if (reward) *reward = h->ro.hout + 12 * N;
-  if (greedy) *greedy = (int32_t*)(h->ro.hout + 12 * N + E);
-  if (done) *done = (uint8_t*)((int32_t*)(h->ro.hout + 12 * N + E) + SSA_N_TASKERS * E);
+  if (obs) *obs = h->ro.host.obs;
+  if (reward) *reward = h->ro.host.reward;
+  if (greedy) *greedy = h->ro.host.greedy;
+  if (done) *done = h->ro.host.done;
   return SSA_OK;
 }
 
@@ -2739,13 +2761,30 @@ static cudaError_t norm_copy_out(ssa_ukf* h, cudaStream_t st) {
   return cudaMemcpyAsync(h->nm.hbuf, h->nm.reward, sizeof(double) * E + sizeof(float) * E * h->nm.F, cudaMemcpyDeviceToHost, st);
 }
 
-// the captured step graphs of the episodic mode (re-captured on the next ssa_ukf_rollout_step)
-static void rollout_drop_graphs(ssa_ukf* h) {
-  for (int i = 0; i < 6; ++i) if (h->ro.gexec[i]) { cudaGraphExecDestroy(h->ro.gexec[i]); h->ro.gexec[i] = nullptr; }
+// The end of ssa_ukf_rollout_reset (mask null, SSA_NORM_RESET) and of ssa_ukf_rollout_reset_envs (SSA_NORM_RESET_ENVS):
+// re-draw the environments in mask (null: every environment), evaluate their fresh objects, then the output block, the
+// 'aer' rows and the normalized rows to their host mirrors.
+static int rollout_redraw(ssa_ukf* h, cudaStream_t st, const uint8_t* mask, int norm_mode) {
+  RolloutParams rp;
+  rollout_params(h, &rp, 0);
+  rp.done = mask;
+  k_env_reset<<<(unsigned)rp.E, 128, 0, st>>>(rp);
+  h->launches++;
+  int rc = rollout_refresh(h, st, mask);
+  if (rc) return rc;
+  launch_obs_aer(h, st);  // (the 'aer' rows of the fresh episodes, whichever layout the steps will use)
+  CK(cudaMemcpyAsync(h->ro.host.obs, h->ro.dev.obs, h->ro.dev.bytes, cudaMemcpyDeviceToHost, st));
+  CK(cudaMemcpyAsync(h->ro.haer, h->ro.daer, sizeof(double) * 4 * h->cfg.n_objects, cudaMemcpyDeviceToHost, st));
+  if (h->nm.on) {
+    launch_normalize(h, st, norm_mode, 0, mask);
+    CK(norm_copy_out(h, st));
+  }
+  CK(cudaGetLastError());
+  return SSA_OK;
 }
 
 int ssa_ukf_rollout_reset(ssa_ukf* h, void* stream) {
-  if (!h || !h->ro.init) return SSA_EINVAL;
+  if (!rollout_ready(h)) return SSA_EINVAL;
   CK(cudaSetDevice(h->device));
   cudaStream_t st = (cudaStream_t)stream;
   if (h->es.on) {  // every environment starts an episode: accumulators and records cleared, accumulation from here on
@@ -2753,21 +2792,7 @@ int ssa_ukf_rollout_reset(ssa_ukf* h, void* stream) {
     CK(cudaMemsetAsync(h->es.buf, 0, sizeof(double) * (N * SSA_EPO + E * (SSA_EPE + SSA_EPR)), st));
     if (!h->es.live) { rollout_drop_graphs(h); h->es.live = 1; }
   }
-  RolloutParams rp;
-  rollout_params(h, &rp, 0);
-  k_env_reset<<<(unsigned)rp.E, 128, 0, st>>>(rp);
-  h->launches++;
-  int rc = rollout_refresh(h, st, nullptr);
-  if (rc) return rc;
-  launch_obs_aer(h, st);  // (the 'aer' rows of the fresh episodes, whichever layout the steps will use)
-  CK(cudaMemcpyAsync(h->ro.hout, h->ro.dout, h->ro.out_bytes, cudaMemcpyDeviceToHost, st));
-  CK(cudaMemcpyAsync(h->ro.haer, h->ro.daer, sizeof(double) * 4 * h->cfg.n_objects, cudaMemcpyDeviceToHost, st));
-  if (h->nm.on) {
-    launch_normalize(h, st, SSA_NORM_RESET, 0, nullptr);
-    CK(norm_copy_out(h, st));
-  }
-  CK(cudaGetLastError());
-  return SSA_OK;
+  return rollout_redraw(h, st, nullptr, SSA_NORM_RESET);
 }
 
 // the kernels of one episodic step (captured into a graph by ssa_ukf_rollout_step)
@@ -2822,7 +2847,7 @@ static void launch_obs_aer(ssa_ukf* h, cudaStream_t st) {
   memcpy(ob.obs_itrs, h->cfg.obs_itrs, sizeof(ob.obs_itrs));
   memcpy(ob.T, h->cfg.T, sizeof(ob.T));
   const long N = h->cfg.n_objects;
-  k_obs_aer<<<(unsigned)((N + 127) / 128), 128, 0, st>>>(h->ro.dout, h->step_idx, h->ro.table, h->ro.n_table, ob, h->cfg.m, N,
+  k_obs_aer<<<(unsigned)((N + 127) / 128), 128, 0, st>>>(h->ro.dev.obs, h->step_idx, h->ro.table, h->ro.n_table, ob, h->cfg.m, N,
                                                          h->ro.daer);
   h->launches++;
 }
@@ -2935,14 +2960,14 @@ __global__ void __launch_bounds__(kNormThreads) k_normalize(const NormParams p) 
 }
 
 static void launch_normalize(ssa_ukf* h, cudaStream_t st, int mode, int auto_reset, const uint8_t* mask) {
-  const size_t N = h->cfg.n_objects, E = h->cfg.n_envs;
+  const size_t E = h->cfg.n_envs;
   const ssa_norm_cfg& c = h->nm.cfg;
   NormParams p;
-  p.obs = c.obs_layout == SSA_NORM_OBS_AER ? h->ro.daer : h->ro.dout;
+  p.obs = c.obs_layout == SSA_NORM_OBS_AER ? h->ro.daer : h->ro.dev.obs;
   p.f32 = c.obs_layout == SSA_NORM_OBS_ROWS_F32;
   p.term = mode == SSA_NORM_STEP && auto_reset ? h->ro.term : nullptr;
-  p.reward = h->ro.dout + 12 * N;
-  p.done = mode == SSA_NORM_RESET_ENVS ? mask : (const uint8_t*)((const int32_t*)(p.reward + E) + SSA_N_TASKERS * E);
+  p.reward = h->ro.dev.reward;
+  p.done = mode == SSA_NORM_RESET_ENVS ? mask : h->ro.dev.done;
   p.state = h->nm.state; p.out = h->nm.obs; p.term_out = h->nm.term; p.reward_out = h->nm.reward;
   p.obs32 = mode == SSA_NORM_STEP && p.f32 ? h->ro.dobs32 : nullptr;
   p.E = (int)E; p.F = h->nm.F; p.mode = mode;
@@ -2965,15 +2990,13 @@ struct EpParams {
 static_assert(SSA_EPR == SSA_EPISODE_STATS_DOUBLES, "episode record layout");
 
 static void ep_params(ssa_ukf* h, EpParams* p, int auto_reset) {
-  const size_t N = h->cfg.n_objects, E = h->cfg.n_envs;
   p->xt = h->xt; p->x = h->x; p->P = h->P; p->ld = h->ld;
   p->step_idx = h->step_idx; p->act_eff = h->ro.act_eff;
   p->updated = h->updated; p->y = h->y; p->S = h->S;
-  p->reward = h->ro.dout + 12 * N;
-  p->done = (const uint8_t*)((const int32_t*)(p->reward + E) + SSA_N_TASKERS * E);
+  p->reward = h->ro.dev.reward; p->done = h->ro.dev.done;
   p->status = h->status;
   p->obj = h->es.obj; p->env = h->es.env; p->rec = h->es.rec;
-  p->E = (int)E; p->m = h->cfg.m; p->auto_reset = auto_reset;
+  p->E = h->cfg.n_envs; p->m = h->cfg.m; p->auto_reset = auto_reset;
 }
 
 // head of an episodic step: row 0 (the fresh draw, before the first predict) of the environments at step index 0, one
@@ -3026,7 +3049,7 @@ static int rollout_chain(ssa_ukf* h, cudaStream_t st, int auto_reset, int obs_f3
   }
   k_env_begin<<<(unsigned)((N + 127) / 128), 128, 0, st>>>(rp);
   h->launches++;
-  StepOverride ov{h->ro.dout, h->ro.act_eff, h->ro.table, h->step_idx, 1, h->ro.n_table, nullptr};
+  StepOverride ov{h->ro.dev.obs, h->ro.act_eff, h->ro.table, h->step_idx, 1, h->ro.n_table, nullptr};
   int rc = step_impl(h, nullptr, SSA_STEP_TRUTH | SSA_STEP_PREDICT | SSA_STEP_UPDATE_ACT | SSA_STEP_EPILOGUE | (stats ? SSA_STEP_RECORD : 0),
                      st, nullptr, -1, &ov);
   if (rc) return rc;
@@ -3038,12 +3061,12 @@ static int rollout_chain(ssa_ukf* h, cudaStream_t st, int auto_reset, int obs_f3
     k_ep_step<<<(unsigned)((rp.E + 3) / 4), 128, 0, st>>>(sp);
     h->launches++;
   }
-  if (auto_reset && !h->use_team && !getenv("SSA_UKF_REFRESH_CHAIN")) {  // one launch (k_env_refresh)
+  if (auto_reset && !h->use_team && !h->refresh_chain) {  // one launch (k_env_refresh)
     EnvParams rep;
     rollout_env_params(h, &rep, 0, 1);
     rep.reset_mask = rep.done;
-    if (rep.m <= 64 && !getenv("SSA_UKF_DET_KERNEL")) rep.det_cur = nullptr;  // determinants inside the reduction
-    StepOverride rov{h->ro.dout, h->ro.act_eff, h->ro.table, h->step_idx, 0, h->ro.n_table, rep.done};
+    if (rep.m <= 64 && !h->det_kernel) rep.det_cur = nullptr;  // determinants inside the reduction
+    StepOverride rov{h->ro.dev.obs, h->ro.act_eff, h->ro.table, h->step_idx, 0, h->ro.n_table, rep.done};
     KParams kp;
     rc = step_impl(h, nullptr, SSA_STEP_EPILOGUE, st, nullptr, -1, &rov, &kp, true);
     if (rc) return rc;
@@ -3058,7 +3081,7 @@ static int rollout_chain(ssa_ukf* h, cudaStream_t st, int auto_reset, int obs_f3
   const bool norm = h->nm.on != 0;
   if (obs_f32 && !norm) {  // (with normalization k_normalize writes the float32 rows)
     const long n2 = 6 * N;  // 12 N doubles, two at a time (the block is cudaMalloc-aligned)
-    k_obs_to_f32<<<(unsigned)((n2 + 255) / 256), 256, 0, st>>>((const double2*)h->ro.dout, (float2*)h->ro.dobs32, n2);
+    k_obs_to_f32<<<(unsigned)((n2 + 255) / 256), 256, 0, st>>>((const double2*)h->ro.dev.obs, (float2*)h->ro.dobs32, n2);
     h->launches++;
   }
   if (obs_aer) launch_obs_aer(h, st);
@@ -3067,31 +3090,28 @@ static int rollout_chain(ssa_ukf* h, cudaStream_t st, int auto_reset, int obs_f3
 }
 
 int ssa_ukf_rollout_obs_aer(ssa_ukf* h, double** host, double** device) {
-  if (!h || !h->ro.init) return SSA_EINVAL;
+  if (!rollout_ready(h)) return SSA_EINVAL;
   if (host) *host = h->ro.haer;
   if (device) *device = h->ro.daer;
   return SSA_OK;
 }
 
 int ssa_ukf_rollout_obs_f32(ssa_ukf* h, float** host, float** device) {
-  if (!h || !h->ro.init) return SSA_EINVAL;
+  if (!rollout_ready(h)) return SSA_EINVAL;
   if (host) *host = h->ro.hobs32;
   if (device) *device = h->ro.dobs32;
   return SSA_OK;
 }
 
 int ssa_ukf_rollout_episode_stats_enable(ssa_ukf* h) {
-  if (!h || !h->ro.init) { snprintf(g_err, sizeof(g_err), "episodic mode not configured"); return SSA_EINVAL; }
+  if (!rollout_ready(h)) return SSA_EINVAL;
   CK(cudaSetDevice(h->device));
   const size_t N = h->cfg.n_objects, E = h->cfg.n_envs;
-  if (h->es.on) { CK(cudaDeviceSynchronize()); cudaFree(h->es.buf); cudaFreeHost(h->es.hbuf); memset(&h->es, 0, sizeof(h->es)); }
+  if (h->es.on) { CK(cudaDeviceSynchronize()); episode_stats_free(h); }
   const size_t acc = N * SSA_EPO + E * (SSA_EPE + SSA_EPR);
-  CK(cudaMalloc(&h->es.buf, sizeof(double) * (acc + E * SSA_EPR) + sizeof(int32_t) * E));
-  CK(cudaMemset(h->es.buf, 0, sizeof(double) * (acc + E * SSA_EPR) + sizeof(int32_t) * E));
+  CK(cudaMalloc(&h->es.buf, sizeof(double) * acc));
+  CK(cudaMemset(h->es.buf, 0, sizeof(double) * acc));
   h->es.obj = h->es.buf; h->es.env = h->es.obj + N * SSA_EPO; h->es.rec = h->es.env + E * SSA_EPE;
-  h->es.gath = h->es.rec + E * SSA_EPR; h->es.didx = (int32_t*)(h->es.gath + E * SSA_EPR);
-  CK(cudaHostAlloc(&h->es.hbuf, sizeof(double) * E * SSA_EPR + sizeof(int32_t) * E, cudaHostAllocDefault));
-  h->es.hidx = (int32_t*)(h->es.hbuf + E * SSA_EPR);
   h->es.on = 1;
   h->es.live = 0;  // (from the next ssa_ukf_rollout_reset)
   rollout_drop_graphs(h);
@@ -3107,49 +3127,42 @@ static int check_envs(const ssa_ukf* h, const int32_t* envs, int n, const void* 
   return SSA_OK;
 }
 
+// the rows envs[0 .. n) (0 < n <= E, checked) of `row` doubles each of src into out, through the gather scratch of the
+// handle; returns once copied, so the downloads can share that scratch (one host thread per handle)
+static int gather_download(ssa_ukf* h, const double* src, long row, const int32_t* envs, int n, void* out, cudaStream_t st) {
+  CK(cudaSetDevice(h->device));
+  memcpy(h->ro.hgidx, envs, sizeof(int32_t) * n);
+  CK(cudaMemcpyAsync(h->ro.gidx, h->ro.hgidx, sizeof(int32_t) * n, cudaMemcpyHostToDevice, st));
+  k_gather_rows<<<(unsigned)((n * row + 255) / 256), 256, 0, st>>>(src, h->ro.gidx, n, row, h->ro.gath);
+  h->launches++;
+  CK(cudaGetLastError());
+  CK(cudaMemcpyAsync(h->ro.hgath, h->ro.gath, sizeof(double) * n * row, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  memcpy(out, h->ro.hgath, sizeof(double) * n * row);
+  return SSA_OK;
+}
+
 int ssa_ukf_rollout_episode_stats_download(ssa_ukf* h, const int32_t* envs, int n, double* out, void* stream) {
   if (!h) return SSA_EINVAL;
   if (!h->es.on) { snprintf(g_err, sizeof(g_err), "episode statistics not enabled"); return SSA_EINVAL; }
   if (check_envs(h, envs, n, out)) return SSA_EINVAL;
   if (n == 0) return SSA_OK;
-  CK(cudaSetDevice(h->device));
-  cudaStream_t st = (cudaStream_t)stream;
-  memcpy(h->es.hidx, envs, sizeof(int32_t) * n);
-  CK(cudaMemcpyAsync(h->es.didx, h->es.hidx, sizeof(int32_t) * n, cudaMemcpyHostToDevice, st));
-  k_gather_rows<<<(unsigned)((n * SSA_EPR + 255) / 256), 256, 0, st>>>(h->es.rec, h->es.didx, n, SSA_EPR, h->es.gath);
-  h->launches++;
-  CK(cudaGetLastError());
-  CK(cudaMemcpyAsync(h->es.hbuf, h->es.gath, sizeof(double) * n * SSA_EPR, cudaMemcpyDeviceToHost, st));
-  CK(cudaStreamSynchronize(st));
-  memcpy(out, h->es.hbuf, sizeof(double) * n * SSA_EPR);
-  return SSA_OK;
+  return gather_download(h, h->es.rec, SSA_EPR, envs, n, out, (cudaStream_t)stream);
 }
 
 int ssa_ukf_rollout_truncated(ssa_ukf* h, uint8_t** host, uint8_t** device) {
-  if (!h || !h->ro.init) { snprintf(g_err, sizeof(g_err), "episodic mode not configured"); return SSA_EINVAL; }
-  const size_t N = h->cfg.n_objects, E = h->cfg.n_envs, off = sizeof(double) * (12 * N + E) + sizeof(int32_t) * SSA_N_TASKERS * E +
-                                                               ((E + 7) / 8) * 8;
-  if (host) *host = (uint8_t*)h->ro.hout + off;
-  if (device) *device = (uint8_t*)h->ro.dout + off;
+  if (!rollout_ready(h)) return SSA_EINVAL;
+  if (host) *host = h->ro.host.truncated;
+  if (device) *device = h->ro.dev.truncated;
   return SSA_OK;
 }
 
 int ssa_ukf_rollout_terminal_obs_download(ssa_ukf* h, const int32_t* envs, int n, double* out, void* stream) {
-  if (!h || !h->ro.init) { snprintf(g_err, sizeof(g_err), "episodic mode not configured"); return SSA_EINVAL; }
+  if (!rollout_ready(h)) return SSA_EINVAL;
   if (check_envs(h, envs, n, out)) return SSA_EINVAL;
   if (n == 0) return SSA_OK;
-  CK(cudaSetDevice(h->device));
-  cudaStream_t st = (cudaStream_t)stream;
-  const long row = (long)h->ro.term_w * h->cfg.m;  // doubles per environment
-  memcpy(h->ro.htidx, envs, sizeof(int32_t) * n);
-  CK(cudaMemcpyAsync(h->ro.tidx, h->ro.htidx, sizeof(int32_t) * n, cudaMemcpyHostToDevice, st));
-  k_gather_rows<<<(unsigned)((n * row + 255) / 256), 256, 0, st>>>(h->ro.term, h->ro.tidx, n, row, h->ro.tgath);
-  h->launches++;
-  CK(cudaGetLastError());
-  CK(cudaMemcpyAsync(h->ro.htbuf, h->ro.tgath, sizeof(double) * n * row, cudaMemcpyDeviceToHost, st));
-  CK(cudaStreamSynchronize(st));
-  memcpy(out, h->ro.htbuf, sizeof(double) * n * row);
-  return SSA_OK;
+  // (rows of term_w doubles per object: the layout of the last auto-reset step)
+  return gather_download(h, h->ro.term, (long)h->ro.term_w * h->cfg.m, envs, n, out, (cudaStream_t)stream);
 }
 
 // ssa_ukf_rollout_reset_envs with episode statistics: the accumulators of the re-drawn environments start afresh
@@ -3159,7 +3172,7 @@ __global__ void __launch_bounds__(128) k_ep_clear(double* env, double* obj, cons
 }
 
 int ssa_ukf_rollout_reset_envs(ssa_ukf* h, const int32_t* envs, int n, void* stream) {
-  if (!h || !h->ro.init) { snprintf(g_err, sizeof(g_err), "episodic mode not configured"); return SSA_EINVAL; }
+  if (!rollout_ready(h)) return SSA_EINVAL;
   if (check_envs(h, envs, n, envs)) return SSA_EINVAL;
   if (n == 0) return SSA_OK;
   CK(cudaSetDevice(h->device));
@@ -3173,26 +3186,11 @@ int ssa_ukf_rollout_reset_envs(ssa_ukf* h, const int32_t* envs, int n, void* str
     k_ep_clear<<<(unsigned)((E + 127) / 128), 128, 0, st>>>(h->es.env, h->es.obj, h->ro.mask, E, h->cfg.m);
     h->launches++;
   }
-  RolloutParams rp;
-  rollout_params(h, &rp, 0);
-  rp.done = h->ro.mask;
-  k_env_reset<<<(unsigned)E, 128, 0, st>>>(rp);
-  h->launches++;
-  int rc = rollout_refresh(h, st, h->ro.mask);
-  if (rc) return rc;
-  launch_obs_aer(h, st);
-  CK(cudaMemcpyAsync(h->ro.hout, h->ro.dout, h->ro.out_bytes, cudaMemcpyDeviceToHost, st));
-  CK(cudaMemcpyAsync(h->ro.haer, h->ro.daer, sizeof(double) * 4 * h->cfg.n_objects, cudaMemcpyDeviceToHost, st));
-  if (h->nm.on) {
-    launch_normalize(h, st, SSA_NORM_RESET_ENVS, 0, h->ro.mask);
-    CK(norm_copy_out(h, st));
-  }
-  CK(cudaGetLastError());
-  return SSA_OK;
+  return rollout_redraw(h, st, h->ro.mask, SSA_NORM_RESET_ENVS);
 }
 
 int ssa_ukf_rollout_step(ssa_ukf* h, int auto_reset, void* stream) {
-  if (!h || !h->ro.init) return SSA_EINVAL;
+  if (!rollout_ready(h)) return SSA_EINVAL;
   CK(cudaSetDevice(h->device));
   cudaStream_t st = (cudaStream_t)stream;
   const size_t E = h->cfg.n_envs;
@@ -3210,24 +3208,11 @@ int ssa_ukf_rollout_step(ssa_ukf* h, int auto_reset, void* stream) {
   if (ar) h->ro.term_w = obs_aer ? 4 : 12;  // (the layout of the final observations this step records)
   const bool device_io = (auto_reset & SSA_ROLLOUT_DEVICE_IO) != 0, tasked = h->ro.tasker != SSA_TASKER_EXTERNAL;
   if (!device_io && !tasked) CK(cudaMemcpyAsync(h->ro.act_in, h->ro.hin, sizeof(int32_t) * E, cudaMemcpyHostToDevice, st));
-  const char* gv = getenv("SSA_UKF_GRAPH");
-  if (!(gv && strcmp(gv, "0") == 0) && !h->use_team) {
+  if (h->use_graph && !h->use_team) {
     if (!h->ro.gexec[a]) {
-      cudaStream_t cs;
-      CK(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
-      const long l0 = h->launches;
-      CK(cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal));
-      const int rc = rollout_chain(h, cs, ar, obs_f32, obs_aer);
-      cudaGraph_t g = nullptr;
-      const cudaError_t ce = cudaStreamEndCapture(cs, &g);
-      h->ro.gkernels[a] = (int)(h->launches - l0);
-      h->launches = l0;
-      cudaStreamDestroy(cs);
-      if (rc) { if (g) cudaGraphDestroy(g); return rc; }
-      if (ce != cudaSuccess) return set_err("cudaStreamEndCapture", ce);
-      const cudaError_t ie = cudaGraphInstantiate(&h->ro.gexec[a], g, 0);
-      cudaGraphDestroy(g);
-      if (ie != cudaSuccess) return set_err("cudaGraphInstantiate", ie);
+      const int rc = capture_chain(h, [&](cudaStream_t cs) { return rollout_chain(h, cs, ar, obs_f32, obs_aer); }, nullptr,
+                                   &h->ro.gexec[a], &h->ro.gkernels[a]);
+      if (rc) return rc;
     }
     CK(cudaGraphLaunch(h->ro.gexec[a], st));
     h->launches += h->ro.gkernels[a];
@@ -3236,28 +3221,22 @@ int ssa_ukf_rollout_step(ssa_ukf* h, int auto_reset, void* stream) {
     if (rc) return rc;
   }
   if (!device_io) {
-    if (h->nm.on) {  // normalized rewards and rows + the raw reward / greedy / done / truncated tail of the double block
-      const size_t N = h->cfg.n_objects;
-      CK(norm_copy_out(h, st));
-      CK(cudaMemcpyAsync(h->ro.hout + 12 * N, h->ro.dout + 12 * N, h->ro.out_bytes - sizeof(double) * 12 * N, cudaMemcpyDeviceToHost, st));
-    } else if (obs_f32) {  // float observations + the reward / greedy / done tail of the double block
-      const size_t N = h->cfg.n_objects;
-      CK(cudaMemcpyAsync(h->ro.hobs32, h->ro.dobs32, sizeof(float) * 12 * N, cudaMemcpyDeviceToHost, st));
-      CK(cudaMemcpyAsync(h->ro.hout + 12 * N, h->ro.dout + 12 * N, h->ro.out_bytes - sizeof(double) * 12 * N, cudaMemcpyDeviceToHost, st));
-    } else if (obs_aer) {  // the 'aer' observations + the same tail
-      const size_t N = h->cfg.n_objects;
-      CK(cudaMemcpyAsync(h->ro.haer, h->ro.daer, sizeof(double) * 4 * N, cudaMemcpyDeviceToHost, st));
-      CK(cudaMemcpyAsync(h->ro.hout + 12 * N, h->ro.dout + 12 * N, h->ro.out_bytes - sizeof(double) * 12 * N, cudaMemcpyDeviceToHost, st));
-    } else {
-      CK(cudaMemcpyAsync(h->ro.hout, h->ro.dout, h->ro.out_bytes, cudaMemcpyDeviceToHost, st));
-    }
+    // the observations in the step's layout: normalized (with the normalized rewards), float, 'aer', or the double rows
+    // of the output block; then the rest of the block (the raw reward, greedy, done and truncated tail)
+    const size_t N = h->cfg.n_objects;
+    size_t from = h->ro.dev.tail;
+    if (h->nm.on) CK(norm_copy_out(h, st));
+    else if (obs_f32) CK(cudaMemcpyAsync(h->ro.hobs32, h->ro.dobs32, sizeof(float) * 12 * N, cudaMemcpyDeviceToHost, st));
+    else if (obs_aer) CK(cudaMemcpyAsync(h->ro.haer, h->ro.daer, sizeof(double) * 4 * N, cudaMemcpyDeviceToHost, st));
+    else from = 0;
+    CK(cudaMemcpyAsync((char*)h->ro.host.obs + from, (char*)h->ro.dev.obs + from, h->ro.dev.bytes - from, cudaMemcpyDeviceToHost, st));
     if (tasked) CK(cudaMemcpyAsync(h->ro.hin, h->ro.act_in, sizeof(int32_t) * E, cudaMemcpyDeviceToHost, st));  // taken
   }
   return SSA_OK;
 }
 
 int ssa_ukf_rollout_tasker(ssa_ukf* h, int tasker, double spoil_p) {
-  if (!h || !h->ro.init) { snprintf(g_err, sizeof(g_err), "episodic mode not configured"); return SSA_EINVAL; }
+  if (!rollout_ready(h)) return SSA_EINVAL;
   if (tasker < SSA_TASKER_EXTERNAL || tasker > SSA_TASKER_VISIBLE_GREEDY_SPOILED) {
     snprintf(g_err, sizeof(g_err), "unknown tasker %d", tasker);
     return SSA_EINVAL;
@@ -3272,13 +3251,8 @@ int ssa_ukf_rollout_tasker(ssa_ukf* h, int tasker, double spoil_p) {
   return SSA_OK;
 }
 
-static void norm_free(ssa_ukf* h) {
-  cudaFree(h->nm.buf); cudaFreeHost(h->nm.hbuf);
-  memset(&h->nm, 0, sizeof(h->nm));
-}
-
 int ssa_ukf_rollout_normalize(ssa_ukf* h, const ssa_norm_cfg* cfg) {
-  if (!h || !h->ro.init) { snprintf(g_err, sizeof(g_err), "episodic mode not configured"); return SSA_EINVAL; }
+  if (!rollout_ready(h)) return SSA_EINVAL;
   CK(cudaSetDevice(h->device));
   if (!cfg) {
     if (h->nm.on) { CK(cudaDeviceSynchronize()); norm_free(h); rollout_drop_graphs(h); }
@@ -3314,21 +3288,20 @@ int ssa_ukf_rollout_normalize(ssa_ukf* h, const ssa_norm_cfg* cfg) {
   }
   if (h->nm.on) { CK(cudaDeviceSynchronize()); norm_free(h); }
   const size_t sd = 4 + E + 3 * F;  // state doubles
-  const size_t bytes = sizeof(double) * (sd + E) + sizeof(float) * 3 * E * F + sizeof(int32_t) * E;
+  const size_t bytes = sizeof(double) * (sd + E) + sizeof(float) * 2 * E * F;
   CK(cudaMalloc(&h->nm.buf, bytes));
   CK(cudaMemset(h->nm.buf, 0, bytes));
   h->nm.state = h->nm.buf; h->nm.reward = h->nm.state + sd;
-  h->nm.obs = (float*)(h->nm.reward + E); h->nm.term = h->nm.obs + E * F; h->nm.gath = h->nm.term + E * F;
-  h->nm.didx = (int32_t*)(h->nm.gath + E * F);
+  h->nm.obs = (float*)(h->nm.reward + E); h->nm.term = h->nm.obs + E * F;
   // RunningMeanStd(): mean 0, var 1, count 1e-4; the returns 0
   std::vector<double> st(sd, 0.0);
   st[1] = 1.0; st[2] = 1e-4; st[3] = c.training;
   for (size_t k = 0; k < F; ++k) { st[4 + E + F + k] = 1.0; st[4 + E + 2 * F + k] = 1e-4; }
   CK(cudaMemcpy(h->nm.state, st.data(), sizeof(double) * sd, cudaMemcpyHostToDevice));
-  const size_t hbytes = sizeof(double) * E + sizeof(float) * 2 * E * F + sizeof(int32_t) * E;
+  const size_t hbytes = sizeof(double) * E + sizeof(float) * E * F;
   CK(cudaHostAlloc(&h->nm.hbuf, hbytes, cudaHostAllocDefault));
   memset(h->nm.hbuf, 0, hbytes);
-  h->nm.hobs = (float*)(h->nm.hbuf + E); h->nm.hgath = h->nm.hobs + E * F; h->nm.hidx = (int32_t*)(h->nm.hgath + E * F);
+  h->nm.hobs = (float*)(h->nm.hbuf + E);
   h->nm.cfg = c; h->nm.F = (int)F; h->nm.on = 1;
   rollout_drop_graphs(h);
   return SSA_OK;
@@ -3385,18 +3358,8 @@ int ssa_ukf_rollout_terminal_obs_norm_download(ssa_ukf* h, const int32_t* envs, 
   if (!h || !h->nm.on) { snprintf(g_err, sizeof(g_err), "normalization not enabled"); return SSA_EINVAL; }
   if (check_envs(h, envs, n, out)) return SSA_EINVAL;
   if (n == 0) return SSA_OK;
-  CK(cudaSetDevice(h->device));
-  cudaStream_t st = (cudaStream_t)stream;
-  const long row = h->nm.F / 2;  // a row of F floats as F / 2 doubles (F = 12 m or 4 m is even)
-  memcpy(h->nm.hidx, envs, sizeof(int32_t) * n);
-  CK(cudaMemcpyAsync(h->nm.didx, h->nm.hidx, sizeof(int32_t) * n, cudaMemcpyHostToDevice, st));
-  k_gather_rows<<<(unsigned)((n * row + 255) / 256), 256, 0, st>>>((const double*)h->nm.term, h->nm.didx, n, row, (double*)h->nm.gath);
-  h->launches++;
-  CK(cudaGetLastError());
-  CK(cudaMemcpyAsync(h->nm.hgath, h->nm.gath, sizeof(float) * n * h->nm.F, cudaMemcpyDeviceToHost, st));
-  CK(cudaStreamSynchronize(st));
-  memcpy(out, h->nm.hgath, sizeof(float) * n * h->nm.F);
-  return SSA_OK;
+  // (a row of F floats as F / 2 doubles: F = 12 m or 4 m is even)
+  return gather_download(h, (const double*)h->nm.term, h->nm.F / 2, envs, n, out, (cudaStream_t)stream);
 }
 
 int ssa_ukf_step_profile(ssa_ukf* h, const double M[9], int flags, void* stream, double ms[5]) {

@@ -32,7 +32,7 @@ def _cfg(**over):
 
 @pytest.fixture
 def launch_path(monkeypatch):
-    """Sets the launch-path variables of one configuration (the handle reads them at creation and at every step)."""
+    """Sets the launch-path variables of one configuration (the handle reads them once, at its creation)."""
     for k in PATH_VARS:
         monkeypatch.delenv(k, raising=False)
 

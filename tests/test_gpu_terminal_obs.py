@@ -340,7 +340,8 @@ def test_reset_at_restarts_episode_statistics():
 
 
 def test_c_abi_refusals():
-    """reset_envs and the terminal download refuse bad lists and calls before rollout_config with SSA_EINVAL."""
+    """reset_envs and the terminal download refuse bad lists, and every episodic entry point refuses calls before
+    rollout_config, with SSA_EINVAL and a message."""
     cfg = _cfg(rso_count=4, steps=5, reward_type="jones")
     vec = VecSSATaskerEnv(cfg, 4, seeds=[1, 2, 3, 4], rng="device")
     u, lib = vec.ukf, vec.ukf.lib
@@ -361,4 +362,11 @@ def test_c_abi_refusals():
     assert b.lib.ssa_ukf_rollout_terminal_obs_download(b.h, H.p(zero), 1, H.p(out), None) == F.SSA_EINVAL
     assert b"not configured" in b.lib.ssa_ukf_last_error()
     assert b.lib.ssa_ukf_rollout_truncated(b.h, None, None) == F.SSA_EINVAL
+    for call in (lambda: b.lib.ssa_ukf_rollout_io(b.h, None, None, None, None, None),
+                 lambda: b.lib.ssa_ukf_rollout_reset(b.h, None), lambda: b.lib.ssa_ukf_rollout_step(b.h, 1, None),
+                 lambda: b.lib.ssa_ukf_rollout_obs_f32(b.h, None, None), lambda: b.lib.ssa_ukf_rollout_obs_aer(b.h, None, None)):
+        assert b.lib.ssa_ukf_download(b.h, -1, H.p(out), 8, None) == F.SSA_EINVAL  # (another message first)
+        assert b"unknown field" in b.lib.ssa_ukf_last_error()
+        assert call() == F.SSA_EINVAL
+        assert b"not configured" in b.lib.ssa_ukf_last_error()
     b.close()
