@@ -1756,6 +1756,38 @@ static RolloutBlock rollout_block(void* base, size_t N, size_t E) {
   return b;
 }
 
+// A parity's block of the double-buffered host pipeline (ssa_ukf_step_host, ssa_ukf_step_pinned), in doubles:
+//   OUT  [obs 12N][dpos ld][status ld int32]        <- one D2H copy in the pinned mode; pinned mirror hout
+//        [dvel ld][spos ld][svel ld][trace ld]      (device only; in hout: the step's reward terms, SSA_F_CATALOG_STATS)
+//   IN   [z_noise 3N][M 9][pad 1][actions E int32]  <- one H2D copy in the pinned mode; pinned mirror hin
+struct PipeBlock {
+  double* obs; double* dpos; int32_t* status; double* dvel; double* spos; double* svel; double* trace;
+  double* stats;  // (hout only)
+  double* z_noise; double* M; int32_t* actions;
+  size_t out, in, dev, hout;  // doubles: the two copies (OUT up to the status words, IN), the device block, hout
+};
+
+// the views of the device block dev, or (dev null) of the pinned mirrors hout and hin; all null: only the sizes
+static PipeBlock pipe_block(double* dev, double* hout, double* hin, size_t N, size_t E, size_t ld) {
+  PipeBlock b = {};
+  b.out = 12 * N + ld + ld / 2;
+  b.in = 3 * N + 10 + (E + 1) / 2;
+  b.dev = b.out + 4 * ld + b.in;
+  b.hout = b.out + 8;
+  double* out = dev ? dev : hout;
+  double* in = dev ? dev + b.out + 4 * ld : hin;
+  if (out) { b.obs = out; b.dpos = out + 12 * N; b.status = (int32_t*)(b.dpos + ld); }
+  if (dev) { b.dvel = b.dpos + ld + ld / 2; b.spos = b.dvel + ld; b.svel = b.spos + ld; b.trace = b.svel + ld; }
+  if (hout) b.stats = hout + b.out;
+  if (in) { b.z_noise = in; b.M = in + 3 * N; b.actions = (int32_t*)(b.M + 10); }
+  return b;
+}
+
+// SSA_UKF_KERNEL, the catalog step's kernels (unset or unknown: tile): tile, the tile kernels; tile2, the two
+// factorisations inside the tile kernels instead of k_factor / k_refactor; fused, one launch per full catalog step
+// (k_step_tile) instead of the four tile kernels; split, the five-kernel split pipeline; team, the 16-lane team kernel
+enum class StepKernel { tile, tile2, fused, split, team };
+
 struct ssa_ukf {
   ssa_ukf_cfg cfg;
   int device;
@@ -1776,11 +1808,8 @@ struct ssa_ukf {
   long staged_max;  // chunks up to this many objects use the TMA-staged k_update (default: all)
   CUtensorMap tm_z, tm_u, tm_s, tm_x;
   int pdl;  // programmatic dependent launch of the step's kernel chain (SSA_UKF_PDL=0 turns it off)
-  int use_tile;   // tile kernels (default); SSA_UKF_KERNEL=split selects the five-kernel split pipeline
-  int use_team;   // SSA_UKF_KERNEL=team selects the fused 16-lane team kernel instead of the split pipeline
-  int use_fused;  // one launch per full catalog step (k_step_tile) instead of the four tile kernels
-  int legacy_act; // SSA_UKF_ACT=split: the RL-mode update of the tasked objects runs as k_hx + k_update instead of k_update_tile
-  int fold_factor;  // tile2: the two factorisations inside the tile kernels instead of k_factor / k_refactor
+  StepKernel kernel;  // SSA_UKF_KERNEL
+  bool act_split;   // SSA_UKF_ACT=split: the RL-mode update of the tasked objects runs as k_hx + k_update instead of k_update_tile
   int use_graph;    // ssa_ukf_step_pinned / ssa_ukf_rollout_step as captured graphs (SSA_UKF_GRAPH=0: plain launches)
   int det_kernel;   // SSA_UKF_DET_KERNEL set: ssa_det_kernel also for m <= 64, not the determinants inside the reduction
   int refresh_chain;  // SSA_UKF_REFRESH_CHAIN set: an auto-reset step re-draws with k_env_reset + the refresh chain
@@ -1791,14 +1820,7 @@ struct ssa_ukf {
     long calls;
     cudaStream_t up, dn;
     cudaEvent_t e_up[2], e_c[2], e_dn[2];
-    // device block per parity, in doubles:
-    //   OUT  [obs 12N][dpos ld][status ld int32]        <- one D2H copy in the pinned mode
-    //        [dvel ld][spos ld][svel ld][trace ld]
-    //   IN   [z_noise 3N][M 9][pad 1][actions E int32]  <- one H2D copy in the pinned mode
-    double* block[2];
-    double* hin[2];     // pinned host mirror of IN  (ssa_ukf_host_io)
-    double* hout[2];    // pinned host mirror of OUT
-    size_t out_doubles, in_off, in_doubles;
+    PipeBlock dev[2], host[2];  // per parity: the device block and its pinned host mirrors (pipe_block, ssa_ukf_host_io)
     cudaGraphExec_t gexec[2];  // the step's kernel chain captured per parity (ssa_ukf_step_pinned)
     int gflags[2], gkernels[2];
   } hp;
@@ -1813,7 +1835,6 @@ struct ssa_ukf {
     int gkernels[4];
     cudaGraphNode_t hx_node[4];
     cudaKernelNodeParams hx_params[4];
-    KParams p[4];
   } sg;
   // device-resident episodic mode (ssa_ukf_rollout_*)
   struct {
@@ -1895,6 +1916,9 @@ static int capture_chain(ssa_ukf* h, Enqueue&& enqueue, cudaGraph_t* keep, cudaG
   cudaGraphDestroy(g);
   return ie == cudaSuccess ? SSA_OK : set_err("cudaGraphInstantiate", ie);
 }
+
+// the team kernel's rule: never captured into a graph; an auto-reset step re-draws with k_env_reset + the refresh chain
+static bool team_kernel(const ssa_ukf* h) { return h->kernel == StepKernel::team; }
 
 // the guard of the ssa_ukf_rollout_* entry points that need ssa_ukf_rollout_config
 static bool rollout_ready(const ssa_ukf* h) {
@@ -2033,12 +2057,11 @@ int ssa_ukf_create(const ssa_ukf_cfg* cfg, int device, ssa_ukf** out) {
   }
   cudaMemset(h->scratch, 0, sizeof(double) * (size_t)(21 + 78 + 39 + 39 + 3) * lds);
   {
-    const char* kv = getenv("SSA_UKF_KERNEL");
-    h->use_team = (kv && strcmp(kv, "team") == 0) ? 1 : 0;
-    h->use_tile = (kv && strcmp(kv, "split") == 0) ? 0 : 1;
-    h->use_fused = (kv && strcmp(kv, "fused") == 0) ? 1 : 0;
-    { const char* av = getenv("SSA_UKF_ACT"); h->legacy_act = (av && strcmp(av, "split") == 0) ? 1 : 0; }
-    h->fold_factor = (kv && strcmp(kv, "tile2") == 0) ? 1 : 0;
+    const char *kv = getenv("SSA_UKF_KERNEL"), *av = getenv("SSA_UKF_ACT");
+    const auto is = [](const char* v, const char* s) { return v && strcmp(v, s) == 0; };
+    h->kernel = is(kv, "team") ? StepKernel::team : is(kv, "split") ? StepKernel::split : is(kv, "fused") ? StepKernel::fused
+              : is(kv, "tile2") ? StepKernel::tile2 : StepKernel::tile;
+    h->act_split = is(av, "split");
     h->sm_count = 148;
     cudaDeviceGetAttribute(&h->sm_count, cudaDevAttrMultiProcessorCount, h->device);
     cudaFuncSetAttribute(k_update_tile<SSA_TILE, kTileThreads, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(UpdateTile<SSA_TILE>));
@@ -2078,7 +2101,7 @@ int ssa_ukf_destroy(ssa_ukf* h) {
   if (h->hp.init) {
     cudaStreamSynchronize(h->hp.up); cudaStreamSynchronize(h->hp.dn);
     for (int b = 0; b < 2; ++b) {
-      cudaFree(h->hp.block[b]); cudaFreeHost(h->hp.hin[b]); cudaFreeHost(h->hp.hout[b]);
+      cudaFree(h->hp.dev[b].obs); cudaFreeHost(h->hp.host[b].z_noise); cudaFreeHost(h->hp.host[b].obs);
       if (h->hp.gexec[b]) cudaGraphExecDestroy(h->hp.gexec[b]);
       cudaEventDestroy(h->hp.e_up[b]); cudaEventDestroy(h->hp.e_c[b]); cudaEventDestroy(h->hp.e_dn[b]);
     }
@@ -2279,18 +2302,16 @@ struct StepOverride {  // episodic mode: redirect the step's inputs / outputs
   const uint8_t* env_gate;  // refresh of the re-drawn environments only (null: every environment)
 };
 
+// the episodic step's: observations in the output block, effective actions, env e's trans_matrix table row step_idx[e] + bias
+static StepOverride rollout_override(const ssa_ukf* h, int bias, const uint8_t* env_gate) {
+  return StepOverride{h->ro.dev.obs, h->ro.act_eff, h->ro.table, h->step_idx, bias, h->ro.n_table, env_gate};
+}
+
 static int cat_stats_launch(ssa_ukf* h, const double* dpos, const double* trace, long index_offset, cudaStream_t st, double* out);
 
-static int step_impl(ssa_ukf* h, const double M[9], int flags, void* stream, cudaEvent_t* ev, int hostbuf = -1,
-                     const StepOverride* ov = nullptr, KParams* p_out = nullptr, bool params_only = false) {
-  if (!h) return SSA_EINVAL;
-  if ((flags & (SSA_STEP_UPDATE_ALL | SSA_STEP_UPDATE_ACT | SSA_STEP_EPILOGUE)) && !M && !(flags & SSA_STEP_M_PER_ENV) &&
-      hostbuf < 0 && !ov) {
-    snprintf(g_err, sizeof(g_err), "trans_matrix required for update/epilogue");
-    return SSA_EINVAL;
-  }
-  cudaStream_t st = (cudaStream_t)stream;
-  CK(cudaSetDevice(h->device));
+// The parameters of the step's kernels over the whole batch (obj0 = 0, Nc = N): inputs and outputs in the handle's
+// arrays, in the block of host-pipeline parity hostbuf (>= 0), or redirected by ov (episodic mode).
+static KParams step_params(const ssa_ukf* h, const double M[9], int flags, int hostbuf, const StepOverride* ov) {
   KParams p;
   memset(&p, 0, sizeof(p));
   const ssa_ukf_cfg& c = h->cfg;
@@ -2310,14 +2331,11 @@ static int step_impl(ssa_ukf* h, const double M[9], int flags, void* stream, cud
   memcpy(p.Wm, c.Wm, sizeof(p.Wm)); memcpy(p.Wc, c.Wc, sizeof(p.Wc));
   p.qr = h->qr;
   if (hostbuf >= 0) {  // outputs / inputs of the double-buffered host pipeline
-    const long N_ = c.n_objects, ld_ = h->ld;
-    double* b = h->hp.block[hostbuf];
-    p.obs = b; p.dpos = b + 12 * N_; p.status_out = (int32_t*)(p.dpos + ld_);
-    p.dvel = p.dpos + ld_ + ld_ / 2; p.spos = p.dvel + ld_; p.svel = p.spos + ld_; p.trace = p.svel + ld_;
-    p.z_noise = b + h->hp.in_off;
-    p.actions = (const int32_t*)(p.z_noise + 3 * N_ + 10);
+    const PipeBlock& b = h->hp.dev[hostbuf];
+    p.obs = b.obs; p.dpos = b.dpos; p.status_out = b.status; p.dvel = b.dvel; p.spos = b.spos; p.svel = b.svel; p.trace = b.trace;
+    p.z_noise = b.z_noise; p.actions = b.actions;
     if (!M && !(flags & SSA_STEP_M_PER_ENV)) {  // pinned mode: the trans_matrix arrives with the input block
-      p.Menv = p.z_noise + 3 * N_;
+      p.Menv = b.M;
       p.Mstride = 0;
     }
   }
@@ -2329,10 +2347,23 @@ static int step_impl(ssa_ukf* h, const double M[9], int flags, void* stream, cud
   if (M) memcpy(p.ob.M, M, sizeof(p.ob.M));
   memcpy(p.ob.obs_itrs, c.obs_itrs, sizeof(p.ob.obs_itrs));
   memcpy(p.ob.T, c.T, sizeof(p.ob.T));
-  if (p_out) *p_out = p;  // single-chunk launches all use these parameters (obj0 = 0, Nc = N)
-  if (params_only) return SSA_OK;
+  return p;
+}
+
+static int step_impl(ssa_ukf* h, const double M[9], int flags, void* stream, cudaEvent_t* ev, int hostbuf = -1,
+                     const StepOverride* ov = nullptr) {
+  if (!h) return SSA_EINVAL;
+  if ((flags & (SSA_STEP_UPDATE_ALL | SSA_STEP_UPDATE_ACT | SSA_STEP_EPILOGUE)) && !M && !(flags & SSA_STEP_M_PER_ENV) &&
+      hostbuf < 0 && !ov) {
+    snprintf(g_err, sizeof(g_err), "trans_matrix required for update/epilogue");
+    return SSA_EINVAL;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  CK(cudaSetDevice(h->device));
+  KParams p = step_params(h, M, flags, hostbuf, ov);
+  const ssa_ukf_cfg& c = h->cfg;
   if (ev) CK(cudaEventRecord(ev[0], st));
-  if (h->use_team) {
+  if (h->kernel == StepKernel::team) {
     const unsigned grid = (unsigned)((c.n_objects + kTeamsPerCta - 1) / kTeamsPerCta);
     ssa_step_kernel<<<grid, kCtaThreads, 0, st>>>(p);
     h->launches++;
@@ -2355,8 +2386,8 @@ static int step_impl(ssa_ukf* h, const double M[9], int flags, void* stream, cud
     const bool pdl = h->pdl && !ev;
     // the tile kernels keep the sigma sets in shared memory; the book-version filter (sigmas_f kept across calls)
     // and the RL-mode update of one tasked object per environment use the split kernels
-    const bool tile = h->use_tile && p.resample;
-    if (tile && h->use_fused && predict && (flags & SSA_STEP_UPDATE_ALL)) {  // the whole step of the chunk in one launch
+    const bool tile = h->kernel != StepKernel::split && p.resample;
+    if (tile && h->kernel == StepKernel::fused && predict && (flags & SSA_STEP_UPDATE_ALL)) {  // the whole step of the chunk in one launch
       launch_chain(pdl, k_step_tile<SSA_TILE, kTileThreads>, gtile, kTileThreads, sizeof(UpdateTile<SSA_TILE>), st, p, h->tm_s, h->tm_u);
       h->launches++;
       if (evc) for (int i = 1; i <= 5; ++i) CK(cudaEventRecord(evc[i], st));
@@ -2364,10 +2395,10 @@ static int step_impl(ssa_ukf* h, const double M[9], int flags, void* stream, cud
     }
     // SSA_UKF_KERNEL=tile2: the factorisations ride inside the tile kernels (two launches per catalog step, the factor
     // never in HBM) instead of running as k_factor / k_refactor (default: four launches, measured faster — DESIGN.md)
-    const bool fold = tile && h->fold_factor && predict;
+    const bool fold = tile && h->kernel == StepKernel::tile2 && predict;
     // (RL mode: the same kernel, only the tasked object of an environment takes the update — the others get the truth
     // measurement and the epilogue; the refresh after an auto-reset, gated per environment, keeps the split kernels)
-    const bool tile_upd = tile && ((flags & SSA_STEP_UPDATE_ALL) || ((flags & SSA_STEP_UPDATE_ACT) && !p.env_gate && !h->legacy_act));
+    const bool tile_upd = tile && ((flags & SSA_STEP_UPDATE_ALL) || ((flags & SSA_STEP_UPDATE_ACT) && !p.env_gate && !h->act_split));
     if ((predict || update) && !fold) { launch_chain(pdl, k_factor, gobj2, kObjThreads, 0, st, p); h->launches++; }
     if (evc) CK(cudaEventRecord(evc[1], st));
     if (predict || truth) {
@@ -2408,18 +2439,10 @@ static int step_impl(ssa_ukf* h, const double M[9], int flags, void* stream, cud
   return SSA_OK;
 }
 
-static void set_last_outputs(ssa_ukf* h, int hostbuf) {
-  if (hostbuf < 0) { h->last_dpos = h->dpos; h->last_trace = h->trace; return; }
-  const long N_ = h->cfg.n_objects, ld_ = h->ld;
-  const double* dpos = h->hp.block[hostbuf] + 12 * N_;
-  h->last_dpos = dpos;
-  h->last_trace = dpos + ld_ + ld_ / 2 + 3 * ld_;   // [dpos ld][status ld/2][dvel ld][spos ld][svel ld][trace ld]
-}
-
 int ssa_ukf_step(ssa_ukf* h, const double M[9], int flags, void* stream) {
   if (!h) return SSA_EINVAL;
-  set_last_outputs(h, -1);
-  if (!h->sg.on || h->use_team || (flags & SSA_STEP_M_PER_ENV) || !M || h->chunk < h->cfg.n_objects)
+  h->last_dpos = h->dpos; h->last_trace = h->trace;
+  if (!h->sg.on || team_kernel(h) || (flags & SSA_STEP_M_PER_ENV) || !M || h->chunk < h->cfg.n_objects)
     return step_impl(h, M, flags, stream, nullptr);
   CK(cudaSetDevice(h->device));
   cudaStream_t st = (cudaStream_t)stream;
@@ -2428,7 +2451,7 @@ int ssa_ukf_step(ssa_ukf* h, const double M[9], int flags, void* stream) {
   if (gi < 0) {  // capture the chain for this flag combination (at most 4 are cached)
     if (h->sg.n == 4) { cudaGraphExecDestroy(h->sg.gexec[3]); cudaGraphDestroy(h->sg.graph[3]); h->sg.n = 3; }
     gi = h->sg.n;
-    const int rc = capture_chain(h, [&](cudaStream_t cs) { return step_impl(h, M, flags, cs, nullptr, -1, nullptr, &h->sg.p[gi]); },
+    const int rc = capture_chain(h, [&](cudaStream_t cs) { return step_impl(h, M, flags, cs, nullptr); },
                                  &h->sg.graph[gi], &h->sg.gexec[gi], &h->sg.gkernels[gi]);
     if (rc) return rc;
     h->sg.hx_node[gi] = nullptr;
@@ -2453,8 +2476,8 @@ int ssa_ukf_step(ssa_ukf* h, const double M[9], int flags, void* stream) {
     h->sg.n = gi + 1;
   }
   if (h->sg.hx_node[gi]) {  // this step's trans_matrix
-    memcpy(h->sg.p[gi].ob.M, M, 9 * sizeof(double));
-    void* args[3] = {&h->sg.p[gi], &h->tm_s, &h->tm_u};  // k_hx takes the first, k_update_tile / k_step_tile all three
+    KParams p = step_params(h, M, flags, -1, nullptr);  // (one chunk: the parameters of every launch of the graph)
+    void* args[3] = {&p, &h->tm_s, &h->tm_u};  // k_hx takes the first, k_update_tile / k_step_tile all three
     cudaKernelNodeParams kp = h->sg.hx_params[gi];
     kp.kernelParams = args;
     kp.extra = nullptr;
@@ -2465,30 +2488,28 @@ int ssa_ukf_step(ssa_ukf* h, const double M[9], int flags, void* stream) {
   return SSA_OK;
 }
 
+// the handle's device current, and the double-buffered host pipeline allocated on first use
 static int hostpipe_init(ssa_ukf* h) {
+  CK(cudaSetDevice(h->device));
   if (h->hp.init) return SSA_OK;
   const size_t N = h->cfg.n_objects, E = h->cfg.n_envs, ld = h->ld;
   CK(cudaStreamCreateWithFlags(&h->hp.up, cudaStreamNonBlocking));
   CK(cudaStreamCreateWithFlags(&h->hp.dn, cudaStreamNonBlocking));
-  h->hp.out_doubles = 12 * N + ld + ld / 2;
-  h->hp.in_off = h->hp.out_doubles + 4 * ld;
-  h->hp.in_doubles = 3 * N + 10 + (E + 1) / 2;
+  const PipeBlock size = pipe_block(nullptr, nullptr, nullptr, N, E, ld);
   for (int b = 0; b < 2; ++b) {
-    const size_t tot = h->hp.in_off + h->hp.in_doubles;
-    CK(cudaMalloc(&h->hp.block[b], sizeof(double) * tot));
-    CK(cudaMemset(h->hp.block[b], 0, sizeof(double) * tot));
-    CK(cudaHostAlloc(&h->hp.hin[b], sizeof(double) * h->hp.in_doubles, cudaHostAllocDefault));
-    CK(cudaHostAlloc(&h->hp.hout[b], sizeof(double) * (h->hp.out_doubles + 8), cudaHostAllocDefault));  // + the step's reward terms
-    memset(h->hp.hin[b], 0, sizeof(double) * h->hp.in_doubles);
-    memset(h->hp.hout[b], 0, sizeof(double) * (h->hp.out_doubles + 8));
-    h->hp.gexec[b] = nullptr;
-    h->hp.gflags[b] = -1;
+    double *dev, *hout, *hin;
+    CK(cudaMalloc(&dev, sizeof(double) * size.dev));
+    CK(cudaMemset(dev, 0, sizeof(double) * size.dev));
+    h->hp.dev[b] = pipe_block(dev, nullptr, nullptr, N, E, ld);
+    CK(cudaHostAlloc(&hin, sizeof(double) * size.in, cudaHostAllocDefault));
+    CK(cudaHostAlloc(&hout, sizeof(double) * size.hout, cudaHostAllocDefault));
+    memset(hin, 0, sizeof(double) * size.in);
+    memset(hout, 0, sizeof(double) * size.hout);
+    h->hp.host[b] = pipe_block(nullptr, hout, hin, N, E, ld);
     CK(cudaEventCreateWithFlags(&h->hp.e_up[b], cudaEventDisableTiming));
     CK(cudaEventCreateWithFlags(&h->hp.e_c[b], cudaEventDisableTiming));
     CK(cudaEventCreateWithFlags(&h->hp.e_dn[b], cudaEventDisableTiming));
   }
-  h->hp.parity = 0;
-  h->hp.calls = 0;
   h->hp.init = 1;
   return SSA_OK;
 }
@@ -2496,33 +2517,30 @@ static int hostpipe_init(ssa_ukf* h) {
 int ssa_ukf_step_host(ssa_ukf* h, const double M[9], int flags, const int32_t* actions_host, const double* z_noise_host,
                       double* obs_host, double* delta_pos_host, int32_t* status_host, void* stream) {
   if (!h) return SSA_EINVAL;
-  CK(cudaSetDevice(h->device));
   int rc = hostpipe_init(h);
   if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
-  const size_t N = h->cfg.n_objects, E = h->cfg.n_envs, ld = h->ld;
+  const size_t N = h->cfg.n_objects, E = h->cfg.n_envs;
   const int b = h->hp.parity;
-  double* blk = h->hp.block[b];
-  int32_t* iblk = (int32_t*)(blk + 12 * N + ld);
-  double* zn_dev = blk + h->hp.in_off;
+  const PipeBlock& blk = h->hp.dev[b];
   if (!M) { snprintf(g_err, sizeof(g_err), "ssa_ukf_step_host: trans_matrix required"); return SSA_EINVAL; }
   // upload stream: buffer b is free once the compute of two calls ago has consumed it
   if (h->hp.calls >= 2) CK(cudaStreamWaitEvent(h->hp.up, h->hp.e_c[b], 0));
-  if (z_noise_host) CK(cudaMemcpyAsync(zn_dev, z_noise_host, sizeof(double) * 3 * N, cudaMemcpyHostToDevice, h->hp.up));
-  if (actions_host) CK(cudaMemcpyAsync(zn_dev + 3 * N + 10, actions_host, sizeof(int32_t) * E, cudaMemcpyHostToDevice, h->hp.up));
+  if (z_noise_host) CK(cudaMemcpyAsync(blk.z_noise, z_noise_host, sizeof(double) * 3 * N, cudaMemcpyHostToDevice, h->hp.up));
+  if (actions_host) CK(cudaMemcpyAsync(blk.actions, actions_host, sizeof(int32_t) * E, cudaMemcpyHostToDevice, h->hp.up));
   CK(cudaEventRecord(h->hp.e_up[b], h->hp.up));
   // compute on the caller's stream: needs this step's inputs and a drained output buffer
   CK(cudaStreamWaitEvent(st, h->hp.e_up[b], 0));
   if (h->hp.calls >= 2) CK(cudaStreamWaitEvent(st, h->hp.e_dn[b], 0));
   rc = step_impl(h, M, flags, stream, nullptr, b);
   if (rc) return rc;
-  set_last_outputs(h, b);
+  h->last_dpos = blk.dpos; h->last_trace = blk.trace;
   CK(cudaEventRecord(h->hp.e_c[b], st));
   // download stream
   CK(cudaStreamWaitEvent(h->hp.dn, h->hp.e_c[b], 0));
-  if (obs_host) CK(cudaMemcpyAsync(obs_host, blk, sizeof(double) * 12 * N, cudaMemcpyDeviceToHost, h->hp.dn));
-  if (delta_pos_host) CK(cudaMemcpyAsync(delta_pos_host, blk + 12 * N, sizeof(double) * N, cudaMemcpyDeviceToHost, h->hp.dn));
-  if (status_host) CK(cudaMemcpyAsync(status_host, iblk, sizeof(int32_t) * N, cudaMemcpyDeviceToHost, h->hp.dn));
+  if (obs_host) CK(cudaMemcpyAsync(obs_host, blk.obs, sizeof(double) * 12 * N, cudaMemcpyDeviceToHost, h->hp.dn));
+  if (delta_pos_host) CK(cudaMemcpyAsync(delta_pos_host, blk.dpos, sizeof(double) * N, cudaMemcpyDeviceToHost, h->hp.dn));
+  if (status_host) CK(cudaMemcpyAsync(status_host, blk.status, sizeof(int32_t) * N, cudaMemcpyDeviceToHost, h->hp.dn));
   CK(cudaEventRecord(h->hp.e_dn[b], h->hp.dn));
   h->hp.parity ^= 1;
   h->hp.calls++;
@@ -2541,28 +2559,24 @@ int ssa_ukf_host_join(ssa_ukf* h, void* stream) {
 int ssa_ukf_host_io(ssa_ukf* h, int parity, double** z_noise, double** M, int32_t** actions, double** obs,
                     double** delta_pos, int32_t** status) {
   if (!h || parity < 0 || parity > 1) return SSA_EINVAL;
-  CK(cudaSetDevice(h->device));
   int rc = hostpipe_init(h);
   if (rc) return rc;
-  const size_t N = h->cfg.n_objects, ld = h->ld;
-  double* in = h->hp.hin[parity];
-  double* out = h->hp.hout[parity];
-  if (z_noise) *z_noise = in;
-  if (M) *M = in + 3 * N;
-  if (actions) *actions = (int32_t*)(in + 3 * N + 10);
-  if (obs) *obs = out;
-  if (delta_pos) *delta_pos = out + 12 * N;
-  if (status) *status = (int32_t*)(out + 12 * N + ld);
+  const PipeBlock& io = h->hp.host[parity];
+  if (z_noise) *z_noise = io.z_noise;
+  if (M) *M = io.M;
+  if (actions) *actions = io.actions;
+  if (obs) *obs = io.obs;
+  if (delta_pos) *delta_pos = io.dpos;
+  if (status) *status = io.status;
   return SSA_OK;
 }
 
 int ssa_ukf_host_stats(ssa_ukf* h, int parity, double** stats_host, double** stats_device) {
   if (!h || parity < 0 || parity > 1) return SSA_EINVAL;
   if (!h->cat_stats) { snprintf(g_err, sizeof(g_err), "call ssa_ukf_catalog_stats first"); return SSA_EINVAL; }
-  CK(cudaSetDevice(h->device));
   int rc = hostpipe_init(h);
   if (rc) return rc;
-  if (stats_host) *stats_host = h->hp.hout[parity] + h->hp.out_doubles;
+  if (stats_host) *stats_host = h->hp.host[parity].stats;
   if (stats_device) *stats_device = h->cat_stats + 5 * (1 + parity);
   return SSA_OK;
 }
@@ -2572,20 +2586,19 @@ int ssa_ukf_step_pinned(ssa_ukf* h, int flags, void* stream, int* parity_used) {
   const bool no_d2h = (flags & SSA_STEP_NO_D2H) != 0;
   flags &= ~SSA_STEP_NO_D2H;
   if (flags & SSA_STEP_M_PER_ENV) { snprintf(g_err, sizeof(g_err), "ssa_ukf_step_pinned: one trans_matrix per call"); return SSA_EINVAL; }
-  CK(cudaSetDevice(h->device));
   int rc = hostpipe_init(h);
   if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   const int b = h->hp.parity;
-  double* blk = h->hp.block[b];
+  const PipeBlock &blk = h->hp.dev[b], &io = h->hp.host[b];
   // upload stream: the device buffer is free once the compute of two calls ago has consumed it
   if (h->hp.calls >= 2) CK(cudaStreamWaitEvent(h->hp.up, h->hp.e_c[b], 0));
-  CK(cudaMemcpyAsync(blk + h->hp.in_off, h->hp.hin[b], sizeof(double) * h->hp.in_doubles, cudaMemcpyHostToDevice, h->hp.up));
+  CK(cudaMemcpyAsync(blk.z_noise, io.z_noise, sizeof(double) * blk.in, cudaMemcpyHostToDevice, h->hp.up));
   CK(cudaEventRecord(h->hp.e_up[b], h->hp.up));
   // compute on the caller's stream: needs this step's inputs and a drained output buffer
   CK(cudaStreamWaitEvent(st, h->hp.e_up[b], 0));
   if (h->hp.calls >= 2) CK(cudaStreamWaitEvent(st, h->hp.e_dn[b], 0));
-  if (h->use_graph && !h->use_team) {
+  if (h->use_graph && !team_kernel(h)) {
     if (!h->hp.gexec[b] || h->hp.gflags[b] != flags) {  // (re)capture the kernel chain of this parity
       if (h->hp.gexec[b]) { cudaGraphExecDestroy(h->hp.gexec[b]); h->hp.gexec[b] = nullptr; }
       rc = capture_chain(h, [&](cudaStream_t cs) { return step_impl(h, nullptr, flags, cs, nullptr, b); }, nullptr, &h->hp.gexec[b],
@@ -2599,13 +2612,13 @@ int ssa_ukf_step_pinned(ssa_ukf* h, int flags, void* stream, int* parity_used) {
     rc = step_impl(h, nullptr, flags, stream, nullptr, b);
     if (rc) return rc;
   }
-  set_last_outputs(h, b);
+  h->last_dpos = blk.dpos; h->last_trace = blk.trace;
   CK(cudaEventRecord(h->hp.e_c[b], st));
   // download stream
   CK(cudaStreamWaitEvent(h->hp.dn, h->hp.e_c[b], 0));
-  if (!no_d2h) CK(cudaMemcpyAsync(h->hp.hout[b], blk, sizeof(double) * h->hp.out_doubles, cudaMemcpyDeviceToHost, h->hp.dn));
+  if (!no_d2h) CK(cudaMemcpyAsync(io.obs, blk.obs, sizeof(double) * blk.out, cudaMemcpyDeviceToHost, h->hp.dn));
   if ((flags & SSA_STEP_CATALOG_STATS) && h->cat_stats)  // the step's reward terms follow on the download stream (40 B)
-    CK(cudaMemcpyAsync(h->hp.hout[b] + h->hp.out_doubles, h->cat_stats + 5 * (1 + b), 5 * sizeof(double), cudaMemcpyDeviceToHost, h->hp.dn));
+    CK(cudaMemcpyAsync(io.stats, h->cat_stats + 5 * (1 + b), 5 * sizeof(double), cudaMemcpyDeviceToHost, h->hp.dn));
   CK(cudaEventRecord(h->hp.e_dn[b], h->hp.dn));
   if (parity_used) *parity_used = b;
   h->hp.parity ^= 1;
@@ -2633,23 +2646,32 @@ static void rollout_params(ssa_ukf* h, RolloutParams* p, int only_done) {
   memcpy(p->ob.T, h->cfg.T, sizeof(p->ob.T));
 }
 
-static void rollout_env_params(ssa_ukf* h, EnvParams* p, int increment, int greedy_only) {
-  p->dpos = h->dpos; p->dvel = h->dvel; p->spos = h->spos; p->trace = h->trace; p->visible = h->visible;
-  p->reward = h->ro.dev.reward; p->greedy = h->ro.dev.greedy; p->done = h->ro.dev.done; p->truncated = h->ro.dev.truncated;
-  p->env_stats = h->env_stats;
-  p->E = h->cfg.n_envs; p->m = h->cfg.m; p->reward_type = h->cfg.reward_type; p->n_steps = h->cfg.n_steps;
-  p->step_index = -1; p->step_idx = h->step_idx; p->increment = increment; p->greedy_only = greedy_only;
-  p->P = h->P; p->ld = h->ld; p->det_prev = h->det_prev; p->det_last = h->det_last; p->det_step = h->det_step;
-  p->det_cur = h->det_cur; p->reset_mask = nullptr;
-  p->rew_hist = h->ro.rew_hist; p->spos_prev = h->ro.spos_prev; p->act_in = h->ro.act_in;
+// The reward / done reduction and greedy taskers of ssa_ukf_env_reduce: every environment at step_index (< 0: at its own
+// step counter), into the handle's reward, done and greedy arrays; the 'shaped' reward is finished on the host.
+static EnvParams env_params(ssa_ukf* h, int step_index) {
+  EnvParams p = {};
+  p.dpos = h->dpos; p.dvel = h->dvel; p.spos = h->spos; p.trace = h->trace; p.visible = h->visible;
+  p.reward = h->reward; p.done = h->done; p.greedy = h->greedy; p.env_stats = h->env_stats;
+  p.E = h->cfg.n_envs; p.m = h->cfg.m; p.reward_type = h->cfg.reward_type; p.n_steps = h->cfg.n_steps;
+  p.step_index = step_index; p.step_idx = h->step_idx;
+  p.P = h->P; p.ld = h->ld; p.det_prev = h->det_prev; p.det_last = h->det_last; p.det_step = h->det_step;
+  p.det_cur = (p.m <= 64 && !h->det_kernel) ? nullptr : h->det_cur;  // null: determinants inside the reduction
+  return p;
+}
+
+// the episodic mode's: into the output block, at the device's step counters, with its 'shaped' state (reset_mask: see EnvParams)
+static EnvParams rollout_env_params(ssa_ukf* h, int increment, int greedy_only, const uint8_t* reset_mask) {
+  EnvParams p = env_params(h, -1);
+  p.reward = h->ro.dev.reward; p.greedy = h->ro.dev.greedy; p.done = h->ro.dev.done; p.truncated = h->ro.dev.truncated;
+  p.increment = increment; p.greedy_only = greedy_only; p.reset_mask = reset_mask;
+  p.rew_hist = h->ro.rew_hist; p.spos_prev = h->ro.spos_prev; p.act_in = h->ro.act_in;
+  return p;
 }
 
 static void launch_env_reduce(ssa_ukf* h, const EnvParams& ep, cudaStream_t st) {
   const int N = h->cfg.n_objects;
-  if (ep.m <= 64 && !h->det_kernel) {  // determinants inside the reduction
-    EnvParams e2 = ep;
-    e2.det_cur = nullptr;
-    ssa_env_reduce_kernel<true><<<(unsigned)((ep.E + 3) / 4), 128, 0, st>>>(e2);
+  if (!ep.det_cur) {  // determinants inside the reduction
+    ssa_env_reduce_kernel<true><<<(unsigned)((ep.E + 3) / 4), 128, 0, st>>>(ep);
     h->launches += 1;
     return;
   }
@@ -2662,14 +2684,11 @@ static void launch_env_reduce(ssa_ukf* h, const EnvParams& ep, cudaStream_t st) 
 // obs / errors / visibility of the current states + greedy taskers (after a reset) of the environments in `mask` (the
 // ones k_env_reset has just re-drawn; null: every environment)
 static int rollout_refresh(ssa_ukf* h, cudaStream_t st, const uint8_t* mask) {
-  EnvParams ep;
-  rollout_env_params(h, &ep, 0, 1);
-  ep.reset_mask = mask;
   // (observations, visibility, determinants and greedy actions of the other environments are this step's already)
-  StepOverride ov{h->ro.dev.obs, h->ro.act_eff, h->ro.table, h->step_idx, 0, h->ro.n_table, mask};
+  const StepOverride ov = rollout_override(h, 0, mask);
   int rc = step_impl(h, nullptr, SSA_STEP_EPILOGUE, st, nullptr, -1, &ov);
   if (rc) return rc;
-  launch_env_reduce(h, ep, st);
+  launch_env_reduce(h, rollout_env_params(h, 0, 1, mask), st);
   return SSA_OK;
 }
 
@@ -3049,28 +3068,19 @@ static int rollout_chain(ssa_ukf* h, cudaStream_t st, int auto_reset, int obs_f3
   }
   k_env_begin<<<(unsigned)((N + 127) / 128), 128, 0, st>>>(rp);
   h->launches++;
-  StepOverride ov{h->ro.dev.obs, h->ro.act_eff, h->ro.table, h->step_idx, 1, h->ro.n_table, nullptr};
+  const StepOverride ov = rollout_override(h, 1, nullptr);
   int rc = step_impl(h, nullptr, SSA_STEP_TRUTH | SSA_STEP_PREDICT | SSA_STEP_UPDATE_ACT | SSA_STEP_EPILOGUE | (stats ? SSA_STEP_RECORD : 0),
                      st, nullptr, -1, &ov);
   if (rc) return rc;
-  EnvParams ep;
-  rollout_env_params(h, &ep, 1, 0);
-  launch_env_reduce(h, ep, st);
+  launch_env_reduce(h, rollout_env_params(h, 1, 0, nullptr), st);
   if (auto_reset) { rp.term = h->ro.term; rp.term_aer = obs_aer; }  // (k_env_refresh / k_env_reset record them)
   if (stats) {
     k_ep_step<<<(unsigned)((rp.E + 3) / 4), 128, 0, st>>>(sp);
     h->launches++;
   }
-  if (auto_reset && !h->use_team && !h->refresh_chain) {  // one launch (k_env_refresh)
-    EnvParams rep;
-    rollout_env_params(h, &rep, 0, 1);
-    rep.reset_mask = rep.done;
-    if (rep.m <= 64 && !h->det_kernel) rep.det_cur = nullptr;  // determinants inside the reduction
-    StepOverride rov{h->ro.dev.obs, h->ro.act_eff, h->ro.table, h->step_idx, 0, h->ro.n_table, rep.done};
-    KParams kp;
-    rc = step_impl(h, nullptr, SSA_STEP_EPILOGUE, st, nullptr, -1, &rov, &kp, true);
-    if (rc) return rc;
-    k_env_refresh<<<(unsigned)rp.E, 128, 0, st>>>(rp, kp, rep);
+  if (auto_reset && !team_kernel(h) && !h->refresh_chain) {  // one launch (k_env_refresh)
+    const StepOverride rov = rollout_override(h, 0, rp.done);
+    k_env_refresh<<<(unsigned)rp.E, 128, 0, st>>>(rp, step_params(h, nullptr, SSA_STEP_EPILOGUE, -1, &rov), rollout_env_params(h, 0, 1, rp.done));
     h->launches++;
   } else if (auto_reset) {  // SSA_UKF_REFRESH_CHAIN=1 / team kernel: k_env_reset, then the gated refresh chain
     k_env_reset<<<(unsigned)rp.E, 128, 0, st>>>(rp);
@@ -3208,7 +3218,7 @@ int ssa_ukf_rollout_step(ssa_ukf* h, int auto_reset, void* stream) {
   if (ar) h->ro.term_w = obs_aer ? 4 : 12;  // (the layout of the final observations this step records)
   const bool device_io = (auto_reset & SSA_ROLLOUT_DEVICE_IO) != 0, tasked = h->ro.tasker != SSA_TASKER_EXTERNAL;
   if (!device_io && !tasked) CK(cudaMemcpyAsync(h->ro.act_in, h->ro.hin, sizeof(int32_t) * E, cudaMemcpyHostToDevice, st));
-  if (h->use_graph && !h->use_team) {
+  if (h->use_graph && !team_kernel(h)) {
     if (!h->ro.gexec[a]) {
       const int rc = capture_chain(h, [&](cudaStream_t cs) { return rollout_chain(h, cs, ar, obs_f32, obs_aer); }, nullptr,
                                    &h->ro.gexec[a], &h->ro.gkernels[a]);
@@ -3390,20 +3400,8 @@ int ssa_ukf_update(ssa_ukf* h, const double M[9], int all, void* stream) {
 int ssa_ukf_env_reduce(ssa_ukf* h, const double M[9], int step_index, void* stream) {
   (void)M;
   if (!h) return SSA_EINVAL;
-  cudaStream_t st = (cudaStream_t)stream;
   CK(cudaSetDevice(h->device));
-  EnvParams p;
-  p.dpos = h->dpos; p.dvel = h->dvel; p.spos = h->spos; p.trace = h->trace; p.visible = h->visible;
-  p.reward = h->reward; p.done = h->done; p.greedy = h->greedy; p.env_stats = h->env_stats;
-  p.E = h->cfg.n_envs; p.m = h->cfg.m; p.reward_type = h->cfg.reward_type; p.n_steps = h->cfg.n_steps;
-  p.step_index = step_index;
-  p.step_idx = h->step_idx;
-  p.increment = 0; p.greedy_only = 0;
-  p.P = h->P; p.ld = h->ld; p.det_prev = h->det_prev; p.det_last = h->det_last; p.det_step = h->det_step;
-  p.det_cur = h->det_cur; p.reset_mask = nullptr;
-  p.rew_hist = nullptr; p.spos_prev = nullptr; p.act_in = nullptr;  // 'shaped': finished on the host
-  p.truncated = nullptr;
-  launch_env_reduce(h, p, st);
+  launch_env_reduce(h, env_params(h, step_index), (cudaStream_t)stream);
   CK(cudaGetLastError());
   return SSA_OK;
 }

@@ -40,6 +40,25 @@ def _ptr(a):
     return a.ctypes.data_as(ctypes.c_void_p)
 
 
+def _host_array(ptr, ctype, shape):
+    """numpy view of `shape` over host memory the handle owns (its pinned blocks), at a ctypes pointer."""
+    n = int(np.prod(shape))
+    return np.ctypeslib.as_array(ctypes.cast(ptr, ctypes.POINTER(ctype)), shape=(n,)).reshape(shape)
+
+
+class _CudaArray:
+    def __init__(self, ptr, shape, typestr):
+        self.__cuda_array_interface__ = {"shape": tuple(shape), "typestr": typestr, "data": (ptr, False), "version": 2}
+
+
+def _device_tensor(ptr, shape, dtype, device):
+    """Zero-copy torch tensor of `shape` over device memory the handle owns, at address ptr on cuda:device."""
+    import torch
+    typestr = {np.dtype(np.float64): "<f8", np.dtype(np.float32): "<f4", np.dtype(np.int32): "<i4",
+               np.dtype(np.uint8): "|u1"}[np.dtype(dtype)]
+    return torch.as_tensor(_CudaArray(ptr, shape, typestr), device=torch.device("cuda", device))
+
+
 class BatchedUKF:
     """N = n_envs * m unscented Kalman filters resident on one GPU.
 
@@ -155,21 +174,13 @@ class BatchedUKF:
     def torch_view(self, field):
         """Zero-copy torch tensor over a handle-owned device buffer (AoS fields keep their host shape;
         SoA fields X_TRUE / X_FILTER / P_FILTER come back as [rows, ld])."""
-        import torch
-        ptr, nbytes = self.device_ptr(field)
+        ptr, _ = self.device_ptr(field)
         shape, dtype = self._shapes[field]
         if field in (_lib.F_X_TRUE, _lib.F_X_FILTER):
             shape = (6, self.ld)
         elif field == _lib.F_P_FILTER:
             shape = (21, self.ld)
-        typestr = {np.dtype(np.float64): "<f8", np.dtype(np.float32): "<f4", np.dtype(np.int32): "<i4",
-                   np.dtype(np.uint8): "|u1"}[np.dtype(dtype)]
-
-        class _CAI:
-            pass
-        o = _CAI()
-        o.__cuda_array_interface__ = {"shape": tuple(shape), "typestr": typestr, "data": (ptr, False), "version": 2}
-        return torch.as_tensor(o, device=torch.device("cuda", self.device))
+        return _device_tensor(ptr, shape, dtype, self.device)
 
     # -- the hot path -----------------------------------------------------------------------------
     def step(self, M, flags, stream=None):
@@ -206,14 +217,9 @@ class BatchedUKF:
             for b in range(2):
                 ptrs = [ctypes.c_void_p() for _ in range(6)]
                 _lib.check(self.lib.ssa_ukf_host_io(self.h, b, *[ctypes.byref(q) for q in ptrs]), "ssa_ukf_host_io")
-
-                def view(q, ctype, shape):
-                    n = int(np.prod(shape))
-                    return np.ctypeslib.as_array(ctypes.cast(q, ctypes.POINTER(ctype)), shape=(n,)).reshape(shape)
-
-                io.append({"z_noise": view(ptrs[0], ctypes.c_double, (N, 3)), "M": view(ptrs[1], ctypes.c_double, (9,)),
-                           "actions": view(ptrs[2], ctypes.c_int32, (E,)), "obs": view(ptrs[3], ctypes.c_double, (N, 12)),
-                           "delta_pos": view(ptrs[4], ctypes.c_double, (N,)), "status": view(ptrs[5], ctypes.c_int32, (N,))})
+                io.append({"z_noise": _host_array(ptrs[0], ctypes.c_double, (N, 3)), "M": _host_array(ptrs[1], ctypes.c_double, (9,)),
+                           "actions": _host_array(ptrs[2], ctypes.c_int32, (E,)), "obs": _host_array(ptrs[3], ctypes.c_double, (N, 12)),
+                           "delta_pos": _host_array(ptrs[4], ctypes.c_double, (N,)), "status": _host_array(ptrs[5], ctypes.c_int32, (N,))})
             self._io = io
             self._parity_out = ctypes.c_int(0)
         return self._io
@@ -223,19 +229,12 @@ class BatchedUKF:
         pinned host copy - valid after host_join() + sync -, device pointer of the slot).  Needs catalog_stats() once."""
         hp, dp = ctypes.c_void_p(), ctypes.c_void_p()
         _lib.check(self.lib.ssa_ukf_host_stats(self.h, int(parity), ctypes.byref(hp), ctypes.byref(dp)), "ssa_ukf_host_stats")
-        host = np.ctypeslib.as_array(ctypes.cast(hp, ctypes.POINTER(ctypes.c_double)), shape=(5,))
-        return host, dp.value
+        return _host_array(hp, ctypes.c_double, (5,)), dp.value
 
     def host_stats_torch(self, parity):
         """Zero-copy torch view [5] of the device slot of host_stats(parity) (input of an NCCL gather)."""
-        import torch
         _, dp = self.host_stats(parity)
-
-        class _CAI:
-            pass
-        o = _CAI()
-        o.__cuda_array_interface__ = {"shape": (5,), "typestr": "<f8", "data": (dp, False), "version": 2}
-        return torch.as_tensor(o, device=torch.device("cuda", self.device))
+        return _device_tensor(dp, (5,), np.float64, self.device)
 
     def step_pinned(self, flags, stream=None):
         """Pipelined step on the pinned blocks of host_io(): fill host_io()[b] of the parity this call will use
@@ -258,26 +257,21 @@ class BatchedUKF:
                                                    _ptr(xs), _ptr(zs), _ptr(P0), int(update_interval)), "ssa_ukf_rollout_config")
         ptrs = [ctypes.c_void_p() for _ in range(5)]
         _lib.check(self.lib.ssa_ukf_rollout_io(self.h, *[ctypes.byref(q) for q in ptrs]), "ssa_ukf_rollout_io")
-
-        def view(q, ctype, shape):
-            n = int(np.prod(shape))
-            return np.ctypeslib.as_array(ctypes.cast(q, ctypes.POINTER(ctype)), shape=(n,)).reshape(shape)
-
         N, E = self.N, self.n_envs
-        self.rollout_io = {"actions": view(ptrs[0], ctypes.c_int32, (E,)), "obs": view(ptrs[1], ctypes.c_double, (N, 12)),
-                           "reward": view(ptrs[2], ctypes.c_double, (E,)),
-                           "greedy": view(ptrs[3], ctypes.c_int32, (E, _lib.N_TASKERS)),
-                           "done": view(ptrs[4], ctypes.c_uint8, (E,))}
+        self.rollout_io = {"actions": _host_array(ptrs[0], ctypes.c_int32, (E,)), "obs": _host_array(ptrs[1], ctypes.c_double, (N, 12)),
+                           "reward": _host_array(ptrs[2], ctypes.c_double, (E,)),
+                           "greedy": _host_array(ptrs[3], ctypes.c_int32, (E, _lib.N_TASKERS)),
+                           "done": _host_array(ptrs[4], ctypes.c_uint8, (E,))}
         h32, d32 = ctypes.c_void_p(), ctypes.c_void_p()
         _lib.check(self.lib.ssa_ukf_rollout_obs_f32(self.h, ctypes.byref(h32), ctypes.byref(d32)), "ssa_ukf_rollout_obs_f32")
-        self.rollout_io["obs_f32"] = view(h32, ctypes.c_float, (N, 12))  # filled by rollout_step(obs_f32=True)
+        self.rollout_io["obs_f32"] = _host_array(h32, ctypes.c_float, (N, 12))  # filled by rollout_step(obs_f32=True)
         self.rollout_obs_f32_device = d32.value
         ha, da = ctypes.c_void_p(), ctypes.c_void_p()
         _lib.check(self.lib.ssa_ukf_rollout_obs_aer(self.h, ctypes.byref(ha), ctypes.byref(da)), "ssa_ukf_rollout_obs_aer")
-        self.rollout_io["obs_aer"] = view(ha, ctypes.c_double, (N, 4))  # filled by rollout_reset and rollout_step(obs_aer=True)
+        self.rollout_io["obs_aer"] = _host_array(ha, ctypes.c_double, (N, 4))  # filled by rollout_reset and rollout_step(obs_aer=True)
         ht = ctypes.c_void_p()
         _lib.check(self.lib.ssa_ukf_rollout_truncated(self.h, ctypes.byref(ht), None), "ssa_ukf_rollout_truncated")
-        self.rollout_io["truncated"] = view(ht, ctypes.c_uint8, (E,))  # done raised by the step limit alone
+        self.rollout_io["truncated"] = _host_array(ht, ctypes.c_uint8, (E,))  # done raised by the step limit alone
         self._term_w = 12
         self.rollout_norm_io = None  # (a new configuration runs without normalization, rollout_normalize)
         return self.rollout_io
@@ -352,9 +346,7 @@ class BatchedUKF:
         self._shapes[_lib.F_ROLLOUT_NORM_STATE] = ((4 + E + 3 * F,), np.float64)
         ho, hr = ctypes.c_void_p(), ctypes.c_void_p()
         _lib.check(self.lib.ssa_ukf_rollout_norm_io(self.h, ctypes.byref(ho), ctypes.byref(hr)), "ssa_ukf_rollout_norm_io")
-        self.rollout_norm_io = {
-            "obs": np.ctypeslib.as_array(ctypes.cast(ho, ctypes.POINTER(ctypes.c_float)), shape=(E * F,)).reshape(E, F),
-            "reward": np.ctypeslib.as_array(ctypes.cast(hr, ctypes.POINTER(ctypes.c_double)), shape=(E,))}
+        self.rollout_norm_io = {"obs": _host_array(ho, ctypes.c_float, (E, F)), "reward": _host_array(hr, ctypes.c_double, (E,))}
         return self.rollout_norm_io
 
     def rollout_norm_state(self, stream=None):
